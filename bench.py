@@ -22,6 +22,11 @@ HBM: fill, every max cell, every traceback.  GCUPS = sum(m*n) / 1e9 / seconds.
 
 `--impl reference` times the reference's CPU path instead: the C restatement of
 SmithWaterman.java under oracle/ (no JVM exists in this image) on all host cores.
+
+`--dump-outputs DIR` writes the results of the last timed step to DIR/<name>.npy (see dump_outputs), so that
+two builds can be compared output for output on identical, seeded inputs.
+
+bench.py compiles nothing: it runs from a tree built by `python __graft_entry__.py` (libswb200 and the CPU oracle).
 """
 from __future__ import annotations
 
@@ -53,7 +58,12 @@ def parse():
     ap.add_argument("--workspace-gb", type=float, default=64.0)
     ap.add_argument("--refs-per-gpu", type=int, default=N_REFS_PER_GPU,
                     help="10000 = BASELINE config 2 per GPU; 15402 x 8 GPUs = config 4 (123,212 refs, ~266 Mbp)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's results to DIR/<name>.npy (float64, at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 def peaks():
@@ -176,6 +186,48 @@ def workload_config(B, refs_per_gpu, world, n_refs_local, ref_bases_local):
             "parallelism": f"refshard{world}" if world > 1 else "single"}
 
 
+DUMP_MAX_BYTES = 64 * 10**6
+DUMP_MAX_PAIRS = 1 << 20
+DUMP_MAX_CELLS = 1 << 19
+DUMP_OPS_CELLS = 4096
+
+
+def dump_outputs(res, out_dir):
+    """What a caller of the timed path receives once it fetches the step's results, as out_dir/<name>.npy in float64
+    (exact for every int32 and int64 value the arrays hold).  Per-pair and per-cell arrays larger than the caps
+    above are cut to a fixed-seed sample; its indices go to pair_index / cell_index.  Pair p is (ref p // n_reads,
+    read p % n_reads); cells are numbered across pairs in the order of the result's flat arrays."""
+    import numpy as np
+
+    def sample(n, cap, seed):
+        if n <= cap:
+            return np.arange(n)
+        return np.sort(np.random.Generator(np.random.PCG64(seed)).choice(n, cap, replace=False))
+
+    res.fetch().cache()
+    pairs = sample(res.n_refs * res.n_reads, DUMP_MAX_PAIRS, 1)
+    cells = sample(res.total_cells, DUMP_MAX_CELLS, 2)
+    out = {"pair_index": pairs,
+           "scores": res.scores.reshape(-1)[pairs],
+           "cell_counts": np.diff(res.cell_offsets)[pairs],       # materialised max cells (none for score-0 pairs)
+           "ref_totals": res.ref_totals,
+           "best_hits": res.best_hits,                            # per read: score, ref, i, j
+           "cell_index": cells,
+           "cells": res.cells[cells],                             # (i, j), 1-based
+           "beginnings": res.beginnings[cells],
+           "op_lens": res.op_lens[cells],
+           # alignment columns (1 aligned, 2 insertion, 3 deletion) of the first sampled cells, concatenated;
+           # op_lens[:DUMP_OPS_CELLS] splits them
+           "ops": np.concatenate([np.zeros(0)] + [res.ops(int(c)) for c in cells[:DUMP_OPS_CELLS]])}
+    out = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in out.items()}
+    total = sum(a.nbytes + 128 for a in out.values())             # + the .npy header
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_MAX_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_reference(args):
     """--impl reference: the reference's CPU implementation of the path, all host cores."""
     rank = int(os.environ.get("RANK", "0"))
@@ -227,11 +279,12 @@ def main():
     import torch
     import sparksmithwaterman_b200 as swb
     from sparksmithwaterman_b200 import synth
-    from sparksmithwaterman_b200.build import build_native
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs writes one GPU's results; run it with --gpus 1")
     dist = None
     if world > 1:
         import torch.distributed as dist
@@ -242,10 +295,6 @@ def main():
         raise SystemExit("bench.py needs a CUDA device (no CPU fallback)")
     torch.cuda.set_device(local_rank)
     numa = bind_to_gpu_numa_node(local_rank) if world > 1 else None
-    if rank == 0:
-        build_native()
-    if dist:
-        dist.barrier()
 
     B, K, W = args.reads_per_step, args.steps, args.warmup
     # weak scaling: 10k refs per GPU; every rank generates the same global set and keeps its shard
@@ -324,7 +373,8 @@ def main():
         for key in agg:
             agg[key] += st[key]
         allgather_best(res)
-        res.free()
+        if k < W + K - 1:
+            res.free()                                            # the last step's results are freed after the clock
     ev1.record(stream)
     torch.cuda.synchronize()
     t_wall = time.perf_counter() - t_wall0
@@ -343,6 +393,9 @@ def main():
     else:
         cells_per_step = float(cells_per_step_local)
     value = cells_per_step / 1e9 / (step_ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(res, args.dump_outputs)
+    res.free()
 
     # ---- e2e: host buffers through swb_align, H2D + D2H inside the timed region ----------
     torch.cuda.synchronize()
