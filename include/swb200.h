@@ -97,6 +97,32 @@ int swb_align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd,
 int swb_result_fetch(swb_result *res);
 void swb_result_free(swb_result *res);
 
+/* HITS MODE: the same call, but alignments only where a read aligns best.  Every pair is still scored; each read's
+ * top_k best pairs are traced, and nothing else.  Arguments as swb_align / swb_align_resident plus
+ *   top_k      1 .. 32
+ *   min_score  >= 1: a hit has score >= min_score (a score-0 pair is never a hit)
+ * anything else is SWB_E_INVALID.
+ *   - scores, ref_totals and best_hits are those of the plain call, bit for bit; SWB_F_SCORES_ONLY, SWB_F_TIE_GT,
+ *     SWB_F_NO_FETCH + swb_result_fetch apply as there.
+ *   - hits (swb_result_hits): hits[(q * k + h) * 4 ..] = (score, ref, i, j), h = 0 .. k-1, read q's k best pairs
+ *     with score >= min_score, score descending, then reference index ascending (the best-hit rule: hits[q][0] ==
+ *     best_hits[q] whenever best_hits[q].score >= min_score).  (i, j) = the pair's first max cell in row-major
+ *     order, (0, 0) under SWB_F_SCORES_ONLY.  A read with fewer than k hits is padded with (0, -1, 0, 0).
+ *   - cells: only hit pairs have max cells, beginnings, op lengths and ops, each equal to what the plain call
+ *     returns for that pair (swb_result_materialize too).  cell_offsets still spans all pairs, so every accessor
+ *     applies; every other pair has an empty range and swb_result_pair_cell_count 0 (no implicit m*n cells).
+ *     A reference set that is cut into parts is aligned as one set here.
+ * Prefer it to SWB_F_SCORES_ONLY when the alignments of a read's best references are wanted, and to the plain call
+ * when the cells of all other pairs are not: the traceback, the assembly and the device->host copy shrink to k
+ * pairs per read. */
+int swb_align_hits(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
+                   int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score,
+                   swb_result **out);
+int swb_align_resident_hits(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
+                            int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_result **out);
+/* [n_reads * k * 4] of a fetched hits-mode result (NULL before the fetch), *top_k = k; NULL and *top_k = 0 for a plain result */
+const int32_t *swb_result_hits(const swb_result *res, int32_t *top_k);
+
 /* ONE pair through the context's submission queue.
  * Replaces: `new SmithWaterman.OptAlignments().call({ref, read}, {match, mismatch, gap}, types)` exactly as the
  * UNCHANGED driver issues it -- once per pair, from N Spark task threads (Distribution.java:419-426, :593;
@@ -134,7 +160,7 @@ const int32_t *swb_result_cells(const swb_result *res);       /* 2 per cell: i, 
 const int32_t *swb_result_beginnings(const swb_result *res);  /* per cell               */
 const int32_t *swb_result_op_lens(const swb_result *res);     /* per cell: #columns     */
 
-/* number of max cells of pair p including the implicit score-0 case */
+/* number of max cells of pair p including the implicit score-0 case (none in hits mode) */
 int64_t swb_result_pair_cell_count(const swb_result *res, int64_t pair);
 /* k-th max cell of pair p (reference list order): i, j, beginning, op_len */
 int swb_result_pair_cell(const swb_result *res, int64_t pair, int64_t k,
@@ -153,7 +179,8 @@ int swb_result_materialize(const swb_result *res, int64_t cell,
 /* timings of the call in milliseconds (CUDA events on the engine's stream) and counters:
  * out[0]=h2d  out[1]=fill  out[2]=locate+sort  out[3]=traceback  out[4]=d2h  out[5]=total device
  * out[6]=cells (sum m*n)  out[7]=pairs  out[8]=materialised max cells  out[9]=kernel launches
- * out[10]=checkpoint bytes written  out[11]=read batches (swb_align_pair: requests served by the pair's batch) */
+ * out[10]=checkpoint bytes written  out[11]=read batches (swb_align_pair: requests served by the pair's batch)
+ * out[12]=hits mode: top-k selection ms (the selections of the short path run inside out[2]'s span) */
 int swb_result_stats(const swb_result *res, double *out, int n);
 
 /* Device pointers of the HBM-resident outputs (for collectives over NVLink without a
@@ -207,6 +234,16 @@ void swb_multi_result_free(swb_multi_result *res);
 swb_result *swb_multi_result_shard(swb_multi_result *res, int32_t d);
 /* merged[4*q .. 4*q+3] = (score, GLOBAL ref index, i, j) of read q over all shards */
 const int32_t *swb_multi_result_best_hits(const swb_multi_result *res);
+/* Hits mode: swb_align_hits on every shard (local reference indices, all cells with their shard), then each shard's
+ * hit lists -> global ids -> one more ncclAllGather (n_reads * k * 16 bytes) -> a k-way merge kernel.  The merged
+ * list is the top k over the union of the shards' lists in the same order -- exact, since the global top k lies in
+ * that union -- so it is the same for any device count and equal to one context's hits over the whole set.
+ * Entries without a reference never win.  (Up to 64 devices.) */
+int  swb_multi_align_hits(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
+                          int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score,
+                          swb_multi_result **out);
+/* merged[(q * k + h) * 4 ..] = (score, GLOBAL ref index, i, j), *top_k = k; NULL and 0 for a plain result */
+const int32_t *swb_multi_result_hits(const swb_multi_result *res, int32_t *top_k);
 /* out[0] = wall ms of the call, out[1] = max over devices of the align's device ms, out[2] = allgather + merge ms */
 int  swb_multi_result_stats(const swb_multi_result *res, double *out, int n);
 
@@ -221,6 +258,10 @@ void swb_comm_destroy(swb_comm *c);
 int  swb_comm_allgather_best(swb_comm *c, const swb_result *res, const int64_t *global_ids, int64_t n_local_refs,
                              int32_t *merged_host);
 int  swb_comm_merged_device_ptr(swb_comm *c, void **ptr, int64_t *n_elems);
+/* The same for the hit lists of a hits-mode result (every rank passes the same top_k): merged_host (nullable)
+ * receives [n_reads * k * 4], (score, GLOBAL ref index, i, j), merged as in swb_multi_align_hits. */
+int  swb_comm_allgather_hits(swb_comm *c, const swb_result *res, const int64_t *global_ids, int64_t n_local_refs,
+                             int32_t *merged_host);
 
 /* Integer / DPX issue-rate microbenchmark (roofline denominator, SURVEY.md 8d). */
 int swb_microbench_json(int device, int iters, char *buf, int buflen);

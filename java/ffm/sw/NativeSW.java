@@ -40,7 +40,11 @@ final class NativeSW
 	static final MethodHandle REFSET_FREE = h( "swb_refset_free" , FunctionDescriptor.ofVoid(ADDRESS) ) ;
 	static final MethodHandle ALIGN       = h( "swb_align" , FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS) ) ;
 	static final MethodHandle ALIGN_PAIR  = h( "swb_align_pair" , FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, JAVA_LONG, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS) ) ;
+	static final MethodHandle ALIGN_HITS  = h( "swb_align_hits" , FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS) ) ;
 	static final MethodHandle RESULT_FREE = h( "swb_result_free" , FunctionDescriptor.ofVoid(ADDRESS) ) ;
+	static final MethodHandle RESULT_HITS = h( "swb_result_hits" , FunctionDescriptor.of(ADDRESS, ADDRESS, ADDRESS) ) ;
+	static final MethodHandle MULTI_ALIGN_HITS = h( "swb_multi_align_hits" , FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS) ) ;
+	static final MethodHandle MULTI_RESULT_HITS = h( "swb_multi_result_hits" , FunctionDescriptor.of(ADDRESS, ADDRESS, ADDRESS) ) ;
 	static final MethodHandle SCORES      = h( "swb_result_scores" , FunctionDescriptor.of(ADDRESS, ADDRESS) ) ;
 	static final MethodHandle REF_TOTALS  = h( "swb_result_ref_totals" , FunctionDescriptor.of(ADDRESS, ADDRESS) ) ;
 	static final MethodHandle CELL_OFFS   = h( "swb_result_cell_offsets" , FunctionDescriptor.of(ADDRESS, ADDRESS) ) ;

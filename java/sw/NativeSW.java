@@ -35,12 +35,16 @@ final class NativeSW
 	static native long align( long ctx , long refset , byte[] readBytes , long[] readOffsets , int match , int mismatch , int gap , int flags ) ;
 	/** one pair through the native submission queue (swb_align_pair): concurrent calls are coalesced into one launch sequence */
 	static native long alignPair( long ctx , byte[] ref , byte[] read , int match , int mismatch , int gap , int flags ) ;
+	/** hits mode (swb_align_hits): every pair scored, only each read's topK best pairs with score >= minScore traced */
+	static native long alignHits( long ctx , long refset , byte[] readBytes , long[] readOffsets , int match , int mismatch , int gap , int flags , int topK , int minScore ) ;
 	static native void resultFree( long result ) ;
 
 	// ---- result arrays ---------------------------------------------------------------------
 	static native int[] scores( long result ) ;
 	static native int[] refTotals( long result ) ;
 	static native int[] bestHits( long result ) ;
+	/** hits mode: {score, ref, i, j} x topK per read, padding (0, -1, 0, 0); empty for a plain result */
+	static native int[] resultHits( long result ) ;
 	static native long[] cellOffsets( long result ) ;
 	static native int[] cells( long result ) ;
 	static native int[] beginnings( long result ) ;
@@ -55,8 +59,10 @@ final class NativeSW
 	static native void multiRefsetLoad( long multi , byte[] bytes , long[] offsets ) ;
 	static native long[] multiShardRefs( long multi , int shard ) ;
 	static native long multiAlign( long multi , byte[] readBytes , long[] readOffsets , int match , int mismatch , int gap , int flags ) ;
+	static native long multiAlignHits( long multi , byte[] readBytes , long[] readOffsets , int match , int mismatch , int gap , int flags , int topK , int minScore ) ;
 	static native long multiShard( long multiResult , int shard ) ;
 	static native int[] multiBestHits( long multiResult , int nReads ) ;
+	static native int[] multiResultHits( long multiResult , int nReads ) ;
 	static native void multiResultFree( long multiResult ) ;
 
 	static final int F_SCORES_ONLY = 1 , F_NO_FETCH = 2 , F_TIE_GT = 4 ;

@@ -87,6 +87,33 @@ JNIEXPORT jlong JNICALL Java_sw_NativeSW_align(JNIEnv *e, jclass c, jlong ctx, j
     if (rc) { throw_last(e, "swb_align"); return 0; }
     return (jlong)(intptr_t)res;
 }
+/* ---- hits mode: every pair scored, only each read's topK best pairs (score >= minScore) traced (swb_align_hits) ---- */
+JNIEXPORT jlong JNICALL Java_sw_NativeSW_alignHits(JNIEnv *e, jclass c, jlong ctx, jlong refset, jbyteArray readBytes,
+                                                   jlongArray readOffsets, jint match, jint mismatch, jint gap, jint flags,
+                                                   jint topK, jint minScore)
+{
+    (void)c;
+    const jsize n = (*e)->GetArrayLength(e, readOffsets) - 1;
+    jlong *o = (jlong *)(*e)->GetPrimitiveArrayCritical(e, readOffsets, 0);
+    jbyte *b = (jbyte *)(*e)->GetPrimitiveArrayCritical(e, readBytes, 0);
+    swb_result *res = 0;
+    const int rc = swb_align_hits(H(swb_ctx, ctx), H(swb_refset, refset), n, (const char *)b, (const int64_t *)o, match, mismatch,
+                                  gap, (uint32_t)flags, topK, minScore, &res);
+    (*e)->ReleasePrimitiveArrayCritical(e, readBytes, b, JNI_ABORT);
+    (*e)->ReleasePrimitiveArrayCritical(e, readOffsets, o, JNI_ABORT);
+    if (rc) { throw_last(e, "swb_align_hits"); return 0; }
+    return (jlong)(intptr_t)res;
+}
+/* {score, ref, i, j} x k per read of a hits-mode result; empty for a plain one */
+JNIEXPORT jintArray JNICALL Java_sw_NativeSW_resultHits(JNIEnv *e, jclass c, jlong res)
+{
+    (void)c;
+    const swb_result *r = H(swb_result, res);
+    int32_t k = 0;
+    const int32_t *h = swb_result_hits(r, &k);
+    return ints(e, h, h ? swb_result_n_reads(r) * k * 4 : 0);
+}
+
 /* ---- one pair through the submission queue: the unchanged driver's per-pair OptAlignments.call (Distribution.java:419-426).
  * The call may wait for other threads' requests, so the bytes are copied out instead of held critical. */
 JNIEXPORT jlong JNICALL Java_sw_NativeSW_alignPair(JNIEnv *e, jclass c, jlong ctx, jbyteArray ref, jbyteArray read, jint match,
@@ -238,6 +265,21 @@ JNIEXPORT jlong JNICALL Java_sw_NativeSW_multiAlign(JNIEnv *e, jclass c, jlong m
     if (rc) { throw_last(e, "swb_multi_align"); return 0; }
     return (jlong)(intptr_t)res;
 }
+JNIEXPORT jlong JNICALL Java_sw_NativeSW_multiAlignHits(JNIEnv *e, jclass c, jlong m, jbyteArray readBytes, jlongArray readOffsets,
+                                                        jint match, jint mismatch, jint gap, jint flags, jint topK, jint minScore)
+{
+    (void)c;
+    const jsize n = (*e)->GetArrayLength(e, readOffsets) - 1;
+    jlong *o = (jlong *)(*e)->GetPrimitiveArrayCritical(e, readOffsets, 0);
+    jbyte *b = (jbyte *)(*e)->GetPrimitiveArrayCritical(e, readBytes, 0);
+    swb_multi_result *res = 0;
+    const int rc = swb_multi_align_hits(H(swb_multi, m), n, (const char *)b, (const int64_t *)o, match, mismatch, gap, (uint32_t)flags,
+                                        topK, minScore, &res);
+    (*e)->ReleasePrimitiveArrayCritical(e, readBytes, b, JNI_ABORT);
+    (*e)->ReleasePrimitiveArrayCritical(e, readOffsets, o, JNI_ABORT);
+    if (rc) { throw_last(e, "swb_multi_align_hits"); return 0; }
+    return (jlong)(intptr_t)res;
+}
 JNIEXPORT jlong JNICALL Java_sw_NativeSW_multiShard(JNIEnv *e, jclass c, jlong mres, jint shard)
 {
     (void)e; (void)c;
@@ -247,5 +289,13 @@ JNIEXPORT jintArray JNICALL Java_sw_NativeSW_multiBestHits(JNIEnv *e, jclass c, 
 {
     (void)c;
     return ints(e, swb_multi_result_best_hits(H(swb_multi_result, mres)), (int64_t)nReads * 4);
+}
+/* merged {score, global ref, i, j} x k per read of a hits-mode multi result; empty for a plain one */
+JNIEXPORT jintArray JNICALL Java_sw_NativeSW_multiResultHits(JNIEnv *e, jclass c, jlong mres, jint nReads)
+{
+    (void)c;
+    int32_t k = 0;
+    const int32_t *h = swb_multi_result_hits(H(swb_multi_result, mres), &k);
+    return ints(e, h, h ? (int64_t)nReads * k * 4 : 0);
 }
 JNIEXPORT void JNICALL Java_sw_NativeSW_multiResultFree(JNIEnv *e, jclass c, jlong mres) { (void)e; (void)c; swb_multi_result_free(H(swb_multi_result, mres)); }

@@ -155,7 +155,7 @@ void swb_destroy(swb_ctx *c)
     c->v_ref.release(); c->v_c0.release(); c->v_len.release(); c->v_skip.release(); c->v_end.release();
     c->w_brow.release(); c->w_rec.release(); c->w_wreads.release(); c->w_rpad.release(); c->w_rpad_off.release(); c->w_rpad_len.release(); c->w_dbg.release(); c->w_mail.release(); c->w_tmx.release(); c->w_prog.release(); c->w_pair_ref.release();
     c->w_pair_read.release(); c->w_band_off.release(); c->w_blk_off.release(); c->w_brow_off.release();
-    c->w_items.release(); c->w_tasks.release();
+    c->w_items.release(); c->w_tasks.release(); c->hit_tmp.release(); c->hit_sel.release();
     for (cudaEvent_t e : c->ev_pool) cudaEventDestroy(e);
     for (auto &b : c->pin_free) cudaFreeHost(b.p);
     cudaStreamSynchronize(c->stream);
@@ -478,9 +478,11 @@ static int pick_k(int m)
 }
 
 // One packed set (a whole small set, or one part of a large one).  ext_scores / ext_totals: rows of the parent's
-// score matrix / totals this part writes into (nullptr: own arrays).
+// score matrix / totals this part writes into (nullptr: own arrays).  top_k > 0: hits mode (swb_align_hits) -- only the
+// pairs of each read's top k and its best pair are traced, and only the top k's cells are kept.
 static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
-                      int32_t gap, uint32_t flags, int32_t *ext_scores, int32_t *ext_totals, swb_result **out)
+                      int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, int32_t *ext_scores, int32_t *ext_totals,
+                      swb_result **out)
 {
     if (!ctx || !rs || !rd || !out) return fail(SWB_E_INVALID, "swb_align: null argument");
     *out = nullptr;
@@ -526,6 +528,17 @@ static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, i
     if (ext_totals) res->d_totals.view(ext_totals, (size_t)n_refs); else CU(res->d_totals.alloc((size_t)n_refs, st));
     CU(res->d_best.alloc((size_t)n_reads * 4, st));
     CU(cudaMemsetAsync(res->d_scores.p, 0, std::max<size_t>(n_pairs, 1) * 4, st));
+    res->top_k = top_k; res->min_score = min_score;
+    if (top_k > 0) CU(res->d_hits.alloc((size_t)n_reads * top_k * 4, st));
+    // hits mode: top k + best pair of the reads `slots` (score rows exact by now) -> `bits` / `hits` (swb_hits.cu)
+    auto select_hits = [&](const int32_t *slots, int64_t n_slots, int with_best, int4 *hits, uint32_t *bits, int64_t bit_slot,
+                      int64_t bit_ref) -> cudaError_t {
+        const size_t te = select_hits_tmp_elems(n_refs, n_slots, top_k);
+        cudaError_t e = ctx->hit_tmp.reserve(te, st);
+        if (e == cudaSuccess) e = launch_select_hits(res->d_scores.p, n_refs, n_reads, slots, n_slots, top_k, min_score, with_best,
+                                                     hits, bits, bit_slot, bit_ref, ctx->hit_tmp.p, te, st);
+        return e;
+    };
 
     const auto t_wall0 = std::chrono::steady_clock::now();
     const bool tlh = getenv("SWB_TIMELINE_HOST") != nullptr;
@@ -663,7 +676,7 @@ static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, i
                 P.read_codes = rd->codes.p; P.read_off = rd->off.p; P.rp_reads = rpb.p; P.read_slot = nullptr;
                 P.n_rp = S.n_rp; P.n_reads = n_reads;
                 P.match = match; P.mismatch = mismatch; P.gap = gap; P.tie_gt = (flags & SWB_F_TIE_GT) ? 1 : 0;
-                P.scores = res->d_scores.p; P.rec = ck.p; P.tmx = tmx.p;
+                P.scores = res->d_scores.p; P.rec = ck.p; P.tmx = tmx.p; P.sel = nullptr;
                 uint32_t *d_work = ctx->counters.p + 4 + S.buf;
                 const bool biased = fill_bias_ok(match, mismatch, gap, (int64_t)std::max({match, mismatch, 0}) * std::min<int64_t>(S.m_max, rs->max_len));
                 P.seam_bias = biased ? -gap : 0;               // the biased fill stores its seams biased
@@ -683,10 +696,17 @@ static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, i
 
             auto trace_stage = [&](int64_t k) -> int {
                 Stage &S = stages[(size_t)k];
+                const bool scores_only = (flags & SWB_F_SCORES_ONLY) != 0;
+                // hits mode: the scan makes the batch's score rows exact, the selection marks the pairs the emit keeps
+                const bool hits_sel = top_k > 0 && !scores_only;
+                const size_t sel_words = ((size_t)S.n_rp * 2 * (size_t)n_refs + 31) / 32;
+                if (hits_sel) {
+                    CU(ctx->hit_sel.reserve(sel_words, st));
+                    S.P.sel = ctx->hit_sel.p;
+                }
                 const BatchParams &P = S.P;
                 const int n_rp = S.n_rp;
                 if (sF != st) CU(cudaStreamWaitEvent(st, S.ev_fill, 0));
-                const bool scores_only = (flags & SWB_F_SCORES_ONLY) != 0;
                 if (scores_only && P.tmx_slack == 0) return SWB_OK;      // the fill's pair scores are exact
                 uint32_t *d_ntasks = ctx->counters.p, *d_ncells = ctx->counters.p + 1;
                 // ---- candidate tiles -> exact scores + max cells -> sorted keys (one host sync: the two counts) ----
@@ -704,6 +724,13 @@ static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, i
                     CU(launch_locate(K, P, ctx->tasks.p, d_ntasks, cap_tasks, ctx->task_hits.p, ctx->keys_tmp.p, cap_cells, d_ncells,
                                      ctx->sm_count, 0, st));
                     launches += 2;
+                    if (hits_sel) {
+                        const int sp_sel = tic(5, st);
+                        CU(cudaMemsetAsync(ctx->hit_sel.p, 0, sel_words * 4, st));
+                        CU(select_hits(P.rp_reads, (int64_t)n_rp * 2, 1, nullptr, ctx->hit_sel.p, n_refs, 1));
+                        CU(toc(sp_sel, st));
+                        launches += 2;
+                    }
                     if (!scores_only) {
                         CU(launch_locate(K, P, ctx->tasks.p, d_ntasks, cap_tasks, ctx->task_hits.p, ctx->keys_tmp.p, cap_cells, d_ncells,
                                          ctx->sm_count, 1, st));
@@ -788,9 +815,50 @@ static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, i
         }
     }
     if (n_refs > 0 && !wide_reads_all.empty()) {
-        int rc = run_wide_path(ctx, rs, rd, wide_reads_all, match, mismatch, gap, flags, res.get(), &launches, &n_batches,
-                               &ck_bytes, tic1, toc1);
-        if (rc) return rc;
+        if (top_k > 0 && !(flags & SWB_F_SCORES_ONLY)) {
+            // hits mode: exact scores of every wide pair first, then the whole wide path over each read's top k + best pair
+            int rc = run_wide_path(ctx, rs, rd, wide_reads_all, match, mismatch, gap, flags | SWB_F_SCORES_ONLY, res.get(), &launches,
+                                   &n_batches, &ck_bytes, tic1, toc1);
+            if (rc) return rc;
+            const int64_t nw = (int64_t)wide_reads_all.size();
+            DevBuf<int32_t> d_wr;
+            CU(d_wr.alloc((size_t)nw, st));
+            CU(cudaMemcpyAsync(d_wr.p, wide_reads_all.data(), (size_t)nw * 4, cudaMemcpyHostToDevice, st));
+            const int sp_sel = tic(5, st);
+            int4 *d_sel = reinterpret_cast<int4 *>(res->d_hits.p);              // scratch here: the final selection rewrites it
+            CU(select_hits(d_wr.p, nw, 1, d_sel, nullptr, 0, 0));
+            CU(toc(sp_sel, st));
+            launches += 2;
+            std::vector<int4> h_sel((size_t)nw * top_k);
+            CU(cudaMemcpyAsync(h_sel.data(), d_sel, h_sel.size() * sizeof(int4), cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            std::vector<std::vector<int32_t>> refs_of((size_t)nw);
+            for (int64_t x = 0; x < nw; ++x) {
+                for (int h = 0; h < top_k; ++h)
+                    if (h_sel[(size_t)(x * top_k + h)].y >= 0) refs_of[(size_t)x].push_back(h_sel[(size_t)(x * top_k + h)].y);
+                std::sort(refs_of[(size_t)x].begin(), refs_of[(size_t)x].end());
+            }
+            rc = run_wide_path(ctx, rs, rd, wide_reads_all, match, mismatch, gap, flags, res.get(), &launches, &n_batches, &ck_bytes,
+                               tic1, toc1, &refs_of);
+            if (rc) return rc;
+        } else {
+            int rc = run_wide_path(ctx, rs, rd, wide_reads_all, match, mismatch, gap, flags, res.get(), &launches, &n_batches,
+                                   &ck_bytes, tic1, toc1);
+            if (rc) return rc;
+        }
+    }
+    // hits mode: the final lists (every score is exact now) and, with cells, the pairs whose cells the assembly keeps
+    DevBuf<uint32_t> keep;
+    if (top_k > 0) {
+        const bool with_cells = !(flags & SWB_F_SCORES_ONLY);
+        if (with_cells) {
+            CU(keep.alloc((n_pairs + 31) / 32, st));
+            CU(cudaMemsetAsync(keep.p, 0, ((n_pairs + 31) / 32) * 4, st));
+        }
+        const int sp_sel = tic(5, st);
+        CU(select_hits(nullptr, n_reads, 0, reinterpret_cast<int4 *>(res->d_hits.p), keep.p, 1, n_reads));
+        CU(toc(sp_sel, st));
+        launches += 2;
     }
     const int sp_misc = tic(4, st);
     CU(launch_ref_totals(res->d_scores.p, n_refs, n_reads, res->d_totals.p, st));
@@ -841,24 +909,38 @@ static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, i
         }
         if (!descs.empty()) CU(cudaMemcpyAsync(d_desc.p, descs.data(), descs.size() * sizeof(BatchDesc), cudaMemcpyHostToDevice, st));
         int pair_bits = 1;
-        while (pair_bits < 64 && ((uint64_t)1 << pair_bits) < (uint64_t)std::max<size_t>(n_pairs, 1)) ++pair_bits;
-        CU(assemble_sort(d_desc.p, (int)descs.size(), N, n_refs, n_reads, d_pair_tmp.p, d_src_tmp.p, d_pair_sorted.p, d_order.p,
+        const uint64_t key_end = keep.p ? 2 * (uint64_t)n_pairs : (uint64_t)n_pairs;    // hits mode: dropped cells sort as p + n_pairs
+        while (pair_bits < 64 && ((uint64_t)1 << pair_bits) < std::max<uint64_t>(key_end, 1)) ++pair_bits;
+        CU(assemble_sort(d_desc.p, (int)descs.size(), N, n_refs, n_reads, keep.p, d_pair_tmp.p, d_src_tmp.p, d_pair_sorted.p, d_order.p,
                          d_tmp.p, tmp_bytes, pair_bits, st));
-        CU(cudaMemsetAsync(d_words.p + N, 0, 8, st));
-        CU(assemble_gather_cells(d_desc.p, (int)descs.size(), N, d_order.p, res->f_cells.p, res->f_beg.p, res->f_len.p,
+        uint32_t NK = N;                          // cells that stay: all of them, or in hits mode those of the hits
+        if (keep.p) {
+            CU(assemble_kept_count(d_pair_sorted.p, N, (int64_t)n_pairs, ctx->counters.p + 2, st));
+            CU(cudaMemcpyAsync(&NK, ctx->counters.p + 2, 4, cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            res->total_cells = NK;
+            res->stats[8] = NK;
+        }
+        CU(cudaMemsetAsync(d_words.p + NK, 0, 8, st));
+        CU(assemble_gather_cells(d_desc.p, (int)descs.size(), NK, d_order.p, res->f_cells.p, res->f_beg.p, res->f_len.p,
                                  d_words.p, res->f_ops_off.p, d_tmp.p, tmp_bytes, st));
         int64_t total_words = 0;
         mark("assemble sort + cells issued");
-        CU(cudaMemcpyAsync(&total_words, res->f_ops_off.p + N, 8, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(&total_words, res->f_ops_off.p + NK, 8, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         mark("total words on the host");
         if (tl4) fprintf(stderr, "[swb assemble] sort + cell gather done at %.3f ms\n", ms4());
         res->total_words = total_words;
         CU(res->f_ops.alloc((size_t)total_words, st));
         if (tl4) fprintf(stderr, "[swb assemble] ops array (%lld words) allocated at %.3f ms\n", (long long)total_words, ms4());
-        CU(assemble_gather_ops(d_desc.p, (int)descs.size(), N, d_order.p, res->f_ops_off.p, res->f_ops.p, st));
-        CU(assemble_offsets(d_pair_sorted.p, N, (int64_t)n_pairs, res->f_cell_off.p, res->d_best.p, n_reads, res->f_cells.p, st));
+        CU(assemble_gather_ops(d_desc.p, (int)descs.size(), NK, d_order.p, res->f_ops_off.p, res->f_ops.p, st));
+        CU(assemble_offsets(d_pair_sorted.p, NK, (int64_t)n_pairs, res->f_cell_off.p, res->d_best.p, n_reads, res->f_cells.p, st));
         launches += 8;
+        if (keep.p) {
+            CU(assemble_hit_cells(d_desc.p, (int)descs.size(), d_pair_sorted.p, d_order.p, N, (int64_t)n_pairs, n_reads, res->f_cell_off.p,
+                                  res->f_cells.p, res->d_best.p, res->d_hits.p, top_k, st));
+            launches += 2;
+        }
         CU(toc(sp_misc, st));
         CU(cudaStreamSynchronize(st));
         mark("assembled (sync)");
@@ -869,7 +951,7 @@ static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, i
         CU(toc(sp_misc, st));
         CU(cudaStreamSynchronize(st));
     }
-    double t_phase[5] = {0, 0, 0, 0, 0};
+    double t_phase[6] = {0, 0, 0, 0, 0, 0};
     if (getenv("SWB_TIMELINE") && !spans.empty())
         for (const Span &sp : spans) {
             float a = 0, b = 0;
@@ -889,7 +971,7 @@ static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, i
     res->stats[5] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_wall0).count();   // wall: phases overlap
     res->stats[6] = (double)rs->total_bases * (double)read_bases;
     res->stats[7] = (double)n_refs * (double)n_reads;
-    res->stats[9] = launches; res->stats[10] = ck_bytes; res->stats[11] = n_batches;
+    res->stats[9] = launches; res->stats[10] = ck_bytes; res->stats[11] = n_batches; res->stats[12] = t_phase[5];
     swb_result *r = res.release();
     mark("before fetch");
     if (!(flags & SWB_F_NO_FETCH)) {
@@ -1032,15 +1114,24 @@ int finish_parts_fetch(swb_result *res)
 
 }  // namespace
 
-int swb_align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
-                       int32_t gap, uint32_t flags, swb_result **out)
+static int check_hits_args(const char *who, int32_t top_k, int32_t min_score)
+{
+    if (top_k < 1 || top_k > 32) return fail(SWB_E_INVALID, std::string(who) + ": top_k must be 1 .. 32");
+    if (min_score < 1) return fail(SWB_E_INVALID, std::string(who) + ": min_score must be >= 1");
+    return SWB_OK;
+}
+
+static int align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
+                          int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_result **out)
 {
     if (!ctx || !rs || !rd || !out) return fail(SWB_E_INVALID, "swb_align: null argument");
     *out = nullptr;
     if (rs->parent) return fail(SWB_E_INVALID, "swb_align: a part of a reference set is not a handle");
-    if (rs->parts.empty()) return align_leaf(ctx, rs, rd, match, mismatch, gap, flags, nullptr, nullptr, out);
-    if (rs->whole && (flags & (SWB_F_NO_FETCH | SWB_F_SCORES_ONLY)))
-        return align_leaf(ctx, rs->whole, rd, match, mismatch, gap, flags, nullptr, nullptr, out);
+    if (rs->parts.empty()) return align_leaf(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, nullptr, nullptr, out);
+    // hits mode also runs on the set as one: its cell arrays are small (nothing to overlap), and the selection is then
+    // over all references at once, so no part keeps cells of a pair that a later part displaces from the top k
+    if (rs->whole && ((flags & (SWB_F_NO_FETCH | SWB_F_SCORES_ONLY)) || top_k > 0))
+        return align_leaf(ctx, rs->whole, rd, match, mismatch, gap, flags, top_k, min_score, nullptr, nullptr, out);
     // ---- a set of several parts: part by part; part k's results cross PCIe while part k + 1 computes -------------
     if (rd->rs != rs) return fail(SWB_E_INVALID, "swb_align: reads were encoded against a different reference set");
     if (rs->ctx != ctx || rd->ctx != ctx) return fail(SWB_E_INVALID, "swb_align: handles belong to another context");
@@ -1069,7 +1160,7 @@ int swb_align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, 
         const int64_t first = rs->part_first[k];
         swb_result *sub = nullptr;
         if (timeline) fprintf(stderr, "[swb parts] part %zu starts at %.3f ms (pinned allocations so far %lld)\n", k, wall_ms(), (long long)ctx->pin_allocs);
-        const int rc = align_leaf(ctx, part, rd, match, mismatch, gap, flags | SWB_F_NO_FETCH, res->d_scores.p + (size_t)first * (size_t)n_reads,
+        const int rc = align_leaf(ctx, part, rd, match, mismatch, gap, flags | SWB_F_NO_FETCH, 0, 1, res->d_scores.p + (size_t)first * (size_t)n_reads,
                                   res->d_totals.p + first, &sub);
         if (rc) return rc;
         res->subs.push_back(sub); res->sub_first.push_back(first); res->sub_copied.push_back(0);
@@ -1096,8 +1187,23 @@ int swb_align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, 
     return SWB_OK;
 }
 
-int swb_align(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
-              int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, swb_result **out)
+int swb_align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
+                       int32_t gap, uint32_t flags, swb_result **out)
+{
+    return align_resident(ctx, rs, rd, match, mismatch, gap, flags, 0, 1, out);
+}
+
+int swb_align_resident_hits(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
+                            int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_result **out)
+{
+    if (out) *out = nullptr;
+    const int rc = check_hits_args("swb_align_resident_hits", top_k, min_score);
+    if (rc) return rc;
+    return align_resident(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, out);
+}
+
+static int align_host(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
+                      int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_result **out)
 {
     if (!out) return fail(SWB_E_INVALID, "swb_align: out is null");
     *out = nullptr;
@@ -1114,10 +1220,25 @@ int swb_align(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *r
     float h2d = 0;
     cudaEventElapsedTime(&h2d, e0, e1);
     cudaEventDestroy(e0); cudaEventDestroy(e1);
-    rc = swb_align_resident(ctx, rs, rd, match, mismatch, gap, flags, out);
+    rc = align_resident(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, out);
     swb_reads_free(rd);
     if (rc == SWB_OK) (*out)->stats[0] = h2d;
     return rc;
+}
+
+int swb_align(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
+              int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, swb_result **out)
+{
+    return align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, 1, out);
+}
+
+int swb_align_hits(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
+                   int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_result **out)
+{
+    if (out) *out = nullptr;
+    const int rc = check_hits_args("swb_align_hits", top_k, min_score);
+    if (rc) return rc;
+    return align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, top_k, min_score, out);
 }
 
 int swb_result_fetch(swb_result *res)
@@ -1146,6 +1267,7 @@ int swb_result_fetch(swb_result *res)
     if ((rc = pull(res->d_scores.p, n_pairs * 4, (const void **)&res->scores))) return rc;
     if ((rc = pull(res->d_totals.p, (size_t)res->n_refs * 4, (const void **)&res->totals))) return rc;
     if ((rc = pull(res->d_best.p, (size_t)res->n_reads * 16, (const void **)&res->best))) return rc;
+    if (res->top_k > 0 && (rc = pull(res->d_hits.p, (size_t)res->n_reads * res->top_k * 16, (const void **)&res->hits))) return rc;
     if (full) {
         if ((rc = pull(res->f_cell_off.p, (n_pairs + 1) * 8, (const void **)&res->cell_off))) return rc;
         if ((rc = pull(res->f_cells.p, N * 8, (const void **)&res->cells))) return rc;
@@ -1185,6 +1307,11 @@ int64_t swb_result_n_reads(const swb_result *r) { return r ? r->n_reads : 0; }
 const int32_t *swb_result_scores(const swb_result *r) { return (r && r->fetched) ? r->scores : nullptr; }
 const int32_t *swb_result_ref_totals(const swb_result *r) { return (r && r->fetched) ? r->totals : nullptr; }
 const int32_t *swb_result_best_hits(const swb_result *r) { return (r && r->fetched) ? r->best : nullptr; }
+const int32_t *swb_result_hits(const swb_result *r, int32_t *top_k)
+{
+    if (top_k) *top_k = r ? r->top_k : 0;
+    return (r && r->fetched && r->top_k > 0) ? r->hits : nullptr;
+}
 const int64_t *swb_result_cell_offsets(const swb_result *r) { return (r && r->fetched) ? r->cell_off : nullptr; }
 int64_t swb_result_total_cells(const swb_result *r) { return r ? (int64_t)r->total_cells : 0; }
 const int32_t *swb_result_cells(const swb_result *r) { return (r && r->fetched) ? r->cells : nullptr; }
@@ -1195,7 +1322,7 @@ int64_t swb_result_pair_cell_count(const swb_result *r, int64_t pair)
 {
     if (!r || !r->fetched || pair < 0 || pair >= r->n_refs * r->n_reads) return -1;
     if (r->flags & SWB_F_SCORES_ONLY) return -1;
-    if (r->scores[(size_t)pair] == 0) {
+    if (r->scores[(size_t)pair] == 0 && r->top_k == 0) {      // hits mode: a score-0 pair is never a hit, its range is empty
         const int64_t ref = pair / r->n_reads, rd = pair % r->n_reads;
         return (int64_t)r->ref_len[(size_t)ref] * r->read_len[(size_t)rd];     // every cell ties at 0
     }
@@ -1208,7 +1335,7 @@ int swb_result_pair_cell(const swb_result *r, int64_t pair, int64_t k, int32_t *
     const int64_t cnt = swb_result_pair_cell_count(r, pair);
     if (cnt < 0) return fail(SWB_E_RANGE, "swb_result_pair_cell: bad pair");
     if (k < 0 || k >= cnt) return fail(SWB_E_RANGE, "swb_result_pair_cell: bad cell index");
-    if (r->scores[(size_t)pair] == 0) {
+    if (r->scores[(size_t)pair] == 0 && r->top_k == 0) {
         const int64_t n = r->ref_len[(size_t)(pair / r->n_reads)];
         if (i) *i = (int32_t)(k / n + 1);
         if (j) *j = (int32_t)(k % n + 1);
@@ -1265,7 +1392,7 @@ int swb_result_materialize(const swb_result *r, int64_t cell, const char *ref, i
 int swb_result_stats(const swb_result *r, double *outp, int n)
 {
     if (!r || !outp) return fail(SWB_E_INVALID, "swb_result_stats: null");
-    for (int k = 0; k < n && k < 12; ++k) outp[k] = r->stats[k];
+    for (int k = 0; k < n && k < 13; ++k) outp[k] = r->stats[k];
     return SWB_OK;
 }
 

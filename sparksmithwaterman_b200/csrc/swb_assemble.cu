@@ -20,8 +20,9 @@ __device__ __forceinline__ int find_batch(const BatchDesc *b, int nb, uint32_t s
     return lo;
 }
 
+// keep (hits mode): cells of pairs without their bit sort after every kept cell, as pair + n_pairs
 __global__ void cell_pairs_kernel(const BatchDesc *batches, int nb, uint32_t n_cells, int64_t n_refs, int64_t n_reads,
-                                  uint64_t *pair_of, uint32_t *src)
+                                  const uint32_t *keep, uint64_t *pair_of, uint32_t *src)
 {
     const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n_cells) return;
@@ -34,6 +35,7 @@ __global__ void cell_pairs_kernel(const BatchDesc *batches, int nb, uint32_t n_c
         const uint64_t slot = pk / (uint64_t)n_refs, ref = pk - slot * (uint64_t)n_refs;
         p = ref * (uint64_t)n_reads + (uint64_t)B.slot_read[slot];
     }
+    if (keep && !((keep[p >> 5] >> (p & 31)) & 1u)) p += (uint64_t)n_refs * (uint64_t)n_reads;
     pair_of[k] = p;
     src[k] = k;
 }
@@ -94,6 +96,45 @@ __global__ void best_cells_kernel2(int32_t *best, int64_t n_reads, const int64_t
     }
 }
 
+__device__ __forceinline__ uint32_t lower_bound_u64(const uint64_t *a, uint32_t n, uint64_t v)
+{
+    uint32_t lo = 0, hi = n;
+    while (lo < hi) { const uint32_t mid = lo + ((hi - lo) >> 1); if (a[mid] < v) lo = mid + 1; else hi = mid; }
+    return lo;
+}
+
+__global__ void kept_count_kernel(const uint64_t *pair_sorted, uint32_t n_cells, int64_t n_pairs, uint32_t *n_kept)
+{
+    *n_kept = lower_bound_u64(pair_sorted, n_cells, (uint64_t)n_pairs);
+}
+
+// hits mode, thread per read: (i, j) of every hit = its pair's first kept cell; a best hit that is not a hit (score below
+// min_score) takes the first of its pair's dropped cells, which sort as pair + n_pairs
+__global__ void hit_cells_kernel(const BatchDesc *batches, int nb, const uint64_t *pair_sorted, const uint32_t *order,
+                                 uint32_t n_all, int64_t n_pairs, int64_t n_reads, const int64_t *cell_off, const int32_t *cells,
+                                 int32_t *best, int32_t *hits, int k)
+{
+    const int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (q >= n_reads) return;
+    for (int h = 0; h < k; ++h) {
+        int32_t *e = hits + (q * k + h) * 4;
+        if (e[1] < 0) break;
+        const int64_t p = (int64_t)e[1] * n_reads + q;
+        if (cell_off[p + 1] > cell_off[p]) { e[2] = cells[2 * cell_off[p]]; e[3] = cells[2 * cell_off[p] + 1]; }
+    }
+    const int ref = best[4 * q + 1];
+    if (ref < 0 || best[4 * q] <= 0) return;
+    const int64_t p = (int64_t)ref * n_reads + q;
+    if (cell_off[p + 1] > cell_off[p]) return;                    // a hit: best_cells_kernel2 has its cell
+    const uint32_t c = lower_bound_u64(pair_sorted, n_all, (uint64_t)(p + n_pairs));
+    if (c >= n_all || pair_sorted[c] != (uint64_t)(p + n_pairs)) return;
+    const uint32_t s = order[c];
+    const BatchDesc &B = batches[find_batch(batches, nb, s)];
+    const uint64_t key = B.keys[s - B.base];
+    best[4 * q + 2] = (int32_t)(B.wide ? wide::wide_key_i(key) : key_i(key));
+    best[4 * q + 3] = (int32_t)(B.wide ? wide::wide_key_j(key) : key_j(key));
+}
+
 size_t assemble_tmp_bytes(uint32_t n_cells)
 {
     size_t a = 0, b = 0;
@@ -104,12 +145,12 @@ size_t assemble_tmp_bytes(uint32_t n_cells)
 }
 
 cudaError_t assemble_sort(const BatchDesc *batches, int nb, uint32_t n_cells, int64_t n_refs, int64_t n_reads,
-                          uint64_t *pair_tmp, uint32_t *src_tmp, uint64_t *pair_sorted, uint32_t *order, void *tmp,
+                          const uint32_t *keep, uint64_t *pair_tmp, uint32_t *src_tmp, uint64_t *pair_sorted, uint32_t *order, void *tmp,
                           size_t tmp_bytes, int pair_bits, cudaStream_t st)
 {
     if (n_cells == 0) return cudaSuccess;
     const int threads = 256;
-    cell_pairs_kernel<<<(n_cells + threads - 1) / threads, threads, 0, st>>>(batches, nb, n_cells, n_refs, n_reads, pair_tmp, src_tmp);
+    cell_pairs_kernel<<<(n_cells + threads - 1) / threads, threads, 0, st>>>(batches, nb, n_cells, n_refs, n_reads, keep, pair_tmp, src_tmp);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     return cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, pair_tmp, pair_sorted, src_tmp, order, (int)n_cells, 0, pair_bits, st);
@@ -148,6 +189,27 @@ cudaError_t assemble_offsets(const uint64_t *pair_sorted, uint32_t n_cells, int6
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess || n_reads == 0) return e;
     best_cells_kernel2<<<(unsigned)((n_reads + threads - 1) / threads), threads, 0, st>>>(best, n_reads, cell_off, cells);
+    return cudaGetLastError();
+}
+
+}  // namespace swb
+
+namespace swb {
+
+cudaError_t assemble_kept_count(const uint64_t *pair_sorted, uint32_t n_cells, int64_t n_pairs, uint32_t *n_kept, cudaStream_t st)
+{
+    kept_count_kernel<<<1, 1, 0, st>>>(pair_sorted, n_cells, n_pairs, n_kept);
+    return cudaGetLastError();
+}
+
+cudaError_t assemble_hit_cells(const BatchDesc *batches, int nb, const uint64_t *pair_sorted, const uint32_t *order, uint32_t n_all,
+                               int64_t n_pairs, int64_t n_reads, const int64_t *cell_off, const int32_t *cells, int32_t *best,
+                               int32_t *hits, int k, cudaStream_t st)
+{
+    if (n_reads == 0) return cudaSuccess;
+    const int threads = 256;
+    hit_cells_kernel<<<(unsigned)((n_reads + threads - 1) / threads), threads, 0, st>>>(batches, nb, pair_sorted, order, n_all, n_pairs,
+                                                                                      n_reads, cell_off, cells, best, hits, k);
     return cudaGetLastError();
 }
 

@@ -167,6 +167,9 @@ struct swb_ctx {
     DevBuf<int64_t> w_band_off, w_blk_off, w_brow_off;
     DevBuf<int2> w_items;
     DevBuf<WideTask> w_tasks;
+    // hits mode (swb_hits.cu): partial top-k lists, the selection bits of one batch
+    DevBuf<uint64_t> hit_tmp;
+    DevBuf<uint32_t> hit_sel;
     // pinned host buffers, recycled between results (cudaHostAlloc is slow; D2H into pageable memory too)
     struct PinBuf { void *p = nullptr; size_t bytes = 0; };
     std::vector<PinBuf> pin_free;
@@ -270,6 +273,9 @@ struct swb_result {
     bool fetched = false;
     std::vector<int32_t> ref_len, read_len;
     DevBuf<int32_t> d_scores, d_totals, d_best;
+    int32_t top_k = 0, min_score = 1;            // hits mode (swb_align_hits): k > 0
+    DevBuf<int32_t> d_hits;                      // [n_reads][k][4] (score, ref, i, j)
+    const int32_t *hits = nullptr;               // host view after fetch
     std::vector<BatchOut> batches;               // released once the result is assembled
     // assembled on the device (swb_assemble.cu), ABI order
     uint32_t total_cells = 0;
@@ -283,7 +289,7 @@ struct swb_result {
     const int64_t *cell_off = nullptr, *ops_off = nullptr;
     const int32_t *cells = nullptr, *beginnings = nullptr, *op_lens = nullptr;
     const uint32_t *ops = nullptr;
-    double stats[12] = {0};
+    double stats[13] = {0};
     std::vector<char> own;                      // host arrays of a 1 x 1 result cut out of a coalesced batch (swb_queue.cu)
     // result of a multi-part reference set: one sub-result per part (device arrays), stitched into the host arrays
     std::vector<swb_result *> subs;
@@ -298,7 +304,9 @@ struct swb_result {
 
 #include <functional>
 namespace swbh {
+// refs_of (nullable): refs_of[k] = the references (ascending) read reads[k] is aligned against; nullptr = all of them
 int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const std::vector<int32_t> &reads,
                   int match, int mismatch, int gap, uint32_t flags, swb_result *res, int *launches, int *n_batches,
-                  double *ck_bytes, const std::function<cudaError_t(int)> &tic, const std::function<cudaError_t()> &toc);
+                  double *ck_bytes, const std::function<cudaError_t(int)> &tic, const std::function<cudaError_t()> &toc,
+                  const std::vector<std::vector<int32_t>> *refs_of = nullptr);
 }

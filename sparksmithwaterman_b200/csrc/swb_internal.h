@@ -116,6 +116,8 @@ struct BatchParams {
     uint32_t *tmx;                  // tile maxima  [n_rp][blocks_per_rp][GL]
     int32_t tmx_slack;              // 0: tile maxima / pair scores of the fill are exact; > 0: subsampled, true max - slack <= tmx <= true max
     int32_t seam_bias;              // seam word of step u, lane t = H + seam_bias * (9 - t + u) (biased fill), 0 = plain
+    const uint32_t *sel;            // hits mode: bit rp_half * n_refs + ref_orig = the pair is selected, only those emit
+                                    // max cells; nullptr = every pair emits
 };
 
 // ---- general ("wide") int32 path: bands of 32 lanes x KL rows, see swb_wide.cu ------------------
@@ -177,8 +179,9 @@ struct BatchDesc {
     int32_t wide;
 };
 size_t      assemble_tmp_bytes(uint32_t n_cells);
+// keep (nullable): hits mode, bit p of the ABI pairs whose cells stay; the others sort after them as p + n_pairs
 cudaError_t assemble_sort(const BatchDesc *batches, int nb, uint32_t n_cells, int64_t n_refs, int64_t n_reads,
-                          uint64_t *pair_tmp, uint32_t *src_tmp, uint64_t *pair_sorted, uint32_t *order, void *tmp,
+                          const uint32_t *keep, uint64_t *pair_tmp, uint32_t *src_tmp, uint64_t *pair_sorted, uint32_t *order, void *tmp,
                           size_t tmp_bytes, int pair_bits, cudaStream_t st);
 cudaError_t assemble_gather_cells(const BatchDesc *batches, int nb, uint32_t n_cells, const uint32_t *order, int32_t *cells,
                                   int32_t *beginnings, int32_t *op_lens, int64_t *words, int64_t *ops_off, void *tmp,
@@ -187,6 +190,19 @@ cudaError_t assemble_gather_ops(const BatchDesc *batches, int nb, uint32_t n_cel
                                 const int64_t *ops_off, uint32_t *ops_out, cudaStream_t st);
 cudaError_t assemble_offsets(const uint64_t *pair_sorted, uint32_t n_cells, int64_t n_pairs, int64_t *cell_off,
                              int32_t *best, int64_t n_reads, const int32_t *cells, cudaStream_t st);
+
+// hits mode: *n_kept = cells of kept pairs (a device word); hits[q][h] (i, j) and the (i, j) of best hits below min_score
+cudaError_t assemble_kept_count(const uint64_t *pair_sorted, uint32_t n_cells, int64_t n_pairs, uint32_t *n_kept, cudaStream_t st);
+cudaError_t assemble_hit_cells(const BatchDesc *batches, int nb, const uint64_t *pair_sorted, const uint32_t *order, uint32_t n_all,
+                               int64_t n_pairs, int64_t n_reads, const int64_t *cell_off, const int32_t *cells, int32_t *best,
+                               int32_t *hits, int k, cudaStream_t st);
+
+// swb_hits.cu: per-read top k (score desc, ref asc) of scores[ref * n_reads + q] over q = slots[s] (slots null: q = s,
+// slot -1: skipped), written to hits[s * k ..] / bits as hits_merge_kernel describes.
+size_t      select_hits_tmp_elems(int64_t n_refs, int64_t n_slots, int k);
+cudaError_t launch_select_hits(const int32_t *scores, int64_t n_refs, int64_t n_reads, const int32_t *slots, int64_t n_slots,
+                               int k, int32_t min_score, int with_best, int4 *hits, uint32_t *bits, int64_t bit_slot,
+                               int64_t bit_ref, uint64_t *tmp, size_t tmp_elems, cudaStream_t st);
 
 cudaError_t launch_wide_pad_reads(const uint8_t *codes, const int64_t *read_off, const int32_t *reads, int n_reads,
                                   const int64_t *rpad_off, const int64_t *rpad_len, uint8_t *rpad, int64_t max_len,

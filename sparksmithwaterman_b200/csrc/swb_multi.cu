@@ -98,12 +98,50 @@ __global__ void merge_best_kernel(const int32_t *gathered, int world, int64_t n_
     reinterpret_cast<int4 *>(merged)[q] = best;
 }
 
+// hits mode: hit lists [n_reads][k] with shard-local reference indices -> global ids; padding stays (0, -1, 0, 0)
+__global__ void hits_to_global_kernel(const int32_t *hits, const int64_t *ids, int64_t n_ids, int64_t n, int32_t *out)
+{
+    const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    int4 h = reinterpret_cast<const int4 *>(hits)[e];
+    if (h.y >= 0 && h.y < n_ids) h.y = (int32_t)ids[h.y];
+    else h = make_int4(0, -1, 0, 0);
+    reinterpret_cast<int4 *>(out)[e] = h;
+}
+
+constexpr int kMaxHitsWorld = 64;
+
+// gathered[w][q][k] -> merged[q][k]: k-way merge of the world's sorted lists in the same order (score descending, then
+// global reference ascending); a list ends at its first entry without a reference, so an empty shard never wins.
+// Exact: the global top k is contained in the union of the shards' top k's.
+__global__ void merge_hits_kernel(const int32_t *gathered, int world, int64_t n_reads, int k, int32_t *merged)
+{
+    const int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (q >= n_reads) return;
+    const int4 *g = reinterpret_cast<const int4 *>(gathered);
+    int pos[kMaxHitsWorld];
+    for (int w = 0; w < world; ++w) pos[w] = 0;
+    for (int h = 0; h < k; ++h) {
+        int bw = -1;
+        int4 best = make_int4(0, -1, 0, 0);
+        for (int w = 0; w < world; ++w) {
+            if (pos[w] >= k) continue;
+            const int4 e = g[((int64_t)w * n_reads + q) * k + pos[w]];
+            if (e.y < 0) continue;
+            if (bw < 0 || e.x > best.x || (e.x == best.x && e.y < best.y)) { best = e; bw = w; }
+        }
+        if (bw >= 0) ++pos[bw];
+        reinterpret_cast<int4 *>(merged)[q * k + h] = best;
+    }
+}
+
 // send/gather/merge buffers of one device
 struct GatherBufs {
     DevBuf<int32_t> send, gathered, merged;
+    DevBuf<int32_t> hsend, hgathered, hmerged;   // hits mode: [n_reads][k][4] per shard
     DevBuf<int64_t> ids;
     int64_t n_ids = 0;
-    void release() { send.release(); gathered.release(); merged.release(); ids.release(); }
+    void release() { send.release(); gathered.release(); merged.release(); hsend.release(); hgathered.release(); hmerged.release(); ids.release(); }
 };
 
 // localize -> allgather -> merge on `st` of the current device.  `grouped`: the caller brackets several devices'
@@ -123,6 +161,26 @@ cudaError_t enqueue_merge(GatherBufs &g, int64_t n_reads, int world, cudaStream_
     if (n_reads == 0) return cudaSuccess;
     const int threads = 256;
     merge_best_kernel<<<(unsigned)((n_reads + threads - 1) / threads), threads, 0, st>>>(g.gathered.p, world, n_reads, g.merged.p);
+    return cudaGetLastError();
+}
+
+// the same two steps for the hit lists of a hits-mode result
+cudaError_t enqueue_localize_hits(GatherBufs &g, const int32_t *d_hits, int64_t n_reads, int k, int world, cudaStream_t st)
+{
+    const size_t n = (size_t)n_reads * k;
+    cudaError_t e = g.hsend.reserve(n * 4, st);
+    if (e == cudaSuccess) e = g.hgathered.reserve(n * 4 * world, st);
+    if (e == cudaSuccess) e = g.hmerged.reserve(n * 4, st);
+    if (e != cudaSuccess || n == 0) return e;
+    const int threads = 256;
+    hits_to_global_kernel<<<(unsigned)((n + threads - 1) / threads), threads, 0, st>>>(d_hits, g.ids.p, g.n_ids, (int64_t)n, g.hsend.p);
+    return cudaGetLastError();
+}
+cudaError_t enqueue_merge_hits(GatherBufs &g, int64_t n_reads, int k, int world, cudaStream_t st)
+{
+    if (n_reads == 0) return cudaSuccess;
+    const int threads = 128;
+    merge_hits_kernel<<<(unsigned)((n_reads + threads - 1) / threads), threads, 0, st>>>(g.hgathered.p, world, n_reads, k, g.hmerged.p);
     return cudaGetLastError();
 }
 
@@ -153,6 +211,8 @@ struct swb_multi_result {
     swb_multi *m = nullptr;
     std::vector<swb_result *> shard;
     std::vector<int32_t> merged;
+    int32_t top_k = 0;                           // hits mode: merged_hits = [n_reads][k][4], global reference ids
+    std::vector<int32_t> merged_hits;
     int64_t n_reads = 0;
     double stats[3] = {0, 0, 0};
 };
@@ -224,6 +284,37 @@ int swb_comm_allgather_best(swb_comm *c, const swb_result *res, const int64_t *g
     }
     CU(enqueue_merge(c->g, n_reads, c->world, st));
     if (merged_host && n_reads) CU(cudaMemcpyAsync(merged_host, c->g.merged.p, (size_t)n_reads * 16, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));        // global_ids / merged_host are the caller's
+    return SWB_OK;
+}
+
+int swb_comm_allgather_hits(swb_comm *c, const swb_result *res, const int64_t *global_ids, int64_t n_local_refs,
+                            int32_t *merged_host)
+{
+    if (!c || !res) return fail(SWB_E_INVALID, "swb_comm_allgather_hits: null argument");
+    if (res->ctx != c->ctx) return fail(SWB_E_INVALID, "swb_comm_allgather_hits: the result belongs to another context");
+    if (res->top_k <= 0) return fail(SWB_E_INVALID, "swb_comm_allgather_hits: not a hits-mode result (swb_align_hits)");
+    if (c->world > kMaxHitsWorld) return fail(SWB_E_UNSUPPORTED, "swb_comm_allgather_hits: more than 64 ranks");
+    if (n_local_refs != res->n_refs) return fail(SWB_E_INVALID, "swb_comm_allgather_hits: global_ids must cover the shard's references");
+    if (n_local_refs > 0 && !global_ids) return fail(SWB_E_INVALID, "swb_comm_allgather_hits: global_ids is null");
+    swb_ctx *ctx = c->ctx;
+    std::lock_guard<std::recursive_mutex> lk(ctx->mu);
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const int64_t n_reads = res->n_reads;
+    const int k = res->top_k;
+    const size_t n = (size_t)n_reads * k;
+    CU(c->g.ids.reserve((size_t)std::max<int64_t>(n_local_refs, 1), st));
+    c->g.n_ids = n_local_refs;
+    if (n_local_refs) CU(cudaMemcpyAsync(c->g.ids.p, global_ids, (size_t)n_local_refs * 8, cudaMemcpyHostToDevice, st));
+    CU(enqueue_localize_hits(c->g, res->d_hits.p, n_reads, k, c->world, st));
+    if (c->world > 1) {
+        if (n) NC(nccl_api()->AllGather(c->g.hsend.p, c->g.hgathered.p, n * 4, ncclInt32, c->comm, st));
+    } else if (n) {
+        CU(cudaMemcpyAsync(c->g.hgathered.p, c->g.hsend.p, n * 16, cudaMemcpyDeviceToDevice, st));
+    }
+    CU(enqueue_merge_hits(c->g, n_reads, k, c->world, st));
+    if (merged_host && n) CU(cudaMemcpyAsync(merged_host, c->g.hmerged.p, n * 16, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));        // global_ids / merged_host are the caller's
     return SWB_OK;
 }
@@ -362,18 +453,22 @@ const int64_t *swb_multi_shard_refs(const swb_multi *m, int32_t d, int64_t *n)
     return m->ids[(size_t)d].data();
 }
 
-int swb_multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
-                    int32_t mismatch, int32_t gap, uint32_t flags, swb_multi_result **out)
+}  // extern "C"
+
+// top_k > 0: hits mode (swb_multi_align_hits)
+static int multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
+                       int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_multi_result **out)
 {
     if (!m || !out) return fail(SWB_E_INVALID, "swb_multi_align: null argument");
     *out = nullptr;
     const int n = (int)m->ctx.size();
+    if (top_k > 0 && n > kMaxHitsWorld) return fail(SWB_E_UNSUPPORTED, "swb_multi_align_hits: more than 64 devices");
     for (int d = 0; d < n; ++d)
         if (!m->rs[(size_t)d]) return fail(SWB_E_INVALID, "swb_multi_align: no reference set loaded");
     std::lock_guard<std::mutex> lk(m->mu);
     const auto t0 = std::chrono::steady_clock::now();
     std::unique_ptr<swb_multi_result> res(new swb_multi_result());
-    res->m = m; res->n_reads = n_reads;
+    res->m = m; res->n_reads = n_reads; res->top_k = top_k;
     res->shard.assign((size_t)n, nullptr);
     auto drop = [&] { for (swb_result *r : res->shard) if (r) swb_result_free(r); res->shard.clear(); };
 
@@ -384,8 +479,11 @@ int swb_multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, const
         std::vector<std::thread> th;
         for (int d = 0; d < n; ++d)
             th.emplace_back([&, d] {
-                rcs[(size_t)d] = swb_align(m->ctx[(size_t)d], m->rs[(size_t)d], n_reads, read_bytes, read_offsets, match, mismatch,
-                                           gap, flags | SWB_F_NO_FETCH, &res->shard[(size_t)d]);
+                rcs[(size_t)d] = top_k > 0
+                    ? swb_align_hits(m->ctx[(size_t)d], m->rs[(size_t)d], n_reads, read_bytes, read_offsets, match, mismatch, gap,
+                                     flags | SWB_F_NO_FETCH, top_k, min_score, &res->shard[(size_t)d])
+                    : swb_align(m->ctx[(size_t)d], m->rs[(size_t)d], n_reads, read_bytes, read_offsets, match, mismatch,
+                                gap, flags | SWB_F_NO_FETCH, &res->shard[(size_t)d]);
                 if (rcs[(size_t)d]) errs[(size_t)d] = swb_last_error();
             });
         for (auto &t : th) t.join();
@@ -399,19 +497,26 @@ int swb_multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, const
         swb_ctx *c = m->ctx[(size_t)d];
         cudaError_t e = cudaSetDevice(c->device);
         if (e == cudaSuccess) e = enqueue_localize(m->g[(size_t)d], res->shard[(size_t)d]->d_best.p, n_reads, n, c->stream);
+        if (e == cudaSuccess && top_k > 0)
+            e = enqueue_localize_hits(m->g[(size_t)d], res->shard[(size_t)d]->d_hits.p, n_reads, top_k, n, c->stream);
         if (e != cudaSuccess) { drop(); return cuda_fail(e, "swb_multi_align: best hits -> global ids"); }
     }
     if (n > 1 && n_reads > 0) {
         NcclApi *a = nccl_api();
         ncclResult_t r = a->GroupStart();
-        for (int d = 0; d < n && r == ncclSuccess; ++d)
+        for (int d = 0; d < n && r == ncclSuccess; ++d) {
             r = a->AllGather(m->g[(size_t)d].send.p, m->g[(size_t)d].gathered.p, (size_t)n_reads * 4, ncclInt32, m->comms[(size_t)d],
                              m->ctx[(size_t)d]->stream);
+            if (r == ncclSuccess && top_k > 0)
+                r = a->AllGather(m->g[(size_t)d].hsend.p, m->g[(size_t)d].hgathered.p, (size_t)n_reads * top_k * 4, ncclInt32,
+                                 m->comms[(size_t)d], m->ctx[(size_t)d]->stream);
+        }
         const ncclResult_t r2 = a->GroupEnd();
         if (r == ncclSuccess) r = r2;
         if (r != ncclSuccess) { drop(); return nccl_fail(r, "swb_multi_align: ncclAllGather"); }
     }
     res->merged.assign((size_t)n_reads * 4, 0);
+    if (top_k > 0) res->merged_hits.assign((size_t)n_reads * top_k * 4, 0);
     for (int d = 0; d < n; ++d) {
         swb_ctx *c = m->ctx[(size_t)d];
         GatherBufs &g = m->g[(size_t)d];
@@ -421,6 +526,13 @@ int swb_multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, const
         if (e == cudaSuccess) e = enqueue_merge(g, n_reads, n, c->stream);
         if (e == cudaSuccess && d == 0 && n_reads)
             e = cudaMemcpyAsync(res->merged.data(), g.merged.p, (size_t)n_reads * 16, cudaMemcpyDeviceToHost, c->stream);
+        if (top_k > 0 && n_reads) {
+            if (e == cudaSuccess && n == 1)
+                e = cudaMemcpyAsync(g.hgathered.p, g.hsend.p, (size_t)n_reads * top_k * 16, cudaMemcpyDeviceToDevice, c->stream);
+            if (e == cudaSuccess) e = enqueue_merge_hits(g, n_reads, top_k, n, c->stream);
+            if (e == cudaSuccess && d == 0)
+                e = cudaMemcpyAsync(res->merged_hits.data(), g.hmerged.p, (size_t)n_reads * top_k * 16, cudaMemcpyDeviceToHost, c->stream);
+        }
         if (e != cudaSuccess) { drop(); return cuda_fail(e, "swb_multi_align: merge"); }
     }
     for (int d = 0; d < n; ++d) {
@@ -449,6 +561,23 @@ int swb_multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, const
     return SWB_OK;
 }
 
+extern "C" {
+
+int swb_multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
+                    int32_t mismatch, int32_t gap, uint32_t flags, swb_multi_result **out)
+{
+    return multi_align(m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, 1, out);
+}
+
+int swb_multi_align_hits(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
+                         int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_multi_result **out)
+{
+    if (out) *out = nullptr;
+    if (top_k < 1 || top_k > 32) return fail(SWB_E_INVALID, "swb_multi_align_hits: top_k must be 1 .. 32");
+    if (min_score < 1) return fail(SWB_E_INVALID, "swb_multi_align_hits: min_score must be >= 1");
+    return multi_align(m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, top_k, min_score, out);
+}
+
 void swb_multi_result_free(swb_multi_result *res)
 {
     if (!res) return;
@@ -461,6 +590,12 @@ swb_result *swb_multi_result_shard(swb_multi_result *res, int32_t d)
     return (res && d >= 0 && d < (int32_t)res->shard.size()) ? res->shard[(size_t)d] : nullptr;
 }
 const int32_t *swb_multi_result_best_hits(const swb_multi_result *res) { return res ? res->merged.data() : nullptr; }
+const int32_t *swb_multi_result_hits(const swb_multi_result *res, int32_t *top_k)
+{
+    const bool ok = res && res->top_k > 0;
+    if (top_k) *top_k = ok ? res->top_k : 0;
+    return ok ? res->merged_hits.data() : nullptr;
+}
 int swb_multi_result_stats(const swb_multi_result *res, double *out, int n)
 {
     if (!res || !out) return fail(SWB_E_INVALID, "swb_multi_result_stats: null");

@@ -474,8 +474,9 @@ static cudaError_t launch_trace_k(const BatchParams &P, const uint64_t *keys, ui
         const cudaError_t e = attr.run([&] { return cudaFuncSetAttribute(trace_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); });
         if (e != cudaSuccess) return e;
     }
-    // chunks of the sorted cell list: several per SM for balance, each long enough to amortise its profile
-    int chunk = (int)std::max<int64_t>(256, ((int64_t)n_cells + sm_count * 4 - 1) / (sm_count * 4));
+    // chunks of the sorted cell list: several per SM for balance, each long enough to amortise its profile (hits mode,
+    // P.sel: a few cells per read, one chunk may be a single cell -- see launch_tile_trace_k)
+    int chunk = (int)std::max<int64_t>(P.sel ? 1 : 256, ((int64_t)n_cells + sm_count * 4 - 1) / (sm_count * 4));
     const int64_t ctas = ((int64_t)n_cells + chunk - 1) / chunk;
     trace_kernel<K><<<(unsigned)ctas, warps * 32, smem, st>>>(P, keys, n_cells, chunk, beginnings, op_lens, ops, ops_stride, 0u);
     return cudaGetLastError();

@@ -481,7 +481,8 @@ __global__ void __launch_bounds__(NT) tile_scan_kernel(const BatchParams P, cons
     }
 }
 
-template <int K>
+// SEL (hits mode): a pair emits only if its bit in P.sel is set; a separate instantiation keeps the plain emit as it was
+template <int K, bool SEL>
 __global__ void __launch_bounds__(NT) tile_emit_kernel(const BatchParams P, const TileTask *tasks,
                                                        const uint32_t *n_tasks_ptr, uint32_t cap_tasks, const TileHit *hits,
                                                        uint64_t *keys, uint32_t cap, uint32_t *count)
@@ -504,6 +505,10 @@ __global__ void __launch_bounds__(NT) tile_emit_kernel(const BatchParams P, cons
             const int64_t ro = P.ref_orig[T.ref_sorted];
             pkey = ((uint64_t)T.rp_half * (uint64_t)P.n_refs + (uint64_t)ro) << (KEY_J_BITS + KEY_I_BITS);
             hot = h.n > 0 && h.emax == P.scores[ro * P.n_reads + read_idx];   // exact since the scan pass
+            if (SEL) {
+                const uint64_t b = (uint64_t)T.rp_half * (uint64_t)P.n_refs + (uint64_t)ro;
+                hot = hot && ((P.sel[b >> 5] >> (b & 31)) & 1u);
+            }
         }
         const uint32_t mine = hot ? min(h.n, 4u) : 0u;
         uint32_t inc = mine;
@@ -551,7 +556,8 @@ cudaError_t launch_tile_locate_k(const BatchParams &P, const TileTask *tasks, co
     // the task count is read on the device; size the grid for the capacity, capped at a few waves
     const int64_t ctas = std::max<int64_t>(1, std::min<int64_t>(((int64_t)cap_tasks + NT - 1) / NT, (int64_t)sm_count * 32));
     if (phase == 0) tile_scan_kernel<K><<<(unsigned)ctas, NT, 0, st>>>(P, tasks, n_tasks, cap_tasks, static_cast<TileHit *>(hits));
-    else tile_emit_kernel<K><<<(unsigned)ctas, NT, 0, st>>>(P, tasks, n_tasks, cap_tasks, static_cast<const TileHit *>(hits), keys, cap, count);
+    else if (P.sel) tile_emit_kernel<K, true><<<(unsigned)ctas, NT, 0, st>>>(P, tasks, n_tasks, cap_tasks, static_cast<const TileHit *>(hits), keys, cap, count);
+    else tile_emit_kernel<K, false><<<(unsigned)ctas, NT, 0, st>>>(P, tasks, n_tasks, cap_tasks, static_cast<const TileHit *>(hits), keys, cap, count);
     return cudaGetLastError();
 }
 
@@ -571,10 +577,12 @@ cudaError_t launch_tile_trace_k(const BatchParams &P, const uint64_t *keys, uint
         });
         if (e != cudaSuccess) return e;
     }
-    // chunks of the sorted cell list: many per SM for balance, each long enough to amortise its profile
+    // chunks of the sorted cell list: many per SM for balance, each long enough to amortise its profile.  In hits mode
+    // (P.sel) a read has a handful of cells: a CTA walks its chunk's reads one after another, so a chunk of 2 * NT
+    // cells would serialise up to 2 * NT walks in one CTA; every cell may start a chunk of its own there.
     static const int env_div = getenv("SWB_TRACE_CHUNKS_PER_SM") ? atoi(getenv("SWB_TRACE_CHUNKS_PER_SM")) : 0;
     const int per_sm = env_div > 0 ? env_div : 16;
-    const int chunk = (int)std::max<int64_t>(2 * NT, ((int64_t)n_cells + (int64_t)sm_count * per_sm - 1) / ((int64_t)sm_count * per_sm));
+    const int chunk = (int)std::max<int64_t>(P.sel ? 1 : 2 * NT, ((int64_t)n_cells + (int64_t)sm_count * per_sm - 1) / ((int64_t)sm_count * per_sm));
     const int64_t ctas = ((int64_t)n_cells + chunk - 1) / chunk;
     if (P.tie_gt) tile_trace_kernel<K, true><<<(unsigned)ctas, NT, smem, st>>>(P, keys, n_cells, chunk, beginnings, op_lens, ops, ops_stride, 65536u);
     else          tile_trace_kernel<K, false><<<(unsigned)ctas, NT, smem, st>>>(P, keys, n_cells, chunk, beginnings, op_lens, ops, ops_stride, 65536u);

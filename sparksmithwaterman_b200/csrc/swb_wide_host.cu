@@ -26,7 +26,8 @@ static int pick_kl(int64_t m)
 
 int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const std::vector<int32_t> &reads,
                   int match, int mismatch, int gap, uint32_t flags, swb_result *res, int *launches, int *n_batches,
-                  double *ck_bytes, const std::function<cudaError_t(int)> &tic, const std::function<cudaError_t()> &toc)
+                  double *ck_bytes, const std::function<cudaError_t(int)> &tic, const std::function<cudaError_t()> &toc,
+                  const std::vector<std::vector<int32_t>> *refs_of)
 {
     cudaStream_t st = ctx->stream;
     const int64_t n_refs = rs->n_refs, n_reads = rd->n_reads;
@@ -59,8 +60,14 @@ int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const
     const int64_t BH = (int64_t)WL * KL, RW = wide_rw(KL);
     // all (read, ref) pairs of this rows-per-lane class with a non-empty matrix, read-major
     std::vector<int32_t> pr, pq;
-    for (int32_t q : reads) {
+    for (size_t x = 0; x < reads.size(); ++x) {
+        const int32_t q = reads[x];
         if (pick_kl(rd->len[(size_t)q]) != KL) continue;
+        if (refs_of) {
+            for (int32_t r : (*refs_of)[x])
+                if (rs->len_orig[(size_t)r] > 0) { pr.push_back(r); pq.push_back(q); }
+            continue;
+        }
         for (int64_t r = 0; r < n_refs; ++r)
             if (rs->len_orig[(size_t)r] > 0) { pr.push_back((int32_t)r); pq.push_back(q); }
     }

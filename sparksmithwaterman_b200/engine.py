@@ -114,16 +114,22 @@ class RefSet:
         return Reads(self, reads)
 
     def align(self, reads, scores=DEFAULT_SCORES, scores_only: bool = False, fetch: bool = True,
-              tie_gt: bool = False) -> "AlignResult":
+              tie_gt: bool = False, *, top_k: int | None = None, min_score: int = 1) -> "AlignResult":
         """Host-buffer path (swb_align): H2D of the reads, compute, D2H of the results.
-        tie_gt: DistributedSW's strict-'>' tie rule in the traceback (SWB_F_TIE_GT)."""
+        tie_gt: DistributedSW's strict-'>' tie rule in the traceback (SWB_F_TIE_GT).
+        top_k: hits mode (swb_align_hits) -- every pair is scored, but only each read's top_k best pairs with
+        score >= min_score are traced (AlignResult.hits / read_hits)."""
         if isinstance(reads, Reads):
-            return reads.align(scores, scores_only, fetch, tie_gt)
+            return reads.align(scores, scores_only, fetch, tie_gt, top_k=top_k, min_score=min_score)
         data, off, bs = concat(reads)
         flags = (SWB_F_SCORES_ONLY if scores_only else 0) | (0 if fetch else SWB_F_NO_FETCH) | (SWB_F_TIE_GT if tie_gt else 0)
         h = C.c_void_p()
-        check(self.eng.lib.swb_align(self.eng.h, self.h, len(bs), data, _i64p(off),
-                                     scores[0], scores[1], scores[2], flags, C.byref(h)))
+        if top_k is None:
+            check(self.eng.lib.swb_align(self.eng.h, self.h, len(bs), data, _i64p(off),
+                                         scores[0], scores[1], scores[2], flags, C.byref(h)))
+        else:
+            check(self.eng.lib.swb_align_hits(self.eng.h, self.h, len(bs), data, _i64p(off),
+                                              scores[0], scores[1], scores[2], flags, top_k, min_score, C.byref(h)))
         return AlignResult(self, bs, h, scores_only)
 
 
@@ -151,16 +157,20 @@ class Reads:
             pass
 
     def align(self, scores=DEFAULT_SCORES, scores_only: bool = False, fetch: bool = True,
-              tie_gt: bool = False) -> "AlignResult":
+              tie_gt: bool = False, *, top_k: int | None = None, min_score: int = 1) -> "AlignResult":
         flags = (SWB_F_SCORES_ONLY if scores_only else 0) | (0 if fetch else SWB_F_NO_FETCH) | (SWB_F_TIE_GT if tie_gt else 0)
         h = C.c_void_p()
-        check(self.rs.eng.lib.swb_align_resident(self.rs.eng.h, self.rs.h, self.h,
-                                                 scores[0], scores[1], scores[2], flags, C.byref(h)))
+        lib = self.rs.eng.lib
+        if top_k is None:
+            check(lib.swb_align_resident(self.rs.eng.h, self.rs.h, self.h, scores[0], scores[1], scores[2], flags, C.byref(h)))
+        else:
+            check(lib.swb_align_resident_hits(self.rs.eng.h, self.rs.h, self.h, scores[0], scores[1], scores[2], flags,
+                                              top_k, min_score, C.byref(h)))
         return AlignResult(self.rs, self.seqs, h, scores_only)
 
 
 STAT_NAMES = ("h2d_ms", "fill_ms", "locate_ms", "trace_ms", "d2h_ms", "device_ms", "cells", "pairs",
-              "max_cells", "launches", "checkpoint_bytes", "batches")
+              "max_cells", "launches", "checkpoint_bytes", "batches", "select_ms")
 
 
 class AlignResult:
@@ -194,8 +204,8 @@ class AlignResult:
 
     @property
     def stats(self) -> dict:
-        out = (C.c_double * 12)()
-        check(self.lib.swb_result_stats(self.h, out, 12))
+        out = (C.c_double * len(STAT_NAMES))()
+        check(self.lib.swb_result_stats(self.h, out, len(STAT_NAMES)))
         return dict(zip(STAT_NAMES, list(out)))
 
     @property
@@ -211,6 +221,26 @@ class AlignResult:
     @property
     def best_hits(self) -> np.ndarray:
         return self._arr(self.lib.swb_result_best_hits(self.h), self.n_reads * 4, np.int32).reshape(self.n_reads, 4)
+
+    @property
+    def hits(self) -> np.ndarray:
+        """Hits mode: [n_reads, k, 4] int32 (score, ref, i, j), each read's k best pairs with score >= min_score,
+        score descending then ref ascending, padded with (0, -1, 0, 0).  [n_reads, 0, 4] for a plain result."""
+        k = C.c_int32()
+        p = self.lib.swb_result_hits(self.h, C.byref(k))
+        if not p:                                 # a plain result, or not fetched yet
+            return np.zeros((self.n_reads, 0, 4), np.int32)
+        return self._arr(p, self.n_reads * k.value * 4, np.int32).reshape(self.n_reads, k.value, 4)
+
+    def read_hits(self, read: int):
+        """Hits mode: [(ref, score, cells, sites)] of read `read`'s hits in hit order; cells / sites as pair()."""
+        out = []
+        for score, ref, _, _ in self.hits[read]:
+            if ref < 0:
+                break
+            _, cells, sites = self.pair(int(ref), read)
+            out.append((int(ref), int(score), cells, sites))
+        return out
 
     @property
     def cell_offsets(self) -> np.ndarray:

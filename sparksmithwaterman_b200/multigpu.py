@@ -38,6 +38,23 @@ def merge_best_hits(records: np.ndarray) -> np.ndarray:
     return rec[win, np.arange(rec.shape[1])].astype(np.int32)
 
 
+def merge_top_hits(records: np.ndarray) -> np.ndarray:
+    """records: [world, n_reads, k, 4] int (score, global ref id, i, j), each rank's hit list in hit order (score
+    descending, then ref ascending), padded with (0, -1, 0, 0).  Returns the top k of the union per read in the same
+    order, [n_reads, k, 4] -- exact, since the global top k lies in the union of the ranks' top k's.  Entries without
+    a reference (padding, an empty shard) never win."""
+    rec = np.asarray(records).astype(np.int64)
+    world, n_reads, k = rec.shape[:3]
+    allr = rec.transpose(1, 0, 2, 3).reshape(n_reads, world * k, 4)
+    ok = allr[:, :, 1] >= 0
+    # sort key: score descending, then ref ascending; padding last
+    key = np.where(ok, -(allr[:, :, 0] * (1 << 32)) + allr[:, :, 1], np.iinfo(np.int64).max)
+    order = np.argsort(key, axis=1, kind="stable")[:, :k]
+    out = np.take_along_axis(allr, order[:, :, None], axis=1)
+    out[~np.take_along_axis(ok, order, axis=1)] = (0, -1, 0, 0)
+    return out.astype(np.int32)
+
+
 def localize(best_local: np.ndarray, my_ids: Sequence[int]) -> np.ndarray:
     """Shard-local ref indices -> global ref ids."""
     out = np.array(best_local, dtype=np.int32, copy=True)
@@ -123,11 +140,17 @@ class MultiEngine:
         check(self.lib.swb_multi_ref_location(self.h, g, _C.byref(sh), _C.byref(loc)))
         return sh.value, loc.value
 
-    def align(self, reads, scores=DEFAULT_SCORES, scores_only: bool = False, fetch: bool = True, tie_gt: bool = False):
+    def align(self, reads, scores=DEFAULT_SCORES, scores_only: bool = False, fetch: bool = True, tie_gt: bool = False,
+              *, top_k: int | None = None, min_score: int = 1):
+        """top_k: hits mode (swb_multi_align_hits), every shard in hits mode and the hit lists merged (MultiResult.hits)."""
         data, off, bs = concat(reads)
         flags = (SWB_F_SCORES_ONLY if scores_only else 0) | (0 if fetch else SWB_F_NO_FETCH) | (SWB_F_TIE_GT if tie_gt else 0)
         h = _C.c_void_p()
-        check(self.lib.swb_multi_align(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags, _C.byref(h)))
+        if top_k is None:
+            check(self.lib.swb_multi_align(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags, _C.byref(h)))
+        else:
+            check(self.lib.swb_multi_align_hits(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags,
+                                                top_k, min_score, _C.byref(h)))
         return MultiResult(self, bs, h, scores_only)
 
 
@@ -156,6 +179,15 @@ class MultiResult:
         n = len(self.reads)
         p = self.lib.swb_multi_result_best_hits(self.h)
         return np.ctypeslib.as_array(p, shape=(n * 4,)).copy().reshape(n, 4) if n else np.zeros((0, 4), np.int32)
+
+    @property
+    def hits(self) -> np.ndarray:
+        """Hits mode: merged [n_reads, k, 4] (score, GLOBAL ref id, i, j); [n_reads, 0, 4] for a plain result."""
+        n, k = len(self.reads), _C.c_int32()
+        p = self.lib.swb_multi_result_hits(self.h, _C.byref(k))
+        if not p or n == 0:
+            return np.zeros((n, k.value, 4), np.int32)
+        return np.ctypeslib.as_array(p, shape=(n * k.value * 4,)).copy().reshape(n, k.value, 4)
 
     @property
     def stats(self) -> dict:
@@ -208,4 +240,14 @@ class Comm:
         out = np.empty((res.n_reads, 4), dtype=np.int32) if want_host else None
         check(self.lib.swb_comm_allgather_best(self.h, res.h, _i64p(ids), len(ids),
                                                out.ctypes.data_as(_C.POINTER(_C.c_int32)) if want_host else None))
+        return out
+
+    def allgather_hits(self, res: AlignResult, global_ids) -> np.ndarray:
+        """Hit lists of a hits-mode result of this rank's shard -> merged [n_reads, k, 4] with global ref ids."""
+        ids = np.ascontiguousarray(global_ids, dtype=np.int64)
+        k = _C.c_int32()
+        self.lib.swb_result_hits(res.h, _C.byref(k))
+        out = np.empty((res.n_reads, k.value, 4), dtype=np.int32)
+        check(self.lib.swb_comm_allgather_hits(self.h, res.h, _i64p(ids), len(ids),
+                                               out.ctypes.data_as(_C.POINTER(_C.c_int32)) if out.size else None))
         return out
