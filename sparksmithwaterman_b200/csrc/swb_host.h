@@ -1,9 +1,10 @@
-// swb_host.h -- host-side structures of libswb200 shared by swb_api.cu and swb_wide_host.cu.
+// swb_host.h -- host-side structures of libswb200 shared by swb_api.cu, swb_align.cu and swb_wide_host.cu.
 #pragma once
 #include "swb_internal.h"
 
 #include <algorithm>
 #include <atomic>
+#include <chrono>
 #include <map>
 #include <tuple>
 #include <cstdio>
@@ -130,6 +131,18 @@ template <class T> struct DevBuf {
 
 inline int upper(int c) { return (c >= 'a' && c <= 'z') ? c - 32 : c; }
 
+// grid of a grid-stride loop over n elements
+inline int grid_for(int64_t n, int threads, int sm_count)
+{
+    return (int)std::max<int64_t>(1, std::min<int64_t>((n + threads - 1) / threads, (int64_t)sm_count * 16));
+}
+
+// the entries of swb_result_stats (include/swb200.h, engine.STAT_NAMES)
+enum Stat {
+    STAT_H2D_MS, STAT_FILL_MS, STAT_LOCATE_MS, STAT_TRACE_MS, STAT_D2H_MS, STAT_DEVICE_MS, STAT_CELLS, STAT_PAIRS,
+    STAT_MAX_CELLS, STAT_LAUNCHES, STAT_CK_BYTES, STAT_BATCHES, STAT_SELECT_MS, STAT_COUNT
+};
+
 }  // namespace swbh
 
 using swbh::DevBuf;
@@ -141,19 +154,14 @@ struct swb_ctx {
     int sm_count = 0;
     int64_t ws_bytes = 0;
     cudaStream_t stream = nullptr;
-    cudaStream_t stream_fill = nullptr;         // second stream: fill of batch k+1 runs beside the traceback of batch k
     cudaStream_t stream_copy = nullptr;         // results of reference part k cross PCIe while part k+1 computes
-    bool pipeline = true;
-    DevBuf<uint32_t> ck2[2], tmx2[2];           // ping-pong checkpoint workspaces
-    DevBuf<int32_t> rp2[2];
     cudaEvent_t ev[2] = {nullptr, nullptr};
     std::recursive_mutex mu;
     std::atomic<int> live{0};                   // handles (refsets, read batches, results) that still point here
     std::atomic<bool> dying{false};             // swb_destroy was called while handles were alive: the last free destroys
     // grow-only scratch reused by every align call on this context
-    DevBuf<uint32_t> ck, tmx, counters;
-    DevBuf<int32_t> rp, slot;
-    DevBuf<int32_t> v_ref, v_c0, v_len, v_skip, v_end;   // fill work units (reference segments) of the current class
+    DevBuf<uint32_t> ck, tmx, counters;         // checkpoint workspace, tile maxima, device counters of one batch
+    DevBuf<int32_t> rp;                         // read pairs of one batch
     DevBuf<TileTask> tasks;
     DevBuf<uint8_t> task_hits;                 // per candidate tile: exact maximum + buffered cells (locate scan -> emit)
     DevBuf<uint64_t> keys_tmp;
@@ -181,7 +189,6 @@ struct swb_ctx {
         while (c < bytes) c <<= 1;
         return c;
     }
-    int64_t pin_allocs = 0;                     // cudaHostAlloc calls so far (SWB_TIMELINE prints them)
     PinBuf pin_get(size_t bytes)
     {
         const size_t want = pin_class(bytes);
@@ -191,7 +198,6 @@ struct swb_ctx {
         if (best != pin_free.size()) { PinBuf b = pin_free[best]; pin_free.erase(pin_free.begin() + best); return b; }
         PinBuf b;
         b.bytes = want;
-        ++pin_allocs;
         if (cudaHostAlloc(&b.p, b.bytes, cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); b.p = nullptr; b.bytes = 0; }
         return b;
     }
@@ -253,7 +259,6 @@ struct swb_reads {
 };
 
 struct BatchOut {
-    int K = 0;
     bool wide = false;                           // produced by the int32 long-pair path (different key layout)
     std::vector<int64_t> wide_pair_p;            // wide: local pair -> ABI pair index p
     uint32_t n_cells = 0;
@@ -261,8 +266,7 @@ struct BatchOut {
     DevBuf<uint64_t> keys;
     DevBuf<int32_t> beg, oplen;
     DevBuf<uint32_t> ops;
-    std::vector<int32_t> slot_read;              // read slot of this batch -> read index of the call
-    DevBuf<int32_t> d_slot_read;                 // the same on the device, for the assembly
+    DevBuf<int32_t> d_slot_read;                 // read slot of this batch -> read index of the call, for the assembly
     DevBuf<int64_t> d_pair_map;                  // wide path: local pair -> p, on the device
 };
 
@@ -289,7 +293,7 @@ struct swb_result {
     const int64_t *cell_off = nullptr, *ops_off = nullptr;
     const int32_t *cells = nullptr, *beginnings = nullptr, *op_lens = nullptr;
     const uint32_t *ops = nullptr;
-    double stats[13] = {0};
+    double stats[swbh::STAT_COUNT] = {0};
     std::vector<char> own;                      // host arrays of a 1 x 1 result cut out of a coalesced batch (swb_queue.cu)
     // result of a multi-part reference set: one sub-result per part (device arrays), stitched into the host arrays
     std::vector<swb_result *> subs;
@@ -302,11 +306,74 @@ struct swb_result {
 };
 
 
-#include <functional>
 namespace swbh {
-// refs_of (nullable): refs_of[k] = the references (ascending) read reads[k] is aligned against; nullptr = all of them
-int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const std::vector<int32_t> &reads,
-                  int match, int mismatch, int gap, uint32_t flags, swb_result *res, int *launches, int *n_batches,
-                  double *ck_bytes, const std::function<cudaError_t(int)> &tic, const std::function<cudaError_t()> &toc,
-                  const std::vector<std::vector<int32_t>> *refs_of = nullptr);
-}
+
+// Device time per phase of one call: event pairs around the work, read once after the call's last sync.  Spans nest
+// (a selection inside the locate span); end() closes the innermost open one.
+struct PhaseTimer {
+    struct Span { cudaEvent_t a, b; Stat stat; };
+    swb_ctx *ctx;
+    cudaStream_t st;
+    std::vector<Span> spans;
+    std::vector<size_t> open;
+    cudaError_t begin(Stat stat)
+    {
+        Span s{nullptr, nullptr, stat};
+        cudaError_t e;
+        if ((e = ctx->next_event(&s.a)) || (e = ctx->next_event(&s.b)) || (e = cudaEventRecord(s.a, st))) return e;
+        open.push_back(spans.size());
+        spans.push_back(s);
+        return cudaSuccess;
+    }
+    cudaError_t end()
+    {
+        const size_t k = open.back();
+        open.pop_back();
+        return cudaEventRecord(spans[k].b, st);
+    }
+    // adds each span's milliseconds to its entry of `stats`
+    cudaError_t add_to(double *stats) const
+    {
+        float ms = 0;
+        for (const Span &s : spans) {
+            if (cudaError_t e = cudaEventElapsedTime(&ms, s.a, s.b)) return e;
+            stats[s.stat] += ms;
+        }
+        return cudaSuccess;
+    }
+};
+
+// One align call over one packed set (a whole set, or one part of a large one), step by step (swb_align.cu; the wide
+// path in swb_wide_host.cu).  top_k > 0: hits mode (swb_align_hits).
+struct AlignCall {
+    swb_ctx *ctx;
+    const swb_refset *rs;
+    const swb_reads *rd;
+    int32_t match, mismatch, gap;
+    uint32_t flags;
+    int32_t top_k, min_score;
+    swb_result *res;
+    cudaStream_t st;
+    PhaseTimer timer;
+    int launches = 1, n_batches = 0;
+    double ck_bytes = 0;
+
+    struct Batch;
+    int run(int32_t *ext_scores, int32_t *ext_totals);
+    void classify_reads(std::vector<std::vector<int32_t>> &classes, std::vector<int32_t> &wide) const;
+    int run_class(int K, std::vector<int32_t> &reads);
+    int seg_tables(int K, bool few_items, std::shared_ptr<swb_refset::SegTables> &out);
+    int fill_batch(int K, const std::vector<int32_t> &reads, int64_t rp0, int n_rp, const swb_refset::SegTables &segt, Batch &b);
+    int trace_batch(int K, Batch &b);
+    int locate_cells(int K, const Batch &b, size_t sel_words, uint32_t &n_cells);
+    cudaError_t select_hits(const int32_t *slots, int64_t n_slots, int with_best, int4 *hits, uint32_t *bits, int64_t bit_slot,
+                            int64_t bit_ref);
+    int run_wide_reads(const std::vector<int32_t> &wide);
+    // refs_of (nullable): refs_of[k] = the references (ascending) read reads[k] is aligned against; nullptr = all of them
+    int run_wide_path(const std::vector<int32_t> &reads, bool scores_only, const std::vector<std::vector<int32_t>> *refs_of = nullptr);
+    int select_final_hits(DevBuf<uint32_t> &keep);
+    int assemble(const DevBuf<uint32_t> &keep);
+    int finish_stats(std::chrono::steady_clock::time_point t_wall0);
+};
+
+}  // namespace swbh

@@ -102,9 +102,9 @@ swb_result *cut_pair(swb_ctx *ctx, const swb_result *big, int64_t r, int64_t q, 
         res->cell_off = cell_off; res->cells = cells; res->beginnings = beg; res->op_lens = len; res->ops_off = ops_off; res->ops = u32;
         res->total_cells = (uint32_t)n; res->total_words = w1 - w0;
     }
-    for (int k = 0; k < 12; ++k) res->stats[k] = big->stats[k];          // timings of the batch the pair rode in
-    res->stats[6] = (double)ref_len * (double)read_len; res->stats[7] = 1; res->stats[8] = (double)n;
-    res->stats[11] = (double)coalesced;                                   // requests served by that batch
+    for (int k = 0; k < STAT_COUNT; ++k) res->stats[k] = big->stats[k];  // timings of the batch the pair rode in
+    res->stats[STAT_CELLS] = (double)ref_len * (double)read_len; res->stats[STAT_PAIRS] = 1; res->stats[STAT_MAX_CELLS] = (double)n;
+    res->stats[STAT_BATCHES] = (double)coalesced;                         // requests served by that batch
     res->fetched = true;
     ctx->live.fetch_add(1);
     return res.release();

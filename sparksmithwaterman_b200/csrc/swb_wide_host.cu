@@ -2,8 +2,6 @@
 // workspace, band tickets, flag -> locate -> sort -> trace, results appended as BatchOut.
 #include "swb_host.h"
 
-#include <functional>
-
 namespace swbh {
 
 using namespace swb::wide;
@@ -24,12 +22,8 @@ static int pick_kl(int64_t m)
     return best;
 }
 
-int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const std::vector<int32_t> &reads,
-                  int match, int mismatch, int gap, uint32_t flags, swb_result *res, int *launches, int *n_batches,
-                  double *ck_bytes, const std::function<cudaError_t(int)> &tic, const std::function<cudaError_t()> &toc,
-                  const std::vector<std::vector<int32_t>> *refs_of)
+int AlignCall::run_wide_path(const std::vector<int32_t> &reads, bool scores_only, const std::vector<std::vector<int32_t>> *refs_of)
 {
-    cudaStream_t st = ctx->stream;
     const int64_t n_refs = rs->n_refs, n_reads = rd->n_reads;
 
     // ---- the wide reads, 16-byte aligned and padded to whole bands (0xFE: matches nothing) ----------------
@@ -51,7 +45,7 @@ int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const
         CU(cudaMemcpyAsync(ctx->w_wreads.p, reads.data(), reads.size() * 4, cudaMemcpyHostToDevice, st));
         CU(launch_wide_pad_reads(rd->codes.p, rd->off.p, ctx->w_wreads.p, (int)reads.size(), ctx->w_rpad_off.p,
                                  ctx->w_rpad_len.p, ctx->w_rpad.p, max_len, st));
-        ++*launches;
+        ++launches;
         CU(cudaStreamSynchronize(st));      // the host tables above are locals
     }
 
@@ -88,8 +82,8 @@ int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const
             bytes += b; ++k1;
         }
         const int np = (int)(k1 - k0);
-        ++*n_batches;
-        *ck_bytes += (double)bytes;
+        ++n_batches;
+        ck_bytes += (double)bytes;
         std::vector<int64_t> band_off((size_t)np + 1), blk_off((size_t)np + 1), brow_off((size_t)np + 1);
         std::vector<int2> items;
         int64_t nbands = 0, nblk = 0;
@@ -144,13 +138,13 @@ int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const
         }
         uint32_t *d_ntasks = ctx->counters.p, *d_ncells = ctx->counters.p + 1, *d_ticket = ctx->counters.p + 2;
 
-        CU(tic(1));
+        CU(timer.begin(STAT_FILL_MS));
         CU(launch_wide_fill(KL, P, ctx->w_items.p, (int)items.size(), d_ticket, ctx->sm_count, st));
-        ++*launches;
-        CU(toc());
-        if (flags & SWB_F_SCORES_ONLY) { CU(cudaStreamSynchronize(st)); k0 = k1; continue; }
+        ++launches;
+        CU(timer.end());
+        if (scores_only) { CU(cudaStreamSynchronize(st)); k0 = k1; continue; }
 
-        CU(tic(2));
+        CU(timer.begin(STAT_LOCATE_MS));
         uint32_t cap_tasks = (uint32_t)std::min<int64_t>((int64_t)np * 4 + 4096, (int64_t)1 << 30);
         uint32_t cap_cells = cap_tasks;
         uint32_t h_counts[2] = {0, 0};
@@ -161,7 +155,7 @@ int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const
             CU(launch_wide_flag(P, nblk, ctx->w_tasks.p, cap_tasks, d_ntasks, ctx->sm_count, st));
             CU(launch_wide_locate(KL, P, ctx->w_tasks.p, d_ntasks, cap_tasks, ctx->keys_tmp.p, cap_cells, d_ncells,
                                   ctx->sm_count, st));
-            *launches += 2;
+            launches += 2;
             CU(cudaMemcpyAsync(h_counts, ctx->counters.p, 8, cudaMemcpyDeviceToHost, st));
             CU(cudaStreamSynchronize(st));
             if (h_counts[0] <= cap_tasks && h_counts[1] <= cap_cells) break;
@@ -180,10 +174,10 @@ int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const
         const size_t tmp_bytes = sort_keys_tmp_bytes(n_cells);
         CU(ctx->sort_tmp.reserve(tmp_bytes, st));
         CU(sort_keys(ctx->keys_tmp.p, bo.keys.p, n_cells, ctx->sort_tmp.p, tmp_bytes, st));
-        *launches += 4;
-        CU(toc());
+        launches += 4;
+        CU(timer.end());
 
-        CU(tic(3));
+        CU(timer.begin(STAT_TRACE_MS));
         // longest alignment of a positive-score path: m rows + the deletions its score can pay for
         const int64_t big = std::max({match, mismatch, 0});
         int64_t lmax = (int64_t)m_max + n_max;
@@ -203,8 +197,8 @@ int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const
             P.mail = ctx->w_mail.p; P.mail_latest = ctx->w_mail.p + (size_t)n_cells * (size_t)stride * 8; P.mail_stride = (int32_t)stride;
         }
         CU(launch_wide_trace(KL, P, bo.keys.p, n_cells, bo.beg.p, bo.oplen.p, bo.ops.p, bo.ops_stride, ctx->sm_count, st));
-        ++*launches;
-        CU(toc());
+        ++launches;
+        CU(timer.end());
         CU(cudaStreamSynchronize(st));      // the host tables of this batch are reused by the next one
         if (P.dbg) {
             unsigned long long h[16];
@@ -213,7 +207,7 @@ int run_wide_path(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, const
                             "cycles (first thread of every CTA): prepare %llu, token wait %llu, consume %llu (chain %llu, re-walk %llu, append %llu)\n",
                     KL, np, n_cells, h[0], h[2], h[1], h[5], h[11], h[3], h[6], h[4], h[8], h[9], h[10]);
         }
-        res->stats[8] += n_cells;
+        res->stats[STAT_MAX_CELLS] += n_cells;
         res->batches.push_back(std::move(bo));
         k0 = k1;
     }

@@ -71,7 +71,7 @@ def test_cfg2_sample(engine):
 
 
 def test_long_references_are_segmented_exactly(engine):
-    """References longer than two fill segments are cut into overlapping windows (swb_api.cu
+    """References longer than two fill segments are cut into overlapping windows (swb_align.cu
     make_segments); results must not depend on it: reads planted across segment boundaries,
     a tie-heavy long repeat (max cells in every segment), scores with long gap runs."""
     rnd = random.Random(77)

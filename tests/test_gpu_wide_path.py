@@ -109,7 +109,7 @@ def test_few_long_walks_cluster_traceback(engine, tie_gt, scores):
 def test_mismatch_above_match_leaves_the_s16_path(engine, scores):
     """A positive mismatch above the match score makes the maximum about max(match, mismatch) * min(m, n): with
     200-256 bp reads that leaves int16 although every single score is small, so these inputs must take the int32
-    wide path (the s16x2 gate bounds the score with max(match, mismatch, 0), swb_api.cu)."""
+    wide path (the s16x2 gate bounds the score with max(match, mismatch, 0), swb_align.cu)."""
     rnd = random.Random(81)
     refs = [_rand(rnd, n) for n in (240, 300, 520, 257)]
     reads = [_rand(rnd, m) for m in (200, 230, 256)] + [refs[2][100:350]]
