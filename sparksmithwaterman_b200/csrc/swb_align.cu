@@ -113,9 +113,8 @@ void AlignCall::classify_reads(std::vector<std::vector<int32_t>> &classes, std::
     const bool short_scores_ok = rs->two_bit_ok && gap < 0 && std::abs((int64_t)match) <= 8000 &&
                                  std::abs((int64_t)mismatch) <= 8000 && std::abs((int64_t)gap) <= 8000;
     // reads of 257 .. 511 rows: the LONG classes (K = 40 .. 64) exist for the biased fill and the tile kernels only;
-    // other score sets send such reads through the wide path as before (SWB_NO_LONG_CLASSES=1: always)
-    static const bool no_long = getenv("SWB_NO_LONG_CLASSES") != nullptr;
-    const bool long_kernels_ok = !no_long && tile_trace_ok(match, mismatch, gap);
+    // other score sets send such reads through the wide path
+    const bool long_kernels_ok = tile_trace_ok(match, mismatch, gap);
     for (int64_t q = 0; q < rd->n_reads; ++q) {
         const int m = rd->len[(size_t)q];
         if (m == 0) continue;                                  // score 0, no cells

@@ -138,7 +138,7 @@ void swb_destroy(swb_ctx *c)
     cudaStreamSynchronize(c->stream);
     c->ck.release(); c->tmx.release(); c->counters.release(); c->rp.release();
     c->tasks.release(); c->task_hits.release(); c->keys_tmp.release(); c->sort_tmp.release();
-    c->w_brow.release(); c->w_rec.release(); c->w_wreads.release(); c->w_rpad.release(); c->w_rpad_off.release(); c->w_rpad_len.release(); c->w_dbg.release(); c->w_mail.release(); c->w_tmx.release(); c->w_prog.release(); c->w_pair_ref.release();
+    c->w_brow.release(); c->w_rec.release(); c->w_wreads.release(); c->w_rpad.release(); c->w_rpad_off.release(); c->w_rpad_len.release(); c->w_mail.release(); c->w_tmx.release(); c->w_pair_ref.release();
     c->w_pair_read.release(); c->w_band_off.release(); c->w_blk_off.release(); c->w_brow_off.release();
     c->w_items.release(); c->w_tasks.release(); c->hit_tmp.release(); c->hit_sel.release();
     for (cudaEvent_t e : c->ev_pool) cudaEventDestroy(e);
@@ -257,8 +257,6 @@ static int build_leaf(swb_ctx *ctx, int64_t n_refs, const int64_t *offsets, cons
 // (74 bytes per base and read pair) in the workspace, so that a typical call is one batch per part
 static int part_count(const swb_ctx *ctx, int64_t total_bases, int64_t n_refs)
 {
-    static const int env_parts = getenv("SWB_REF_PARTS") ? atoi(getenv("SWB_REF_PARTS")) : 0;
-    if (env_parts > 0) return (int)std::min<int64_t>(env_parts, std::max<int64_t>(n_refs, 1));
     const double part_bases = (double)ctx->ws_bytes / (74.0 * 96.0);
     int s = (int)((double)total_bases / std::max(part_bases, 1.0) + 0.5);
     if (s >= 2) ++s;                  // one more, smaller, last part: 8 ranks of one box pull their results at the same moment and share the host's memory bandwidth (measured 8 x B200: 120 MB per rank in 3.7 ms exposed with 2 parts)

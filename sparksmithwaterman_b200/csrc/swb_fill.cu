@@ -212,13 +212,10 @@ static cudaError_t launch_fill_k(const BatchParams &P, uint32_t *work_counter, i
 {
     using G = Geo<K>;
     const int n_quads = (P.n_vrefs + 3) / 4;
-    static const int env_warps = getenv("SWB_FILL_WARPS") ? atoi(getenv("SWB_FILL_WARPS")) : 0;
-    static const int env_ctas = getenv("SWB_FILL_CTAS_PER_SM") ? atoi(getenv("SWB_FILL_CTAS_PER_SM")) : 0;
-    const int warps = env_warps > 0 ? env_warps : 12;
-    const int ctas_per_sm = env_ctas > 0 ? env_ctas : 1;   // one CTA per SM: measured 54 ms vs 69 ms for two (warp starvation)
+    const int warps = 12;
     const int64_t items = (int64_t)n_quads * P.n_rp;
-    // persistent CTAs, never more than there is work
-    const int64_t ctas = std::min<int64_t>((items + warps - 1) / warps, (int64_t)sm_count * ctas_per_sm);
+    // persistent CTAs, never more than there is work; one CTA per SM: measured 54 ms vs 69 ms for two (warp starvation)
+    const int64_t ctas = std::min<int64_t>((items + warps - 1) / warps, (int64_t)sm_count);
     const size_t smem = (size_t)warps * G::PROF_WORDS * sizeof(uint32_t);
     cudaError_t e = cudaSuccess;
     {

@@ -297,9 +297,8 @@ static cudaError_t launch_fill_bias_k2(const BatchParams &P, uint32_t *work_coun
 {
     using G = Geo<K>;
     const int n_quads = (P.n_vrefs + 3) / 4;
-    static const int env_warps = getenv("SWB_FILL_WARPS") ? atoi(getenv("SWB_FILL_WARPS")) : 0;
     const int max_warps = fill_bias_threads(K) / 32;
-    const int warps = std::min(env_warps > 0 ? env_warps : 16, max_warps);   // measured (K = 19): 10/12/14/16 warps -> 42.0/39.8/39.4/39.2 ms
+    const int warps = std::min(16, max_warps);   // measured (K = 19): 10/12/14/16 warps -> 42.0/39.8/39.4/39.2 ms
     const int64_t items = (int64_t)n_quads * P.n_rp;
     const int64_t ctas = std::min<int64_t>((items + warps - 1) / warps, (int64_t)sm_count);   // one CTA per SM
     const size_t smem = (size_t)warps * G::PROF_WORDS * sizeof(uint32_t);
@@ -354,8 +353,7 @@ cudaError_t launch_fill_bias(int K, const BatchParams &P, uint32_t *work_counter
 // behind a tracked maximum of 0, i.e. one match has to exceed the slack (then score_lo == 0 implies score == 0).
 int fill_sub_slack(int match, int mismatch, int gap)
 {
-    static const bool disabled = getenv("SWB_NO_SUBSAMPLE") != nullptr;
-    if (disabled || gap >= 0) return 0;
+    if (gap >= 0) return 0;
     const int ag = -gap;
     const int diag = mismatch >= 0 ? 0 : std::min(-mismatch, 2 * ag);   // (r+1, u+1) >= H + max(mismatch, 2 gap)
     const int slack = std::max(ag, diag);
@@ -366,8 +364,7 @@ bool fill_bias_ok(int match, int mismatch, int gap, int64_t max_score)
 {
     if (gap >= 0) return false;
     const int ag = -gap;
-    static const bool disabled = getenv("SWB_NO_BIAS_FILL") != nullptr;
-    return !disabled && match + ag >= 0 && mismatch + ag >= 0 && match + ag <= 4000 && mismatch + ag <= 4000 &&
+    return match + ag >= 0 && mismatch + ag >= 0 && match + ag <= 4000 && mismatch + ag <= 4000 &&
            max_score + 32LL * ag <= 30000;
 }
 

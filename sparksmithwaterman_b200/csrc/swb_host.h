@@ -167,10 +167,9 @@ struct swb_ctx {
     DevBuf<uint64_t> keys_tmp;
     DevBuf<uint8_t> sort_tmp;
     // wide (int32, long-pair) path scratch
-    DevBuf<int32_t> w_brow, w_rec, w_tmx, w_prog, w_pair_ref, w_pair_read, w_wreads;
+    DevBuf<int32_t> w_brow, w_rec, w_tmx, w_pair_ref, w_pair_read, w_wreads;
     DevBuf<uint8_t> w_rpad;                     // wide reads, aligned + padded (0xFE) to whole bands
     DevBuf<int64_t> w_rpad_off, w_rpad_len;
-    DevBuf<unsigned long long> w_dbg;
     DevBuf<int32_t> w_mail;                     // tokens of the pipelined CTA-wide traceback
     DevBuf<int64_t> w_band_off, w_blk_off, w_brow_off;
     DevBuf<int2> w_items;

@@ -165,7 +165,6 @@ struct WideParams {
     int32_t *mail_latest;        // [cells] highest token index published
     int32_t mail_stride;         // tokens per cell = rounds + 2
     int32_t pipe_c;              // CTAs per cell (cluster size), set by the launcher
-    unsigned long long *dbg;     // optional counters (SWB_WIDE_DEBUG): [0] traceback rounds, [1] tiles walked, [2] tiles recomputed
 };
 
 // one batch of max cells as the assembly kernels see it (swb_assemble.cu)
@@ -236,8 +235,6 @@ cudaError_t launch_tile_trace(int K, const BatchParams &P, const uint64_t *keys,
                               int32_t *beginnings, int32_t *op_lens, uint32_t *ops, int ops_stride_words,
                               int sm_count, cudaStream_t st);
 bool tile_trace_ok(int match, int mismatch, int gap);
-cudaError_t launch_cell_offsets(const uint64_t *keys, uint32_t n_cells, const int64_t *pair_ids, int64_t n_pairs,
-                                int64_t *offsets, cudaStream_t st);
 cudaError_t launch_ref_totals(const int32_t *scores, int64_t n_refs, int64_t n_reads, int32_t *totals, cudaStream_t st);
 cudaError_t launch_best_hits(const int32_t *scores, int64_t n_refs, int64_t n_reads, int32_t *best, int sm_count, cudaStream_t st);
 cudaError_t sort_keys(uint64_t *keys_in, uint64_t *keys_out, uint32_t n, void *tmp, size_t tmp_bytes, cudaStream_t st);

@@ -9,7 +9,7 @@
 //                scores with the priority of the ">=" cascade (:228,:236,:245): alignment, then insertion, then
 //                deletion.  Blocks are recomputed lazily, right to left, each from its own checkpoints (all 8
 //                lanes of the group), so every H the walk reads is exact.
-//   ref_totals, best_hits, cell_offsets, key sort: the per-call reductions of Distribution.MapRef (:424) and
+//   ref_totals, best_hits, key sort: the per-call reductions of Distribution.MapRef (:424) and
 //                the best-hit records merged across GPUs.
 // Max-cell enumeration and the default traceback live in swb_trace_tile.cu.
 #include "swb_internal.h"
@@ -501,28 +501,6 @@ cudaError_t launch_trace(int K, const BatchParams &P, const uint64_t *keys, uint
 }
 
 // ---------------------------------------------------------------------------------------
-// offsets[k] = first sorted key whose pair id >= pair_ids[k]  (pair_ids ascending; last = +inf)
-__global__ void cell_offsets_kernel(const uint64_t *keys, uint32_t n_cells, const int64_t *pair_ids, int64_t n_pairs,
-                                    int64_t *offsets)
-{
-    const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (k > n_pairs) return;
-    if (k == n_pairs) { offsets[k] = n_cells; return; }
-    const uint64_t target = make_key((uint64_t)pair_ids[k], 0, 0);
-    uint32_t lo = 0, hi = n_cells;
-    while (lo < hi) { const uint32_t mid = lo + ((hi - lo) >> 1); if (keys[mid] < target) lo = mid + 1; else hi = mid; }
-    offsets[k] = lo;
-}
-
-cudaError_t launch_cell_offsets(const uint64_t *keys, uint32_t n_cells, const int64_t *pair_ids, int64_t n_pairs,
-                                int64_t *offsets, cudaStream_t st)
-{
-    const int threads = 256;
-    const int64_t blocks = (n_pairs + 1 + threads - 1) / threads;
-    cell_offsets_kernel<<<(unsigned)blocks, threads, 0, st>>>(keys, n_cells, pair_ids, n_pairs, offsets);
-    return cudaGetLastError();
-}
-
 // per-reference wrapping int32 total over reads (Distribution.java:424): one warp per ref
 __global__ void ref_totals_kernel(const int32_t *scores, int64_t n_refs, int64_t n_reads, int32_t *totals)
 {

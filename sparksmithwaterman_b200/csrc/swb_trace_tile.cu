@@ -580,8 +580,7 @@ cudaError_t launch_tile_trace_k(const BatchParams &P, const uint64_t *keys, uint
     // chunks of the sorted cell list: many per SM for balance, each long enough to amortise its profile.  In hits mode
     // (P.sel) a read has a handful of cells: a CTA walks its chunk's reads one after another, so a chunk of 2 * NT
     // cells would serialise up to 2 * NT walks in one CTA; every cell may start a chunk of its own there.
-    static const int env_div = getenv("SWB_TRACE_CHUNKS_PER_SM") ? atoi(getenv("SWB_TRACE_CHUNKS_PER_SM")) : 0;
-    const int per_sm = env_div > 0 ? env_div : 16;
+    const int per_sm = 16;
     const int chunk = (int)std::max<int64_t>(P.sel ? 1 : 2 * NT, ((int64_t)n_cells + (int64_t)sm_count * per_sm - 1) / ((int64_t)sm_count * per_sm));
     const int64_t ctas = ((int64_t)n_cells + chunk - 1) / chunk;
     if (P.tie_gt) tile_trace_kernel<K, true><<<(unsigned)ctas, NT, smem, st>>>(P, keys, n_cells, chunk, beginnings, op_lens, ops, ops_stride, 65536u);
@@ -594,8 +593,7 @@ cudaError_t launch_tile_trace_k(const BatchParams &P, const uint64_t *keys, uint
 // Equality of the low 8 bits must be equality: a candidate lies at most 2*(smax+|gap|) + max|s| below H.
 bool tile_trace_ok(int match, int mismatch, int gap)
 {
-    static const bool disabled = getenv("SWB_NO_TILE_TRACE") != nullptr;
-    if (disabled || gap >= 0) return false;
+    if (gap >= 0) return false;
     const int64_t smax = std::max<int64_t>({match, mismatch, 0});
     const int64_t sabs = std::max<int64_t>(std::llabs((long long)match), std::llabs((long long)mismatch));
     return 2 * (smax - (int64_t)gap) + sabs < 250;

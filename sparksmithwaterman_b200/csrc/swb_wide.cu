@@ -12,9 +12,9 @@
 //     DPX ops (VIADDMNMX.RELU, VIADDMNMX) on the integer pipe -- SmithWaterman.java:217-252, :277-280,
 //     :309-318;
 //   * consecutive bands of a pair run concurrently on different warps, coupled through the band's
-//     bottom row in HBM (brow) and a per-band progress counter (release / acquire).  Work is handed
-//     out by a global ticket in (band, pair) order, so a warp only ever waits for a lower ticket,
-//     which is held by a running warp: no deadlock, no cooperative launch;
+//     bottom row in HBM (brow), whose words validate themselves (no counter, no fence; see ld_relaxed).
+//     Work is handed out by a global ticket in (band, pair) order, so a warp only ever waits for a
+//     lower ticket, which is held by a running warp: no deadlock, no cooperative launch;
 //   * the fill is score-only and leaves, per (band, block of 32 steps, lane), one contiguous RECORD:
 //     the lane's CHECKPOINT (KL cells + the diagonal boundary at the block start) and its SEAM (the
 //     boundary row it receives at each of the 32 steps), plus the lane's tile maximum.  A record is
@@ -288,7 +288,7 @@ wide_fill_kernel(const WideParams P, const int2 *items, int n_items, uint32_t *t
                     if (feeds_below && lane == WL - 1) st_relaxed(my_brow + s0 + u, H[KL - 1]);
                 }
             }
-            // ---- block boundary: tile maximum, next block's checkpoint, progress
+            // ---- block boundary: tile maximum, next block's checkpoint
             tmxp[(int64_t)ch * WL] = tmax;
             bmax = max(bmax, tmax);
             tmax = 0;
@@ -682,7 +682,6 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                         cacc |= (uint32_t)c << (8 * (u & 3));
                         if ((u & 3) == 3) { cw[KL / 4 + (u >> 2)] = cacc; cacc = 0; }
                     });
-                    if (P.dbg) atomicAdd(P.dbg + 2, 1ull);
                 }
                 slot_blk[tg] = myblk;
             }
@@ -740,7 +739,6 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
             };
             for (;;) {
                 // ---- (a) chain
-                const long long dc0 = P.dbg ? clock64() : 0;
                 int nv = 0, hc = hcur, xi = ci, xj = cj;
                 int my_slot = 0, my_r = 0, my_c = 0, my_n = 0;
                 if (hc > 0 && xi >= 1 && xj >= 1) {
@@ -778,9 +776,7 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                 }
                 if (nv > 0) {
                     // lane v: the moves of visit v (walk order), 2 bits each
-                    const long long dc1 = P.dbg ? clock64() : 0;
                     unsigned long long lo = 0, hi = 0;
-                    int last_beg = 0;
                     if (wl < nv) {
                         const uint8_t *base = reinterpret_cast<const uint8_t *>(slots + (size_t)my_slot * TW);
                         const uint8_t *p = base + my_c * COLB + my_r * ES;
@@ -796,9 +792,7 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                             p -= up * ES + left * COLB;
                             if (k < 32) lo |= (unsigned long long)op << (2 * k); else hi |= (unsigned long long)op << (2 * k - 64);
                         }
-                        (void)last_beg;
                     }
-                    const long long dc2 = P.dbg ? clock64() : 0;
                     const int n = wl < nv ? my_n : 0;
                     int pn = n;
 #pragma unroll
@@ -831,11 +825,6 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                     __syncwarp();
                     oplen = oplen_new;
                     hcur = hc; ci = xi; cj = xj;
-                    if (P.dbg && wl == 0) {
-                        atomicAdd(P.dbg + 5, (unsigned long long)nv);
-                        atomicAdd(P.dbg + 8, (unsigned long long)(dc1 - dc0)); atomicAdd(P.dbg + 9, (unsigned long long)(dc2 - dc1));
-                        atomicAdd(P.dbg + 10, (unsigned long long)(clock64() - dc2)); atomicAdd(P.dbg + 11, 1ull);
-                    }
                     continue;
                 }
                 // ---- (b) exact walker (SmithWaterman.java:380-409), one tile visit, all 32 lanes in lock step: lane k probes
@@ -853,7 +842,6 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                 slot += dd;
                 int r = ci - T * KL;                           // 1..KL
                 int c = step - b * WCB + 1;                    // 1..WCB
-                if (P.dbg && wl == 0) atomicAdd(P.dbg + 1, 1ull);
                 const uint8_t *base = reinterpret_cast<const uint8_t *>(slots + (size_t)slot * TW);
                 const uint8_t *p = base + c * COLB + r * ES;
                 const uint8_t *pr = base + TG::CODE0 * 4 + (r - 1);
@@ -915,9 +903,7 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
             __syncthreads();
             if (tdone) break;
             const int row_r = r == 0 ? ci0 : (Tr_hi + 1) * KL;
-            const long long dbg_t0 = P.dbg ? clock64() : 0;
             prepare(row_r, tcj - (tci - row_r), Tr_lo);
-            const long long dbg_t1 = P.dbg ? clock64() : 0;
             // ---- 2. the round's token
             if (r > 0) {
                 if (threadIdx.x == 0) {
@@ -938,7 +924,6 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                 __syncthreads();
                 if (done) break;
             }
-            const long long dbg_t2 = P.dbg ? clock64() : 0;
             // ---- 3. walk the round's lane-rows
             bool first = true;
             for (;;) {
@@ -953,7 +938,6 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                 __syncthreads();
                 if (!first && ci == ci_before && cj == cj_before) hcur = 0;   // cannot happen (a corridor around the true cell holds it); never spin
                 first = false;
-                if (P.dbg && threadIdx.x == 0) atomicAdd(P.dbg, 1ull);
                 if (hcur <= 0 || ci < 1 || cj < 1 || (ci - 1) / KL < Tr_lo) break;
             }
             // ---- 4. publish the next token
@@ -970,7 +954,6 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                     beginnings[cell] = beginning;
                     op_lens[cell] = (int32_t)oplen;
                 }
-                if (P.dbg) { atomicAdd(P.dbg + 3, (unsigned long long)(dbg_t1 - dbg_t0)); atomicAdd(P.dbg + 6, (unsigned long long)(dbg_t2 - dbg_t1)); atomicAdd(P.dbg + 4, (unsigned long long)(clock64() - dbg_t2)); }
             }
             if (done) break;
         }
@@ -994,7 +977,6 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
             const int T0 = (ci - 1) / KL;
             const int k = tg / DB, d = tg % DB;
             const int Tk = T0 - k;
-            const long long dbg_t0 = P.dbg ? clock64() : 0;
             int myblk = -1;
             if (tg >= 0 && Tk >= 0) {
                 const int t = Tk % WL;
@@ -1019,10 +1001,8 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                 });
             }
             if (tg >= 0) slot_blk[myslot] = myblk;
-            if (P.dbg) { if (gl == 0) atomicAdd(P.dbg, 1ull); if (myblk >= 0) atomicAdd(P.dbg + 2, 1ull); }
             if (G == 32) __syncwarp(gmask);
             else if (G > 32) __syncthreads();
-            const long long dbg_t1 = P.dbg ? clock64() : 0;
             if (G == 1) {
                 // ---- walk (SmithWaterman.java:380-409): one thread per max cell
                 for (;;) {
@@ -1041,7 +1021,6 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                     }
                     int r = ci - T * KL;                           // 1..KL
                     int c = step - b * WCB + 1;                    // 1..WCB
-                    if (P.dbg) atomicAdd(P.dbg + 1, 1ull);
                     const uint8_t *base = reinterpret_cast<const uint8_t *>(slots + (size_t)slot * TW);
                     const uint8_t *p = base + c * COLB + r * ES;   // element (r, c)
                     const uint8_t *pr = base + TG::CODE0 * 4 + (r - 1);          // read code of row r
@@ -1124,7 +1103,6 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                     }
                     int r = ci - T * KL;                           // 1..KL
                     int c = step - b * WCB + 1;                    // 1..WCB
-                    if (P.dbg && wl == 0) atomicAdd(P.dbg + 1, 1ull);
                     const uint8_t *base = reinterpret_cast<const uint8_t *>(slots + (size_t)slot * TW);
                     const uint8_t *p = base + c * COLB + r * ES;   // element (r, c)
                     const uint8_t *pr = base + TG::CODE0 * 4 + (r - 1);          // read code of row r
@@ -1171,7 +1149,6 @@ __global__ void __launch_bounds__(NT) wide_trace_kernel(const WideParams P, cons
                     if (hcur <= 0) break;
                 }
             }
-            if (P.dbg && gl == 0) { atomicAdd(P.dbg + 3, (unsigned long long)(dbg_t1 - dbg_t0)); atomicAdd(P.dbg + 4, (unsigned long long)(clock64() - dbg_t1)); }
             if (G == 32) {
                 __syncwarp(gmask);                                 // every lane walked: the state is already uniform
             } else if (G > 32) {
@@ -1197,10 +1174,8 @@ cudaError_t launch_fill_k(const WideParams &P, const int2 *items, int n_items, u
 {
     constexpr int PW = NC > 0 ? NC * KL * WL : 0, SW = 2 * (WL + 16);
     const size_t smem = (size_t)4 * (PW + SW) * sizeof(int32_t);
-    static const int env_ctas = getenv("SWB_WIDE_CTAS_PER_SM") ? atoi(getenv("SWB_WIDE_CTAS_PER_SM")) : 0;
     int per_sm = KL >= 32 ? 2 : 4;                                          // registers (__launch_bounds__)
     per_sm = std::min<int>(per_sm, (int)((220 * 1024) / (smem + 1024)));    // shared memory
-    if (env_ctas > 0) per_sm = std::min(per_sm, env_ctas);
     per_sm = std::max(per_sm, 1);
     const int ctas = (int)std::min<int64_t>(((int64_t)n_items + 3) / 4, (int64_t)sm_count * per_sm);
     cudaError_t e = cudaFuncSetAttribute(wide_fill_kernel<KL, NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -1212,9 +1187,8 @@ cudaError_t launch_fill_k(const WideParams &P, const int2 *items, int n_items, u
 template <int KL>
 cudaError_t launch_fill_kl(const WideParams &P, const int2 *items, int n_items, uint32_t *ticket, int sm_count, cudaStream_t st)
 {
-    static const bool no_prof = getenv("SWB_WIDE_NO_PROFILE") != nullptr;
-    if (P.gap < 0 && P.n_symbols <= 4 && !no_prof) return launch_fill_k<KL, 4>(P, items, n_items, ticket, sm_count, st);
-    if (P.gap < 0 && P.n_symbols <= 8 && !no_prof) return launch_fill_k<KL, 8>(P, items, n_items, ticket, sm_count, st);
+    if (P.gap < 0 && P.n_symbols <= 4) return launch_fill_k<KL, 4>(P, items, n_items, ticket, sm_count, st);
+    if (P.gap < 0 && P.n_symbols <= 8) return launch_fill_k<KL, 8>(P, items, n_items, ticket, sm_count, st);
     return launch_fill_k<KL, 0>(P, items, n_items, ticket, sm_count, st);
 }
 
@@ -1241,13 +1215,11 @@ cudaError_t launch_trace_pipe(const WideParams &P0, const uint64_t *keys, uint32
     const size_t smem = TraceGeo<KL, true>::smem_bytes(CTAW_TILES) + (size_t)SUB_SMEM_WORDS * 4;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    static const int env_c = getenv("SWB_WIDE_PIPE") ? atoi(getenv("SWB_WIDE_PIPE")) : 0;
     // CTAs per cell.  Measured on cfg3 (ten 100 kbp pairs): 1 / 2 / 3 / 4 / 8 CTAs -> 9.3 / 4.9 / 4.7 / 5.6 / 7.8 ms.  Three keep one
     // prepare hidden behind two walks; more only lengthen the distance over which the entry point is predicted (the
     // path drifts off the predicted diagonal and the prepared corridor has to be redone).
     int c = 3;
     while (c > 1 && (int64_t)n_cells * c > (int64_t)sm_count) --c;           // every cluster resident at once
-    if (env_c > 0) c = std::min(env_c, 8);
     WideParams P = P0;
     for (;; --c) {
         cudaLaunchConfig_t cfg = {};
@@ -1272,10 +1244,9 @@ cudaError_t launch_trace_kl(const WideParams &P, const uint64_t *keys, uint32_t 
                             int32_t *op_lens, uint32_t *ops, int64_t ops_stride, int sm_count, cudaStream_t st)
 {
     const bool bytes = tile_trace_ok(P.match, P.mismatch, P.gap);        // same bound as the short path's byte tiles
-    static const int env_g = getenv("SWB_WIDE_TRACE_G") ? atoi(getenv("SWB_WIDE_TRACE_G")) : 0;
     // lanes per max cell: a whole CTA (corridor of 32 lane-rows x 4 blocks) while there are fewer cells than SMs, a warp
     // (16 x 2) while the cells cannot fill the machine with one thread each, else one thread per cell
-    const int g = env_g ? env_g : ((int64_t)n_cells <= (int64_t)sm_count ? 128 : ((int64_t)n_cells < (int64_t)sm_count * 256 ? 32 : 1));
+    const int g = (int64_t)n_cells <= (int64_t)sm_count ? 128 : ((int64_t)n_cells < (int64_t)sm_count * 256 ? 32 : 1);
     constexpr int NTB = KL >= 32 ? 64 : 128;                              // byte tiles: 80 / 91 / 56 KB per CTA
     if (bytes) {
         if (g >= 128 && P.mail) return launch_trace_pipe<KL>(P, keys, n_cells, beginnings, op_lens, ops, ops_stride, sm_count, st);

@@ -9,8 +9,6 @@ using namespace swb::wide;
 // rows per lane for a read of m rows: the band count times the per-step cost of a band (3 ops per row + ~25 per step)
 static int pick_kl(int64_t m)
 {
-    static const int env_kl = getenv("SWB_WIDE_KL") ? atoi(getenv("SWB_WIDE_KL")) : 0;
-    if (env_kl == 8 || env_kl == 16 || env_kl == 32) return env_kl;
     int best = 0;
     int64_t best_cost = 0;
     for (int k = 0; k < kNumKL; ++k) {
@@ -129,13 +127,6 @@ int AlignCall::run_wide_path(const std::vector<int32_t> &reads, bool scores_only
         P.band_off = ctx->w_band_off.p; P.blk_off = ctx->w_blk_off.p; P.brow_off = ctx->w_brow_off.p;
         P.brow = ctx->w_brow.p; P.rec = ctx->w_rec.p; P.tmx = ctx->w_tmx.p;
         P.scores = res->d_scores.p;
-        static const bool wide_debug = getenv("SWB_WIDE_DEBUG") != nullptr;
-        P.dbg = nullptr;
-        if (wide_debug) {
-            CU(ctx->w_dbg.reserve(16, st));
-            CU(cudaMemsetAsync(ctx->w_dbg.p, 0, 128, st));
-            P.dbg = ctx->w_dbg.p;
-        }
         uint32_t *d_ntasks = ctx->counters.p, *d_ncells = ctx->counters.p + 1, *d_ticket = ctx->counters.p + 2;
 
         CU(timer.begin(STAT_FILL_MS));
@@ -200,13 +191,6 @@ int AlignCall::run_wide_path(const std::vector<int32_t> &reads, bool scores_only
         ++launches;
         CU(timer.end());
         CU(cudaStreamSynchronize(st));      // the host tables of this batch are reused by the next one
-        if (P.dbg) {
-            unsigned long long h[16];
-            CU(cudaMemcpy(h, P.dbg, 128, cudaMemcpyDeviceToHost));
-            fprintf(stderr, "[swb wide] KL=%d pairs=%d cells=%u: traceback rounds=%llu, tiles: recomputed %llu, walked exactly %llu, chained %llu in %llu batches; "
-                            "cycles (first thread of every CTA): prepare %llu, token wait %llu, consume %llu (chain %llu, re-walk %llu, append %llu)\n",
-                    KL, np, n_cells, h[0], h[2], h[1], h[5], h[11], h[3], h[6], h[4], h[8], h[9], h[10]);
-        }
         res->stats[STAT_MAX_CELLS] += n_cells;
         res->batches.push_back(std::move(bo));
         k0 = k1;

@@ -1,13 +1,12 @@
 #!/usr/bin/env python
 """Throughput of whole batches of reads of one length against the cfg2-shaped reference set (10,000 lognormal
 references, 21.3 Mbp): where does the s16x2 path end?  Reads up to 256 rows use the classes K <= 32, reads of
-257 .. 511 rows the LONG classes K = 40 .. 64 (same kernels), longer reads the int32 wide path.  With
-SWB_NO_LONG_CLASSES=1 (second pass, in a child process) 257+ row reads take the wide path as they did before
-the long classes existed.
+257 .. 511 rows the LONG classes K = 40 .. 64 (same kernels), longer reads the int32 wide path.  The wide path's
+numbers for 257 .. 511 rows, from before the long classes, are kept in profiles/readlen_tput_r02.json.
 
     python tests/checks/run_readlen_tput.py --out profiles/readlen_tput_r02.json
 """
-import argparse, json, os, subprocess, sys, time
+import argparse, json, os, sys, time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
@@ -42,26 +41,13 @@ def run(cases):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=None)
-    ap.add_argument("--child", action="store_true")
     a = ap.parse_args()
-    if a.child:
-        print("JSON " + json.dumps(run([c for c in CASES if 256 < c[0] < 512])))
-        return
-    # the child first: it must see the whole HBM for its workspace
-    env = dict(os.environ, SWB_NO_LONG_CLASSES="1")
-    out = subprocess.run([sys.executable, os.path.abspath(__file__), "--child"], env=env, capture_output=True, text=True, timeout=900)
-    wide = []
-    for line in out.stdout.splitlines():
-        if line.startswith("JSON "):
-            wide = json.loads(line[5:])
     rows = run(CASES)
     doc = {"what": "whole batches of one read length x 10,000 references through swb_align (host buffers, incl. traceback)",
-           "rows": rows, "rows_with_SWB_NO_LONG_CLASSES": wide}
+           "rows": rows}
     if a.out:
         with open(a.out, "w") as f:
             json.dump(doc, f, indent=1)
-    for r in wide:
-        print("wide path:", r)
 
 
 if __name__ == "__main__":

@@ -276,3 +276,15 @@ def test_rows_per_lane_classes_cover_the_short_path():
         text = open(os.path.join(csrc, fname)).read()
         got = sorted(int(x) for x in re.findall(r"case (\d+):\s+return " + fn + r"<\1>", text))
         assert got == wanted, (fname, fn, got)
+
+
+def test_library_reads_only_documented_environment_variables():
+    """Every kernel and launch shape follows from the inputs: the library reads only the two variables INTEGRATION.md
+    documents, SWB_NCCL_LIB (where NCCL is) and SWB_QUEUE_LINGER_US (how long the submission queue waits for more
+    pairs), neither of which selects an implementation."""
+    csrc = os.path.join(ROOT, "sparksmithwaterman_b200", "csrc")
+    names = set()
+    for fname in sorted(os.listdir(csrc)):
+        with open(os.path.join(csrc, fname)) as f:
+            names.update(re.findall(r"getenv\s*\(\s*([^)]*?)\s*\)", f.read()))
+    assert names == {'"SWB_NCCL_LIB"', '"SWB_QUEUE_LINGER_US"'}, names

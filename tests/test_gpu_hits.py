@@ -1,10 +1,7 @@
 """GPU: hits mode (swb_align_hits).  Every case runs the plain call and the hits call on the same inputs: scores,
 totals and best hits must be the plain ones, the hit lists the numpy top k of the plain scores, every hit pair's
 cells / beginnings / op lengths / alignments the plain ones, and every other pair must have no cells."""
-import os
 import random
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -12,11 +9,10 @@ import pytest
 import oracle
 import sparksmithwaterman_b200 as swb
 from sparksmithwaterman_b200 import synth
+from tests.helpers import launched_kernels, launches, parts_workspace
 from tests.test_hits_host import top_hits_ref
 
 pytestmark = pytest.mark.gpu
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _rand(rnd, n, alphabet="ACGT"):
@@ -160,30 +156,22 @@ def test_hit_pairs_against_the_oracle(engine):
     hr.free(); rs.free()
 
 
-PARTS_SCRIPT = r"""
-import sys
-sys.path.insert(0, %r)
-import sparksmithwaterman_b200 as swb
-from sparksmithwaterman_b200 import synth
-from tests.test_gpu_hits import check_hits
-eng = swb.Engine(0)
-refs = synth.make_refs(90, lo=50, hi=3000)
-reads = synth.make_reads(10, 150, refs, seed=3) + synth.make_reads(3, 600, refs, seed=6)
-for k, ms in ((1, 1), (3, 1), (5, 60)):
-    check_hits(eng, refs, reads, k=k, min_score=ms)
-check_hits(eng, refs, reads, k=3, min_score=1, fetch=False)
-eng.close()
-print("checked")
-""" % ROOT
-
-
 def test_reference_set_in_three_parts():
     """A set cut into parts is aligned as one set in hits mode: this checks that a parted set gives the whole-set
     answer (the same hits and cells as the plain call on the parted set), not any per-part selection."""
-    env = dict(os.environ, SWB_REF_PARTS="3")
-    p = subprocess.run([sys.executable, "-c", PARTS_SCRIPT], env=env, cwd=ROOT, capture_output=True, text=True, timeout=600)
-    assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-4000:]
-    assert "checked" in p.stdout
+    refs = synth.make_refs(90, lo=50, hi=3000)
+    reads = synth.make_reads(10, 150, refs, seed=3) + synth.make_reads(3, 600, refs, seed=6)
+    eng = swb.Engine(0, workspace_bytes=parts_workspace(refs, 3))
+    try:
+        rs = eng.load_refset(refs)
+        res, kernels = launched_kernels(lambda: rs.align(reads))
+        assert len(launches(kernels, r"\bfold_best_kernel\b")) >= 2          # the plain call ran part by part
+        res.free(); rs.free()
+        for k, ms in ((1, 1), (3, 1), (5, 60)):
+            check_hits(eng, refs, reads, k=k, min_score=ms)
+        check_hits(eng, refs, reads, k=3, min_score=1, fetch=False)
+    finally:
+        eng.close()
 
 
 def _device_count():
