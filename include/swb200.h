@@ -45,6 +45,30 @@ extern "C" {
                                    on equal candidates deletion wins over insertion over alignment.  Scores and
                                    the max-cell SET are unchanged; cells are still listed row-major (the host
                                    layer re-orders them diagonal-major + stable by beginning, :209, :480)   */
+#define SWB_F_BOTH_STRANDS  8u  /* align every read as given AND its reverse complement (see BOTH STRANDS below) */
+
+/* BOTH STRANDS (SWB_F_BOTH_STRANDS; accepted by swb_align, swb_align_resident, swb_align_hits,
+ * swb_align_resident_hits, swb_multi_align and swb_multi_align_hits, combinable with every other flag;
+ * swb_align_pair refuses it with SWB_E_INVALID).  Sequencing reads come from either strand; this mode aligns
+ * each read q and its reverse complement rc(q) against every reference in the same call.
+ *   - the result has swb_result_n_refs == 2 * R ORIENTED references over the set's R references:
+ *     o = 2r is reference r with the read as given, o = 2r + 1 is reference r with rc(read).  Pair
+ *     p = o * n_reads + q; every accessor applies unchanged (scores, cell offsets, cells, beginnings,
+ *     op lengths, ops, pair_cell_count, pair_cell, hits).
+ *   - for an odd o, cell (i, j) has i = row of rc(read) (1-based) and j = column of reference r: positions are
+ *     forward-reference coordinates.  Beginnings, op lengths and ops are those of that alignment.
+ *   - ref_totals[o] sums over reads per oriented reference; best_hits[q] and the hit lists are taken over all 2R
+ *     oriented references with the usual rule (score descending, then lowest index): on a tie the lower reference
+ *     wins, and on the same reference the forward strand wins (a palindromic read reports o = 2r).
+ *   - swb_result_materialize takes the caller's ORIGINAL read; for a cell of an odd o it builds the read string
+ *     from rc(read), keeping case (a -> t).
+ *   - complement: the IUPAC DNA involution A<->T, C<->G, R<->Y, K<->M, B<->V, D<->H; S, W, N map to themselves
+ *     (case-insensitive).  A set with any other symbol is SWB_E_UNSUPPORTED for this mode.  Position i of rc(read)
+ *     matches nothing when read[m-1-i], or its complement, is absent from the set.
+ *   - stats out[6] / out[7] (cells, pairs) count both strands.
+ *   - multi-GPU: shard results are oriented over the shard's references; the merge works on oriented global ids
+ *     2 * global_ref + s, so the merged records equal one context's.  swb_comm_allgather_best / _hits take oriented
+ *     ids for a both-strands result: n_local_refs = 2 * shard refs, global_ids[2r + s] = 2 * gid(r) + s. */
 
 typedef struct swb_ctx    swb_ctx;     /* one CUDA device + streams + workspace                */
 typedef struct swb_refset swb_refset;  /* packed reference set resident in HBM                  */

@@ -52,6 +52,9 @@ final class NativeSW
 	static final MethodHandle PAIR_CELL   = h( "swb_result_pair_cell" , FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_LONG, JAVA_LONG, ADDRESS, ADDRESS, ADDRESS, ADDRESS) ) ;
 	static final MethodHandle MATERIALIZE = h( "swb_result_materialize" , FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_LONG, ADDRESS, JAVA_LONG, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_LONG) ) ;
 
+	/** swb_align flags (swb200.h); F_BOTH_STRANDS: every read and its reverse complement, o = 2r + strand */
+	static final int F_SCORES_ONLY = 1 , F_NO_FETCH = 2 , F_TIE_GT = 4 , F_BOTH_STRANDS = 8 ;
+
 	/** process-wide engine context (thread-safe on the native side) */
 	static final MemorySegment CTX = create() ;
 

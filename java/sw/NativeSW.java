@@ -66,6 +66,8 @@ final class NativeSW
 	static native void multiResultFree( long multiResult ) ;
 
 	static final int F_SCORES_ONLY = 1 , F_NO_FETCH = 2 , F_TIE_GT = 4 ;
+	/** every read and its reverse complement: results over 2 * nRefs oriented references, o = 2r + strand (swb200.h) */
+	static final int F_BOTH_STRANDS = 8 ;
 
 	/** process-wide engine context on CUDA device -Dswb.device (default 0); thread-safe on the native side */
 	private static long ctx = 0 ;

@@ -13,6 +13,7 @@ SWB_OK = 0
 SWB_F_SCORES_ONLY = 1
 SWB_F_NO_FETCH = 2
 SWB_F_TIE_GT = 4
+SWB_F_BOTH_STRANDS = 8
 
 # every symbol include/swb200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p

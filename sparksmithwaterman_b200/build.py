@@ -18,7 +18,7 @@ LIB = os.path.join(LIB_DIR, "libswb200.so")
 MICROBENCH = os.path.join(BIN_DIR, "dpx_microbench")
 PAIR_BENCH = os.path.join(BIN_DIR, "pair_bench")
 
-SOURCES = ["swb_api.cu", "swb_align.cu", "swb_fill.cu", "swb_fill_bias.cu", "swb_trace.cu", "swb_trace_tile.cu", "swb_wide.cu", "swb_wide_host.cu", "swb_multi.cu", "swb_queue.cu", "swb_assemble.cu", "swb_hits.cu", "dpx_microbench.cu"]
+SOURCES = ["swb_api.cu", "swb_align.cu", "swb_fill.cu", "swb_fill_bias.cu", "swb_trace.cu", "swb_trace_tile.cu", "swb_wide.cu", "swb_wide_host.cu", "swb_multi.cu", "swb_queue.cu", "swb_assemble.cu", "swb_hits.cu", "swb_strands.cu", "dpx_microbench.cu"]
 HEADERS = ["swb_internal.h", "swb_device.cuh", "swb_host.h", os.path.join("..", "..", "include", "swb200.h")]
 NVCC_FLAGS = ["-std=c++17", "-O3", "-lineinfo", "-gencode", "arch=compute_100a,code=sm_100a",
               "-Xcompiler", "-fPIC", "-cudart", "static"]

@@ -52,7 +52,8 @@ int pick_k(int m)
 int record_words(int K) { return ((K + 1 + 7) / 8 + CB / 8) * 8; }         // per (block, lane): Geo<K>::RW
 
 // a result of rs x rd; it counts as a live handle of its context from here on (swb_result_free releases it, also on the
-// error paths)
+// error paths).  SWB_F_BOTH_STRANDS: rd holds the 2n internal reads and the result is oriented, 2R references x n reads;
+// its cells and pairs count both strands.
 using ResultPtr = std::unique_ptr<swb_result, void (*)(swb_result *)>;
 ResultPtr new_result(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, uint32_t flags)
 {
@@ -60,6 +61,12 @@ ResultPtr new_result(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, ui
     ctx->live.fetch_add(1);
     res->ctx = ctx; res->n_refs = rs->n_refs; res->n_reads = rd->n_reads; res->flags = flags;
     res->ref_len = rs->len_orig; res->read_len = rd->len;
+    if (flags & SWB_F_BOTH_STRANDS) {
+        res->n_refs = 2 * rs->n_refs; res->n_reads = rd->n_reads / 2;
+        res->ref_len.resize((size_t)res->n_refs);
+        for (int64_t o = 0; o < res->n_refs; ++o) res->ref_len[(size_t)o] = rs->len_orig[(size_t)(o >> 1)];
+        res->read_len.resize((size_t)res->n_reads);
+    }
     int64_t read_bases = 0;
     for (int32_t m : rd->len) read_bases += m;
     res->stats[STAT_CELLS] = (double)rs->total_bases * (double)read_bases;
@@ -81,11 +88,11 @@ int AlignCall::run(int32_t *ext_scores, int32_t *ext_totals)
     const int64_t n_refs = rs->n_refs, n_reads = rd->n_reads;
     const size_t n_pairs = (size_t)(n_refs * n_reads);
     if (ext_scores) res->d_scores.view(ext_scores, n_pairs); else CU(res->d_scores.alloc(n_pairs, st));
-    if (ext_totals) res->d_totals.view(ext_totals, (size_t)n_refs); else CU(res->d_totals.alloc((size_t)n_refs, st));
-    CU(res->d_best.alloc((size_t)n_reads * 4, st));
+    if (ext_totals) res->d_totals.view(ext_totals, (size_t)o_refs); else CU(res->d_totals.alloc((size_t)o_refs, st));
+    CU(res->d_best.alloc((size_t)o_reads * 4, st));
     CU(cudaMemsetAsync(res->d_scores.p, 0, std::max<size_t>(n_pairs, 1) * 4, st));
     res->top_k = top_k; res->min_score = min_score;
-    if (top_k > 0) CU(res->d_hits.alloc((size_t)n_reads * top_k * 4, st));
+    if (top_k > 0) CU(res->d_hits.alloc((size_t)o_reads * top_k * 4, st));
 
     const auto t_wall0 = std::chrono::steady_clock::now();
     ctx->ev_used = 0;                                    // the timer's spans reuse the context's events
@@ -105,7 +112,9 @@ int AlignCall::run(int32_t *ext_scores, int32_t *ext_totals)
     return finish_stats(t_wall0);
 }
 
-// reads by rows-per-lane class of the short path, longest first inside a class after run_class; the rest take the wide path
+// reads by rows-per-lane class of the short path, longest first inside a class after run_class; the rest take the wide path.
+// Both strands: read q and its reverse complement n + q go in next to each other.  They have the same length, so the
+// stable length sort keeps them next to each other, and every class holds whole (q, n + q) read pairs.
 void AlignCall::classify_reads(std::vector<std::vector<int32_t>> &classes, std::vector<int32_t> &wide) const
 {
     // s16x2 short-read kernels: gap < 0 (padding stays below the maximum), small scores, 2-bit alphabet;
@@ -115,7 +124,8 @@ void AlignCall::classify_reads(std::vector<std::vector<int32_t>> &classes, std::
     // reads of 257 .. 511 rows: the LONG classes (K = 40 .. 64) exist for the biased fill and the tile kernels only;
     // other score sets send such reads through the wide path
     const bool long_kernels_ok = tile_trace_ok(match, mismatch, gap);
-    for (int64_t q = 0; q < rd->n_reads; ++q) {
+    for (int64_t x = 0; x < rd->n_reads; ++x) {
+        const int64_t q = both ? (x >> 1) + (x & 1) * o_reads : x;
         const int m = rd->len[(size_t)q];
         if (m == 0) continue;                                  // score 0, no cells
         const int64_t smax = (int64_t)std::max({match, mismatch, 0}) * std::min<int64_t>(m, rs->max_len);   // a positive mismatch scores too
@@ -194,8 +204,13 @@ int AlignCall::fill_batch(int K, const std::vector<int32_t> &reads, int64_t rp0,
             }
         }
     ++n_batches;
+    // both strands in hits mode: the selection's slots, the forward read of each read pair, follow the read pairs
+    const bool fwd_slots = both && top_k > 0 && !(flags & SWB_F_SCORES_ONLY);
+    if (fwd_slots)
+        for (int r = 0; r < n_rp; ++r) b.h_rp.push_back(b.h_rp[(size_t)r * 2]);
     CU(ctx->rp.reserve(b.h_rp.size(), st));
     CU(cudaMemcpyAsync(ctx->rp.p, b.h_rp.data(), b.h_rp.size() * 4, cudaMemcpyHostToDevice, st));
+    if (fwd_slots) b.h_rp.resize((size_t)n_rp * 2);
     const size_t ck_words = (size_t)n_rp * rs->blocks_per_rp * record_words(K) * GL;
     const size_t tmx_words = (size_t)n_rp * rs->blocks_per_rp * GL;
     CU(ctx->ck.reserve(ck_words, st));
@@ -297,7 +312,12 @@ int AlignCall::locate_cells(int K, const Batch &b, size_t sel_words, uint32_t &n
         if (sel_words) {
             CU(timer.begin(STAT_SELECT_MS));
             CU(cudaMemsetAsync(ctx->hit_sel.p, 0, sel_words * 4, st));
-            CU(select_hits(P.rp_reads, (int64_t)b.n_rp * 2, 1, nullptr, ctx->hit_sel.p, rs->n_refs, 1));
+            // both strands: one slot per read pair over the 2R oriented references; oriented o = 2r + s marks bit
+            // (2 * rp + s) * R + r, the emit's bit of pair (r, strand s of read pair rp)
+            if (both)
+                CU(select_hits(P.rp_reads + (size_t)b.n_rp * 2, b.n_rp, 1, nullptr, ctx->hit_sel.p, 2 * rs->n_refs, rs->n_refs, true));
+            else
+                CU(select_hits(P.rp_reads, (int64_t)b.n_rp * 2, 1, nullptr, ctx->hit_sel.p, rs->n_refs, 1));
             CU(timer.end());
             launches += 2;
         }
@@ -319,27 +339,31 @@ int AlignCall::locate_cells(int K, const Batch &b, size_t sel_words, uint32_t &n
 }
 
 // hits mode: top k + best pair of the reads `slots` (score rows exact by now) -> `bits` / `hits` (swb_hits.cu)
+// over the oriented view: slots are oriented reads, the references oriented references
 cudaError_t AlignCall::select_hits(const int32_t *slots, int64_t n_slots, int with_best, int4 *hits, uint32_t *bits, int64_t bit_slot,
-                                   int64_t bit_ref)
+                                   int64_t bit_ref, bool oriented_bits)
 {
-    const size_t te = select_hits_tmp_elems(rs->n_refs, n_slots, top_k);
+    const size_t te = select_hits_tmp_elems(o_refs, n_slots, top_k);
     cudaError_t e = ctx->hit_tmp.reserve(te, st);
-    if (e == cudaSuccess) e = launch_select_hits(res->d_scores.p, rs->n_refs, rd->n_reads, slots, n_slots, top_k, min_score, with_best,
-                                                 hits, bits, bit_slot, bit_ref, ctx->hit_tmp.p, te, st);
+    if (e == cudaSuccess) e = launch_select_hits(res->d_scores.p, o_refs, o_reads, slots, n_slots, top_k, min_score, with_best,
+                                                 hits, bits, bit_slot, bit_ref, oriented_bits, ctx->hit_tmp.p, te, st);
     return e;
 }
 
 // the reads of the int32 wide path; hits mode: exact scores of every wide pair first, then the whole wide path over each
-// read's top k + best pair
+// read's top k + best pair.  Both strands: `wide` holds (q, n + q) next to each other (classify_reads); the selection
+// runs once per read q over the oriented references, and each strand takes the references of its own orientation.
 int AlignCall::run_wide_reads(const std::vector<int32_t> &wide)
 {
     if (top_k <= 0 || (flags & SWB_F_SCORES_ONLY)) return run_wide_path(wide, (flags & SWB_F_SCORES_ONLY) != 0);
     int rc = run_wide_path(wide, true);
     if (rc) return rc;
-    const int64_t nw = (int64_t)wide.size();
+    std::vector<int32_t> slots;
+    for (size_t x = 0; x < wide.size(); x += both ? 2 : 1) slots.push_back(wide[x]);
+    const int64_t nw = (int64_t)slots.size();
     DevBuf<int32_t> d_wr;
     CU(d_wr.alloc((size_t)nw, st));
-    CU(cudaMemcpyAsync(d_wr.p, wide.data(), (size_t)nw * 4, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_wr.p, slots.data(), (size_t)nw * 4, cudaMemcpyHostToDevice, st));
     CU(timer.begin(STAT_SELECT_MS));
     int4 *d_sel = reinterpret_cast<int4 *>(res->d_hits.p);              // scratch here: the final selection rewrites it
     CU(select_hits(d_wr.p, nw, 1, d_sel, nullptr, 0, 0));
@@ -348,11 +372,16 @@ int AlignCall::run_wide_reads(const std::vector<int32_t> &wide)
     std::vector<int4> h_sel((size_t)nw * top_k);
     CU(cudaMemcpyAsync(h_sel.data(), d_sel, h_sel.size() * sizeof(int4), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    std::vector<std::vector<int32_t>> refs_of((size_t)nw);
-    for (int64_t x = 0; x < nw; ++x) {
-        for (int h = 0; h < top_k; ++h)
-            if (h_sel[(size_t)(x * top_k + h)].y >= 0) refs_of[(size_t)x].push_back(h_sel[(size_t)(x * top_k + h)].y);
-        std::sort(refs_of[(size_t)x].begin(), refs_of[(size_t)x].end());
+    std::vector<std::vector<int32_t>> refs_of(wide.size());
+    for (size_t x = 0; x < wide.size(); ++x) {
+        const size_t sx = both ? x / 2 : x;
+        for (int h = 0; h < top_k; ++h) {
+            const int32_t o = h_sel[sx * top_k + h].y;
+            if (o < 0) continue;
+            if (!both) refs_of[x].push_back(o);
+            else if ((o & 1) == (int32_t)(x & 1)) refs_of[x].push_back(o >> 1);
+        }
+        std::sort(refs_of[x].begin(), refs_of[x].end());
     }
     return run_wide_path(wide, false, &refs_of);
 }
@@ -366,7 +395,7 @@ int AlignCall::select_final_hits(DevBuf<uint32_t> &keep)
         CU(cudaMemsetAsync(keep.p, 0, ((n_pairs + 31) / 32) * 4, st));
     }
     CU(timer.begin(STAT_SELECT_MS));
-    CU(select_hits(nullptr, rd->n_reads, 0, reinterpret_cast<int4 *>(res->d_hits.p), keep.p, 1, rd->n_reads));
+    CU(select_hits(nullptr, o_reads, 0, reinterpret_cast<int4 *>(res->d_hits.p), keep.p, 1, o_reads));
     CU(timer.end());
     launches += 2;
     return SWB_OK;
@@ -377,8 +406,8 @@ int AlignCall::assemble(const DevBuf<uint32_t> &keep)
 {
     const int64_t n_refs = rs->n_refs, n_reads = rd->n_reads;
     const size_t n_pairs = (size_t)(n_refs * n_reads);
-    CU(launch_ref_totals(res->d_scores.p, n_refs, n_reads, res->d_totals.p, st));
-    CU(launch_best_hits(res->d_scores.p, n_refs, n_reads, res->d_best.p, ctx->sm_count, st));
+    CU(launch_ref_totals(res->d_scores.p, o_refs, o_reads, res->d_totals.p, st));
+    CU(launch_best_hits(res->d_scores.p, o_refs, o_reads, res->d_best.p, ctx->sm_count, st));
     launches += 3;
     if (flags & SWB_F_SCORES_ONLY) {
         CU(cudaStreamSynchronize(st));
@@ -436,10 +465,10 @@ int AlignCall::assemble(const DevBuf<uint32_t> &keep)
     res->total_words = total_words;
     CU(res->f_ops.alloc((size_t)total_words, st));
     CU(assemble_gather_ops(d_desc.p, (int)descs.size(), NK, d_order.p, res->f_ops_off.p, res->f_ops.p, st));
-    CU(assemble_offsets(d_pair_sorted.p, NK, (int64_t)n_pairs, res->f_cell_off.p, res->d_best.p, n_reads, res->f_cells.p, st));
+    CU(assemble_offsets(d_pair_sorted.p, NK, (int64_t)n_pairs, res->f_cell_off.p, res->d_best.p, o_reads, res->f_cells.p, st));
     launches += 8;
     if (keep.p) {
-        CU(assemble_hit_cells(d_desc.p, (int)descs.size(), d_pair_sorted.p, d_order.p, N, (int64_t)n_pairs, n_reads, res->f_cell_off.p,
+        CU(assemble_hit_cells(d_desc.p, (int)descs.size(), d_pair_sorted.p, d_order.p, N, (int64_t)n_pairs, o_reads, res->f_cell_off.p,
                               res->f_cells.p, res->d_best.p, res->d_hits.p, top_k, st));
         launches += 2;
     }
@@ -457,11 +486,13 @@ int AlignCall::finish_stats(std::chrono::steady_clock::time_point t_wall0)
 }
 
 // the checks of an align call on a reference set handle, before it takes the context
-static int check_call(const swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch, int32_t gap)
+static int check_call(const swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch, int32_t gap,
+                      uint32_t flags)
 {
     if (rd->rs != rs) return fail(SWB_E_INVALID, "swb_align: reads were encoded against a different reference set");
     if (rs->ctx != ctx || rd->ctx != ctx) return fail(SWB_E_INVALID, "swb_align: handles belong to another context");
-    if (rs->n_refs * rd->n_reads >= ((int64_t)1 << 33)) return fail(SWB_E_UNSUPPORTED, "swb_align: more than 2^33 pairs per call");
+    const int64_t strands = (flags & SWB_F_BOTH_STRANDS) ? 2 : 1;
+    if (strands * rs->n_refs * rd->n_reads >= ((int64_t)1 << 33)) return fail(SWB_E_UNSUPPORTED, "swb_align: more than 2^33 pairs per call");
     int32_t max_m = 0;
     for (int32_t m : rd->len) max_m = std::max(max_m, m);
     // Java int arithmetic wraps; this engine refuses inputs whose scores could leave int32 instead
@@ -480,6 +511,8 @@ static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, i
     CU(cudaSetDevice(ctx->device));
     ResultPtr res = new_result(ctx, rs, rd, flags);
     AlignCall call{ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, res.get(), ctx->stream, {ctx, ctx->stream}};
+    call.both = (flags & SWB_F_BOTH_STRANDS) != 0;
+    call.o_refs = res->n_refs; call.o_reads = res->n_reads;
     int rc = call.run(ext_scores, ext_totals);
     if (rc) return rc;
     swb_result *r = res.release();
@@ -627,8 +660,15 @@ static int align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *r
     if (!ctx || !rs || !rd || !out) return fail(SWB_E_INVALID, "swb_align: null argument");
     *out = nullptr;
     if (rs->parent) return fail(SWB_E_INVALID, "swb_align: a part of a reference set is not a handle");
-    int rc = check_call(ctx, rs, rd, match, mismatch, gap);
+    int rc = check_call(ctx, rs, rd, match, mismatch, gap, flags);
     if (rc) return rc;
+    // both strands: the 2n internal reads [reads; rc(reads)] of this call, on the set as one (whole, when it has parts)
+    if (flags & SWB_F_BOTH_STRANDS) {
+        std::unique_ptr<swb_reads> rd2;
+        if ((rc = both_strands_reads(ctx, rs, rd, rd2))) return rc;
+        return align_leaf(ctx, rs->parts.empty() ? rs : rs->whole, rd2.get(), match, mismatch, gap, flags, top_k, min_score, nullptr,
+                          nullptr, out);
+    }
     if (rs->parts.empty()) return align_leaf(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, nullptr, nullptr, out);
     // hits mode also runs on the set as one: its cell arrays are small (nothing to overlap), and the selection is then
     // over all references at once, so no part keeps cells of a pair that a later part displaces from the top k

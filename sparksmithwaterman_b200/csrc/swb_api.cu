@@ -504,6 +504,17 @@ int swb_result_materialize(const swb_result *r, int64_t cell, const char *ref, i
     std::vector<uint8_t> ops((size_t)len + 1);
     int rc = swb_result_ops(r, cell, ops.data(), len);
     if (rc) return rc;
+    // both strands: a cell of an odd oriented reference is a cell of the read's reverse complement (case kept)
+    std::string rc_read;
+    if ((r->flags & SWB_F_BOTH_STRANDS) && r->cell_off) {
+        const int64_t n_pairs = r->n_refs * r->n_reads;
+        const int64_t p = (int64_t)(std::upper_bound(r->cell_off, r->cell_off + n_pairs + 1, cell) - r->cell_off) - 1;
+        if ((p / r->n_reads) & 1) {
+            rc_read.resize((size_t)std::max<int64_t>(read_len, 0));
+            for (int64_t k = 0; k < read_len; ++k) rc_read[(size_t)k] = complement_keep_case(read[read_len - 1 - k]);
+            read = rc_read.data();
+        }
+    }
     // walk the columns backwards from the end cell (SmithWaterman.java:380-409), fill forwards
     int64_t i = r->cells[2 * (size_t)cell], j = r->cells[2 * (size_t)cell + 1];
     if (i > read_len || j > ref_len) return fail(SWB_E_RANGE, "swb_result_materialize: sequences shorter than the cell");

@@ -68,7 +68,9 @@ __global__ void __launch_bounds__(128) hits_partial_kernel(const int32_t *__rest
 
 // warp per slot: merge the slot's partial lists.  Entry h is TAKEN if it exists and (score >= min_score, or h = 0 and
 // with_best: the read's best pair).  Taken entries go to hits[slot * k + h] = (score, ref, 0, 0), the others are
-// padding (0, -1, 0, 0); a taken entry also sets bit slot * bit_slot + ref * bit_ref of `bits`.
+// padding (0, -1, 0, 0); a taken entry also sets bit slot * bit_slot + ref * bit_ref of `bits`.  Oriented (both strands,
+// the refs are oriented o = 2r + s): bit slot * bit_slot + s * bit_ref + r, the bit of strand s's half of the read pair.
+template <bool Oriented>
 __global__ void __launch_bounds__(128) hits_merge_kernel(const uint64_t *part, int n_chunks, int k, const int32_t *slots,
                                                          int64_t slot0, int64_t n_slots, int32_t min_score, int with_best,
                                                          int4 *hits, uint32_t *bits, int64_t bit_slot, int64_t bit_ref)
@@ -92,7 +94,7 @@ __global__ void __launch_bounds__(128) hits_merge_kernel(const uint64_t *part, i
     const bool take = mine != 0 && (score >= min_score || (lane == 0 && with_best));
     if (hits) hits[slot * k + lane] = take ? make_int4(score, ref, 0, 0) : make_int4(0, -1, 0, 0);
     if (bits && take) {
-        const int64_t bit = slot * bit_slot + (int64_t)ref * bit_ref;
+        const int64_t bit = Oriented ? slot * bit_slot + (int64_t)(ref & 1) * bit_ref + (ref >> 1) : slot * bit_slot + (int64_t)ref * bit_ref;
         atomicOr(bits + (bit >> 5), 1u << (bit & 31));
     }
 }
@@ -114,7 +116,7 @@ size_t select_hits_tmp_elems(int64_t n_refs, int64_t n_slots, int k)
 
 cudaError_t launch_select_hits(const int32_t *scores, int64_t n_refs, int64_t n_reads, const int32_t *slots, int64_t n_slots,
                                int k, int32_t min_score, int with_best, int4 *hits, uint32_t *bits, int64_t bit_slot,
-                               int64_t bit_ref, uint64_t *tmp, size_t tmp_elems, cudaStream_t st)
+                               int64_t bit_ref, bool oriented_bits, uint64_t *tmp, size_t tmp_elems, cudaStream_t st)
 {
     if (n_slots <= 0) return cudaSuccess;
     const int64_t chunk = chunk_refs_of(n_refs);
@@ -126,8 +128,11 @@ cudaError_t launch_select_hits(const int32_t *scores, int64_t n_refs, int64_t n_
         const int64_t warps1 = ns * n_chunks;
         hits_partial_kernel<<<(unsigned)((warps1 * 32 + threads - 1) / threads), threads, 0, st>>>(scores, n_refs, n_reads, slots, s0, ns,
                                                                                                  chunk, n_chunks, k, tmp);
-        hits_merge_kernel<<<(unsigned)((ns * 32 + threads - 1) / threads), threads, 0, st>>>(tmp, n_chunks, k, slots, s0, ns, min_score,
-                                                                                           with_best, hits, bits, bit_slot, bit_ref);
+        const unsigned blocks2 = (unsigned)((ns * 32 + threads - 1) / threads);
+        if (oriented_bits)
+            hits_merge_kernel<true><<<blocks2, threads, 0, st>>>(tmp, n_chunks, k, slots, s0, ns, min_score, with_best, hits, bits, bit_slot, bit_ref);
+        else
+            hits_merge_kernel<false><<<blocks2, threads, 0, st>>>(tmp, n_chunks, k, slots, s0, ns, min_score, with_best, hits, bits, bit_slot, bit_ref);
         const cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return e;
     }

@@ -342,8 +342,18 @@ struct PhaseTimer {
     }
 };
 
+// both-strands mode (swb_strands.cu): the IUPAC DNA complement of a byte keeping case (a -> t; a byte outside the
+// table stays itself), the complement codes of a set's alphabet, and the 2n internal reads [reads; rc(reads)] of a call
+char complement_keep_case(char c);
+int strand_complement_codes(const swb_refset *rs, uint8_t comp_code[256]);
+int both_strands_reads(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, std::unique_ptr<swb_reads> &out);
+
 // One align call over one packed set (a whole set, or one part of a large one), step by step (swb_align.cu; the wide
 // path in swb_wide_host.cu).  top_k > 0: hits mode (swb_align_hits).
+// Two views of the pairs: the fill, locate, traceback and assembly sort run over (rs->n_refs, rd->n_reads); the
+// totals, best hits and selections over the result's oriented (o_refs, o_reads).  They are the same unless `both`
+// (SWB_F_BOTH_STRANDS): rd then holds the 2n internal reads [reads; rc(reads)], and pair r * 2n + s * n + q of the
+// internal view is pair (2r + s) * n + q of the oriented one -- the same index.
 struct AlignCall {
     swb_ctx *ctx;
     const swb_refset *rs;
@@ -356,6 +366,8 @@ struct AlignCall {
     PhaseTimer timer;
     int launches = 1, n_batches = 0;
     double ck_bytes = 0;
+    bool both = false;
+    int64_t o_refs = 0, o_reads = 0;
 
     struct Batch;
     int run(int32_t *ext_scores, int32_t *ext_totals);
@@ -366,7 +378,7 @@ struct AlignCall {
     int trace_batch(int K, Batch &b);
     int locate_cells(int K, const Batch &b, size_t sel_words, uint32_t &n_cells);
     cudaError_t select_hits(const int32_t *slots, int64_t n_slots, int with_best, int4 *hits, uint32_t *bits, int64_t bit_slot,
-                            int64_t bit_ref);
+                            int64_t bit_ref, bool oriented_bits = false);
     int run_wide_reads(const std::vector<int32_t> &wide);
     // refs_of (nullable): refs_of[k] = the references (ascending) read reads[k] is aligned against; nullptr = all of them
     int run_wide_path(const std::vector<int32_t> &reads, bool scores_only, const std::vector<std::vector<int32_t>> *refs_of = nullptr);

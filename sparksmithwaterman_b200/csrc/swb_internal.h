@@ -201,7 +201,7 @@ cudaError_t assemble_hit_cells(const BatchDesc *batches, int nb, const uint64_t 
 size_t      select_hits_tmp_elems(int64_t n_refs, int64_t n_slots, int k);
 cudaError_t launch_select_hits(const int32_t *scores, int64_t n_refs, int64_t n_reads, const int32_t *slots, int64_t n_slots,
                                int k, int32_t min_score, int with_best, int4 *hits, uint32_t *bits, int64_t bit_slot,
-                               int64_t bit_ref, uint64_t *tmp, size_t tmp_elems, cudaStream_t st);
+                               int64_t bit_ref, bool oriented_bits, uint64_t *tmp, size_t tmp_elems, cudaStream_t st);
 
 cudaError_t launch_wide_pad_reads(const uint8_t *codes, const int64_t *read_off, const int32_t *reads, int n_reads,
                                   const int64_t *rpad_off, const int64_t *rpad_len, uint8_t *rpad, int64_t max_len,

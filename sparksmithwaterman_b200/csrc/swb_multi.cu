@@ -141,19 +141,20 @@ struct GatherBufs {
     DevBuf<int32_t> hsend, hgathered, hmerged;   // hits mode: [n_reads][k][4] per shard
     DevBuf<int64_t> ids;
     int64_t n_ids = 0;
-    void release() { send.release(); gathered.release(); merged.release(); hsend.release(); hgathered.release(); hmerged.release(); ids.release(); }
+    DevBuf<int64_t> oids;                        // both strands: oriented local 2r + s -> oriented global 2 * ids[r] + s
+    void release() { send.release(); gathered.release(); merged.release(); hsend.release(); hgathered.release(); hmerged.release(); ids.release(); oids.release(); }
 };
 
 // localize -> allgather -> merge on `st` of the current device.  `grouped`: the caller brackets several devices'
 // collectives with ncclGroupStart / ncclGroupEnd (single-process form) and launches the merge afterwards.
-cudaError_t enqueue_localize(GatherBufs &g, const int32_t *d_best, int64_t n_reads, int world, cudaStream_t st)
+cudaError_t enqueue_localize(GatherBufs &g, const int64_t *ids, int64_t n_ids, const int32_t *d_best, int64_t n_reads, int world, cudaStream_t st)
 {
     cudaError_t e = g.send.reserve((size_t)n_reads * 4, st);
     if (e == cudaSuccess) e = g.gathered.reserve((size_t)n_reads * 4 * world, st);
     if (e == cudaSuccess) e = g.merged.reserve((size_t)n_reads * 4, st);
     if (e != cudaSuccess || n_reads == 0) return e;
     const int threads = 256;
-    best_to_global_kernel<<<(unsigned)((n_reads + threads - 1) / threads), threads, 0, st>>>(d_best, g.ids.p, g.n_ids, n_reads, g.send.p);
+    best_to_global_kernel<<<(unsigned)((n_reads + threads - 1) / threads), threads, 0, st>>>(d_best, ids, n_ids, n_reads, g.send.p);
     return cudaGetLastError();
 }
 cudaError_t enqueue_merge(GatherBufs &g, int64_t n_reads, int world, cudaStream_t st)
@@ -165,7 +166,8 @@ cudaError_t enqueue_merge(GatherBufs &g, int64_t n_reads, int world, cudaStream_
 }
 
 // the same two steps for the hit lists of a hits-mode result
-cudaError_t enqueue_localize_hits(GatherBufs &g, const int32_t *d_hits, int64_t n_reads, int k, int world, cudaStream_t st)
+cudaError_t enqueue_localize_hits(GatherBufs &g, const int64_t *ids, int64_t n_ids, const int32_t *d_hits, int64_t n_reads, int k, int world,
+                                  cudaStream_t st)
 {
     const size_t n = (size_t)n_reads * k;
     cudaError_t e = g.hsend.reserve(n * 4, st);
@@ -173,7 +175,7 @@ cudaError_t enqueue_localize_hits(GatherBufs &g, const int32_t *d_hits, int64_t 
     if (e == cudaSuccess) e = g.hmerged.reserve(n * 4, st);
     if (e != cudaSuccess || n == 0) return e;
     const int threads = 256;
-    hits_to_global_kernel<<<(unsigned)((n + threads - 1) / threads), threads, 0, st>>>(d_hits, g.ids.p, g.n_ids, (int64_t)n, g.hsend.p);
+    hits_to_global_kernel<<<(unsigned)((n + threads - 1) / threads), threads, 0, st>>>(d_hits, ids, n_ids, (int64_t)n, g.hsend.p);
     return cudaGetLastError();
 }
 cudaError_t enqueue_merge_hits(GatherBufs &g, int64_t n_reads, int k, int world, cudaStream_t st)
@@ -276,7 +278,7 @@ int swb_comm_allgather_best(swb_comm *c, const swb_result *res, const int64_t *g
     CU(c->g.ids.reserve((size_t)std::max<int64_t>(n_local_refs, 1), st));
     c->g.n_ids = n_local_refs;
     if (n_local_refs) CU(cudaMemcpyAsync(c->g.ids.p, global_ids, (size_t)n_local_refs * 8, cudaMemcpyHostToDevice, st));
-    CU(enqueue_localize(c->g, res->d_best.p, n_reads, c->world, st));
+    CU(enqueue_localize(c->g, c->g.ids.p, c->g.n_ids, res->d_best.p, n_reads, c->world, st));
     if (c->world > 1) {
         if (n_reads) NC(nccl_api()->AllGather(c->g.send.p, c->g.gathered.p, (size_t)n_reads * 4, ncclInt32, c->comm, st));
     } else if (n_reads) {
@@ -307,7 +309,7 @@ int swb_comm_allgather_hits(swb_comm *c, const swb_result *res, const int64_t *g
     CU(c->g.ids.reserve((size_t)std::max<int64_t>(n_local_refs, 1), st));
     c->g.n_ids = n_local_refs;
     if (n_local_refs) CU(cudaMemcpyAsync(c->g.ids.p, global_ids, (size_t)n_local_refs * 8, cudaMemcpyHostToDevice, st));
-    CU(enqueue_localize_hits(c->g, res->d_hits.p, n_reads, k, c->world, st));
+    CU(enqueue_localize_hits(c->g, c->g.ids.p, c->g.n_ids, res->d_hits.p, n_reads, k, c->world, st));
     if (c->world > 1) {
         if (n) NC(nccl_api()->AllGather(c->g.hsend.p, c->g.hgathered.p, n * 4, ncclInt32, c->comm, st));
     } else if (n) {
@@ -424,6 +426,10 @@ int swb_multi_refset_load(swb_multi *m, int64_t n_refs, const char *bytes, const
                 cudaError_t e = cudaSetDevice(c->device);
                 if (e == cudaSuccess) e = g.ids.reserve(std::max<size_t>(v.size(), 1), c->stream);
                 if (e == cudaSuccess && !v.empty()) e = cudaMemcpyAsync(g.ids.p, v.data(), v.size() * 8, cudaMemcpyHostToDevice, c->stream);
+                std::vector<int64_t> ov(2 * v.size());
+                for (size_t k = 0; k < ov.size(); ++k) ov[k] = 2 * v[k / 2] + (int64_t)(k & 1);
+                if (e == cudaSuccess) e = g.oids.reserve(std::max<size_t>(ov.size(), 1), c->stream);
+                if (e == cudaSuccess && !ov.empty()) e = cudaMemcpyAsync(g.oids.p, ov.data(), ov.size() * 8, cudaMemcpyHostToDevice, c->stream);
                 if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
                 g.n_ids = (int64_t)v.size();
                 if (e != cudaSuccess) rc = cuda_fail(e, "swb_multi_refset_load: id table");
@@ -491,14 +497,20 @@ static int multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, co
     for (int d = 0; d < n; ++d)
         if (rcs[(size_t)d]) { const int rc = rcs[(size_t)d]; const std::string e = errs[(size_t)d]; drop(); return fail(rc, "shard " + std::to_string(d) + ": " + e); }
 
-    // phase 2: best hits -> global ids -> one all-gather over NVLink -> merge, on every device's engine stream
+    // phase 2: best hits -> global ids -> one all-gather over NVLink -> merge, on every device's engine stream.  Both
+    // strands: the shards' records hold oriented local ids 2r + s, localized to oriented global ids 2 * gid + s, so the
+    // merge's order is the single-context order over the oriented references
     const auto t1 = std::chrono::steady_clock::now();
+    const bool both = (flags & SWB_F_BOTH_STRANDS) != 0;
     for (int d = 0; d < n; ++d) {
         swb_ctx *c = m->ctx[(size_t)d];
+        GatherBufs &g = m->g[(size_t)d];
+        const int64_t *ids = both ? g.oids.p : g.ids.p;
+        const int64_t n_ids = both ? 2 * g.n_ids : g.n_ids;
         cudaError_t e = cudaSetDevice(c->device);
-        if (e == cudaSuccess) e = enqueue_localize(m->g[(size_t)d], res->shard[(size_t)d]->d_best.p, n_reads, n, c->stream);
+        if (e == cudaSuccess) e = enqueue_localize(g, ids, n_ids, res->shard[(size_t)d]->d_best.p, n_reads, n, c->stream);
         if (e == cudaSuccess && top_k > 0)
-            e = enqueue_localize_hits(m->g[(size_t)d], res->shard[(size_t)d]->d_hits.p, n_reads, top_k, n, c->stream);
+            e = enqueue_localize_hits(g, ids, n_ids, res->shard[(size_t)d]->d_hits.p, n_reads, top_k, n, c->stream);
         if (e != cudaSuccess) { drop(); return cuda_fail(e, "swb_multi_align: best hits -> global ids"); }
     }
     if (n > 1 && n_reads > 0) {

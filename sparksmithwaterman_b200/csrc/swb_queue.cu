@@ -172,6 +172,7 @@ int swb_align_pair(swb_ctx *ctx, const char *ref, int64_t ref_len, const char *r
     if (!ctx) return fail(SWB_E_INVALID, "swb_align_pair: ctx is null");
     if (ref_len < 0 || read_len < 0 || (ref_len > 0 && !ref) || (read_len > 0 && !read))
         return fail(SWB_E_INVALID, "swb_align_pair: bad sequence argument");
+    if (flags & SWB_F_BOTH_STRANDS) return fail(SWB_E_INVALID, "swb_align_pair: SWB_F_BOTH_STRANDS is not accepted here");
     PairReq rq;
     rq.ref = ref; rq.ref_len = ref_len; rq.read = read; rq.read_len = read_len;
     rq.match = match; rq.mismatch = mismatch; rq.gap = gap; rq.flags = flags & ~SWB_F_NO_FETCH;

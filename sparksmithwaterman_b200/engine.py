@@ -8,7 +8,7 @@ from typing import List, Sequence, Tuple
 import numpy as np
 
 from . import _ffi
-from ._ffi import SWB_F_NO_FETCH, SWB_F_SCORES_ONLY, SWB_F_TIE_GT, check
+from ._ffi import SWB_F_BOTH_STRANDS, SWB_F_NO_FETCH, SWB_F_SCORES_ONLY, SWB_F_TIE_GT, check
 
 DEFAULT_SCORES = (5, -3, -4)          # Distribution.java:36 of the reference: match, mismatch, gap
 
@@ -27,6 +27,22 @@ def concat(seqs: Sequence) -> Tuple[bytes, np.ndarray, List[bytes]]:
 
 def _i64p(a: np.ndarray):
     return a.ctypes.data_as(C.POINTER(C.c_int64))
+
+
+# IUPAC DNA complement (the library's table for SWB_F_BOTH_STRANDS): an involution that keeps case; S, W and N map to
+# themselves, and any other byte stays itself
+_COMP_FROM, _COMP_TO = b"ACGTRYKMBVDHSWN", b"TGCAYRMKVBHDSWN"
+COMPLEMENT = bytes.maketrans(_COMP_FROM + _COMP_FROM.lower(), _COMP_TO + _COMP_TO.lower())
+
+
+def reverse_complement(seq) -> bytes:
+    """The reverse complement of a read, as a both-strands call aligns it (o = 2r + 1), case kept."""
+    return _b(seq).translate(COMPLEMENT)[::-1]
+
+
+def _flags(scores_only: bool, fetch: bool, tie_gt: bool, both_strands: bool) -> int:
+    return ((SWB_F_SCORES_ONLY if scores_only else 0) | (0 if fetch else SWB_F_NO_FETCH) | (SWB_F_TIE_GT if tie_gt else 0)
+            | (SWB_F_BOTH_STRANDS if both_strands else 0))
 
 
 class Engine:
@@ -114,15 +130,18 @@ class RefSet:
         return Reads(self, reads)
 
     def align(self, reads, scores=DEFAULT_SCORES, scores_only: bool = False, fetch: bool = True,
-              tie_gt: bool = False, *, top_k: int | None = None, min_score: int = 1) -> "AlignResult":
+              tie_gt: bool = False, *, top_k: int | None = None, min_score: int = 1,
+              both_strands: bool = False) -> "AlignResult":
         """Host-buffer path (swb_align): H2D of the reads, compute, D2H of the results.
         tie_gt: DistributedSW's strict-'>' tie rule in the traceback (SWB_F_TIE_GT).
         top_k: hits mode (swb_align_hits) -- every pair is scored, but only each read's top_k best pairs with
-        score >= min_score are traced (AlignResult.hits / read_hits)."""
+        score >= min_score are traced (AlignResult.hits / read_hits).
+        both_strands: every read and its reverse complement (SWB_F_BOTH_STRANDS); the result has 2 * n_refs oriented
+        references, o = 2r (read as given) and o = 2r + 1 (reverse complement) -- AlignResult.oriented."""
         if isinstance(reads, Reads):
-            return reads.align(scores, scores_only, fetch, tie_gt, top_k=top_k, min_score=min_score)
+            return reads.align(scores, scores_only, fetch, tie_gt, top_k=top_k, min_score=min_score, both_strands=both_strands)
         data, off, bs = concat(reads)
-        flags = (SWB_F_SCORES_ONLY if scores_only else 0) | (0 if fetch else SWB_F_NO_FETCH) | (SWB_F_TIE_GT if tie_gt else 0)
+        flags = _flags(scores_only, fetch, tie_gt, both_strands)
         h = C.c_void_p()
         if top_k is None:
             check(self.eng.lib.swb_align(self.eng.h, self.h, len(bs), data, _i64p(off),
@@ -130,7 +149,7 @@ class RefSet:
         else:
             check(self.eng.lib.swb_align_hits(self.eng.h, self.h, len(bs), data, _i64p(off),
                                               scores[0], scores[1], scores[2], flags, top_k, min_score, C.byref(h)))
-        return AlignResult(self, bs, h, scores_only)
+        return AlignResult(self, bs, h, scores_only, both_strands=both_strands)
 
 
 class Reads:
@@ -157,8 +176,9 @@ class Reads:
             pass
 
     def align(self, scores=DEFAULT_SCORES, scores_only: bool = False, fetch: bool = True,
-              tie_gt: bool = False, *, top_k: int | None = None, min_score: int = 1) -> "AlignResult":
-        flags = (SWB_F_SCORES_ONLY if scores_only else 0) | (0 if fetch else SWB_F_NO_FETCH) | (SWB_F_TIE_GT if tie_gt else 0)
+              tie_gt: bool = False, *, top_k: int | None = None, min_score: int = 1,
+              both_strands: bool = False) -> "AlignResult":
+        flags = _flags(scores_only, fetch, tie_gt, both_strands)
         h = C.c_void_p()
         lib = self.rs.eng.lib
         if top_k is None:
@@ -166,7 +186,7 @@ class Reads:
         else:
             check(lib.swb_align_resident_hits(self.rs.eng.h, self.rs.h, self.h, scores[0], scores[1], scores[2], flags,
                                               top_k, min_score, C.byref(h)))
-        return AlignResult(self.rs, self.seqs, h, scores_only)
+        return AlignResult(self.rs, self.seqs, h, scores_only, both_strands=both_strands)
 
 
 STAT_NAMES = ("h2d_ms", "fill_ms", "locate_ms", "trace_ms", "d2h_ms", "device_ms", "cells", "pairs",
@@ -174,8 +194,9 @@ STAT_NAMES = ("h2d_ms", "fill_ms", "locate_ms", "trace_ms", "d2h_ms", "device_ms
 
 
 class AlignResult:
-    def __init__(self, rs: RefSet, reads: List[bytes], h, scores_only: bool, owned: bool = True):
+    def __init__(self, rs: RefSet, reads: List[bytes], h, scores_only: bool, owned: bool = True, both_strands: bool = False):
         self.rs, self.reads, self.h, self.scores_only = rs, reads, h, scores_only
+        self.both_strands = both_strands        # n_refs counts oriented references o = 2r + strand
         self._owned = owned                     # False: a shard of a MultiResult, freed with it
         self.lib = rs.eng.lib
         self.n_refs = int(self.lib.swb_result_n_refs(h))
@@ -233,14 +254,23 @@ class AlignResult:
         return self._arr(p, self.n_reads * k.value * 4, np.int32).reshape(self.n_reads, k.value, 4)
 
     def read_hits(self, read: int):
-        """Hits mode: [(ref, score, cells, sites)] of read `read`'s hits in hit order; cells / sites as pair()."""
+        """Hits mode: [(ref, score, cells, sites)] of read `read`'s hits in hit order; cells / sites as pair().
+        A both-strands result gives [(ref, strand, score, cells, sites)], ref the reference's own index."""
         out = []
         for score, ref, _, _ in self.hits[read]:
             if ref < 0:
                 break
             _, cells, sites = self.pair(int(ref), read)
-            out.append((int(ref), int(score), cells, sites))
+            if self.both_strands:
+                out.append(self.oriented(int(ref)) + (int(score), cells, sites))
+            else:
+                out.append((int(ref), int(score), cells, sites))
         return out
+
+    def oriented(self, o: int) -> Tuple[int, int]:
+        """Oriented reference o of a both-strands result -> (reference index, strand): 0 = read as given, 1 = its
+        reverse complement."""
+        return o >> 1, o & 1
 
     @property
     def cell_offsets(self) -> np.ndarray:
@@ -296,7 +326,8 @@ class AlignResult:
 
     def pair(self, ref: int, read: int, max_cells: int | None = None):
         """(score, [(i, j)], [(beginning, ref_aln, read_aln)]) of one pair, in the reference's
-        list order -- the value OptAlignments.call returns (SmithWaterman.java:91)."""
+        list order -- the value OptAlignments.call returns (SmithWaterman.java:91).  A both-strands result takes the
+        oriented reference o as `ref`; for odd o the read string is the reverse complement of the read."""
         p = self.pair_index(ref, read)
         score = int(self.scores[ref, read]) if not hasattr(self, "_scores") else int(self._scores[ref, read])
         cnt = int(self.lib.swb_result_pair_cell_count(self.h, p))
@@ -310,7 +341,8 @@ class AlignResult:
             if score == 0:
                 sites.append((0, "", ""))
             else:
-                ra, qa = self.materialize(base + k, self.rs.seqs[ref], self.reads[read], ln.value)
+                seq = self.rs.seqs[ref >> 1] if self.both_strands else self.rs.seqs[ref]
+                ra, qa = self.materialize(base + k, seq, self.reads[read], ln.value)
                 sites.append((bg.value, ra, qa))
         return score, cells, sites
 

@@ -55,6 +55,13 @@ def merge_top_hits(records: np.ndarray) -> np.ndarray:
     return out.astype(np.int32)
 
 
+def oriented_ids(global_ids: Sequence[int]) -> np.ndarray:
+    """A shard's global reference ids -> the oriented ids a both-strands result needs (Comm.allgather_best / _hits):
+    entry 2r + s is 2 * global_ids[r] + s."""
+    g = np.asarray(global_ids, dtype=np.int64)
+    return (2 * g[:, None] + np.arange(2, dtype=np.int64)[None, :]).reshape(-1)
+
+
 def localize(best_local: np.ndarray, my_ids: Sequence[int]) -> np.ndarray:
     """Shard-local ref indices -> global ref ids."""
     out = np.array(best_local, dtype=np.int32, copy=True)
@@ -83,8 +90,8 @@ def allgather_best_hits(best_global, group=None):
 import ctypes as _C
 
 from . import _ffi
-from .engine import AlignResult, DEFAULT_SCORES, concat, _i64p
-from ._ffi import SWB_F_NO_FETCH, SWB_F_SCORES_ONLY, SWB_F_TIE_GT, check
+from .engine import AlignResult, DEFAULT_SCORES, concat, _flags, _i64p
+from ._ffi import SWB_F_NO_FETCH, SWB_F_SCORES_ONLY, SWB_F_TIE_GT, check  # noqa: F401
 
 
 class _Lib:
@@ -141,22 +148,24 @@ class MultiEngine:
         return sh.value, loc.value
 
     def align(self, reads, scores=DEFAULT_SCORES, scores_only: bool = False, fetch: bool = True, tie_gt: bool = False,
-              *, top_k: int | None = None, min_score: int = 1):
-        """top_k: hits mode (swb_multi_align_hits), every shard in hits mode and the hit lists merged (MultiResult.hits)."""
+              *, top_k: int | None = None, min_score: int = 1, both_strands: bool = False):
+        """top_k: hits mode (swb_multi_align_hits), every shard in hits mode and the hit lists merged (MultiResult.hits).
+        both_strands: SWB_F_BOTH_STRANDS; merged records and MultiResult.pair use oriented global ids 2 * ref + strand."""
         data, off, bs = concat(reads)
-        flags = (SWB_F_SCORES_ONLY if scores_only else 0) | (0 if fetch else SWB_F_NO_FETCH) | (SWB_F_TIE_GT if tie_gt else 0)
+        flags = _flags(scores_only, fetch, tie_gt, both_strands)
         h = _C.c_void_p()
         if top_k is None:
             check(self.lib.swb_multi_align(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags, _C.byref(h)))
         else:
             check(self.lib.swb_multi_align_hits(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags,
                                                 top_k, min_score, _C.byref(h)))
-        return MultiResult(self, bs, h, scores_only)
+        return MultiResult(self, bs, h, scores_only, both_strands)
 
 
 class MultiResult:
-    def __init__(self, eng: MultiEngine, reads, h, scores_only):
+    def __init__(self, eng: MultiEngine, reads, h, scores_only, both_strands: bool = False):
         self.eng, self.reads, self.h, self.scores_only = eng, reads, h, scores_only
+        self.both_strands = both_strands
         self.lib = eng.lib
         self._shards = {}
 
@@ -201,10 +210,15 @@ class MultiResult:
             ids = self.eng.shard_refs(d)
             seqs = [self.eng.seqs[int(g)] for g in ids]
             hp = _C.c_void_p(self.lib.swb_multi_result_shard(self.h, d))
-            self._shards[d] = AlignResult(_ShardRefs(self.lib, seqs), self.reads, hp, self.scores_only, owned=False).cache()
+            self._shards[d] = AlignResult(_ShardRefs(self.lib, seqs), self.reads, hp, self.scores_only, owned=False,
+                                          both_strands=self.both_strands).cache()
         return self._shards[d]
 
     def pair(self, global_ref: int, read: int, max_cells=None):
+        """A both-strands result takes the oriented global id 2 * ref + strand."""
+        if self.both_strands:
+            sh, loc = self.eng.ref_location(global_ref >> 1)
+            return self.shard(sh).pair(2 * loc + (global_ref & 1), read, max_cells)
         sh, loc = self.eng.ref_location(global_ref)
         return self.shard(sh).pair(loc, read, max_cells)
 
