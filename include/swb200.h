@@ -48,7 +48,7 @@ extern "C" {
 #define SWB_F_BOTH_STRANDS  8u  /* align every read as given AND its reverse complement (see BOTH STRANDS below) */
 
 /* BOTH STRANDS (SWB_F_BOTH_STRANDS; accepted by swb_align, swb_align_resident, swb_align_hits,
- * swb_align_resident_hits, swb_multi_align and swb_multi_align_hits, combinable with every other flag;
+ * swb_align_resident_hits, the all-hits entries, swb_multi_align and swb_multi_align_hits, combinable with every other flag;
  * swb_align_pair refuses it with SWB_E_INVALID).  Sequencing reads come from either strand; this mode aligns
  * each read q and its reverse complement rc(q) against every reference in the same call.
  *   - the result has swb_result_n_refs == 2 * R ORIENTED references over the set's R references:
@@ -146,6 +146,38 @@ int swb_align_resident_hits(swb_ctx *ctx, const swb_refset *rs, const swb_reads 
                             int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_result **out);
 /* [n_reads * k * 4] of a fetched hits-mode result (NULL before the fetch), *top_k = k; NULL and *top_k = 0 for a plain result */
 const int32_t *swb_result_hits(const swb_result *res, int32_t *top_k);
+
+/* ALL-HITS MODE: the same call, but every good hit of a read, with no cap on the count.  Every pair is still scored;
+ * with best_q = read q's best score in the call, pair (ref, q) is LISTED iff score >= min_score and
+ * score >= best_q - margin (computed in 64 bits: a large margin cannot wrap).  Arguments as swb_align /
+ * swb_align_resident plus
+ *   min_score  >= 1 (a score-0 pair is never listed)
+ *   margin     >= 0: 0 gives the co-optimal set (the multi-mapping set), INT32_MAX the plain threshold score >= min_score
+ * anything else is SWB_E_INVALID.
+ *   - lists (swb_result_hit_offsets / swb_result_hit_list): read q's entries are hit_list[4 * k ..], k = hit_offsets[q] ..
+ *     hit_offsets[q + 1] - 1, each (score, ref, i, j), score descending, then reference index ascending.  (i, j) is the
+ *     pair's first max cell in row-major order, (0, 0) under SWB_F_SCORES_ONLY.  Whenever hits mode lists k entries for
+ *     a read, its list is the first k entries of this one (same min_score, a large margin).
+ *   - scores, ref_totals and best_hits are those of the plain call, bit for bit.  Only listed pairs have max cells,
+ *     beginnings, op lengths and ops, each equal to what the plain call returns (swb_result_materialize too); every
+ *     other pair has an empty range and swb_result_pair_cell_count 0.  A read's best pair below min_score is traced
+ *     too, so best_hits keeps its (i, j).
+ *   - SWB_F_SCORES_ONLY, SWB_F_TIE_GT, SWB_F_NO_FETCH + swb_result_fetch and SWB_F_BOTH_STRANDS apply; under both
+ *     strands `ref` is the oriented index o = 2r + s and best_q is taken over both strands.  A reference set that is cut
+ *     into parts is aligned as one set here.
+ * Prefer it to hits mode when a read may have more than 32 good references (a repeat family) or when the question is
+ * a threshold, and to the plain call + a host filter when only good hits need alignments: the traceback, the assembly
+ * and the device->host copy shrink to the listed pairs.  The margin is the caller's cost knob: with a very large
+ * margin and a low min_score almost every pair is listed, and the call costs about what the plain call costs. */
+int swb_align_all_hits(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
+                       int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t min_score, int32_t margin,
+                       swb_result **out);
+int swb_align_resident_all_hits(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
+                                int32_t gap, uint32_t flags, int32_t min_score, int32_t margin, swb_result **out);
+/* fetched all-hits result: [n_reads + 1] offsets into the list, *n_hits = total; NULL / 0 for any other result */
+const int64_t *swb_result_hit_offsets(const swb_result *res, int64_t *n_hits);
+/* [n_hits * 4] (score, ref, i, j) */
+const int32_t *swb_result_hit_list(const swb_result *res);
 
 /* ONE pair through the context's submission queue.
  * Replaces: `new SmithWaterman.OptAlignments().call({ref, read}, {match, mismatch, gap}, types)` exactly as the
@@ -268,6 +300,20 @@ int  swb_multi_align_hits(swb_multi *m, int64_t n_reads, const char *read_bytes,
                           swb_multi_result **out);
 /* merged[(q * k + h) * 4 ..] = (score, GLOBAL ref index, i, j), *top_k = k; NULL and 0 for a plain result */
 const int32_t *swb_multi_result_hits(const swb_multi_result *res, int32_t *top_k);
+/* All-hits mode: swb_align_all_hits on every shard.  Each shard selects against its LOCAL best score, which is never
+ * above the global one, so a shard's list holds every pair of it that survives.  Merge: the lists -> global ids, one
+ * ncclAllGather of the per-read offsets, one host sync for the largest per-shard total, one ncclAllGather of the
+ * lists padded to that total, then a merge kernel per read: the global best from the lists' heads, the entries
+ * filtered to score >= max(min_score, global best - margin), a k-way merge in list order.  The merged lists are the
+ * same for any device count and equal to one context's lists over the whole set.  A shard result keeps the cells of
+ * its LOCAL selection, a superset of the merged one's pairs on that shard.  (Up to 64 devices.) */
+int  swb_multi_align_all_hits(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
+                              int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t min_score, int32_t margin,
+                              swb_multi_result **out);
+/* merged lists of an all-hits result: [n_reads + 1] offsets, *n_hits = total, and [n_hits * 4] (score, GLOBAL ref
+ * index, i, j); NULL / 0 for any other result */
+const int64_t *swb_multi_result_hit_offsets(const swb_multi_result *res, int64_t *n_hits);
+const int32_t *swb_multi_result_hit_list(const swb_multi_result *res);
 /* out[0] = wall ms of the call, out[1] = max over devices of the align's device ms, out[2] = allgather + merge ms */
 int  swb_multi_result_stats(const swb_multi_result *res, double *out, int n);
 
@@ -286,6 +332,12 @@ int  swb_comm_merged_device_ptr(swb_comm *c, void **ptr, int64_t *n_elems);
  * receives [n_reads * k * 4], (score, GLOBAL ref index, i, j), merged as in swb_multi_align_hits. */
 int  swb_comm_allgather_hits(swb_comm *c, const swb_result *res, const int64_t *global_ids, int64_t n_local_refs,
                              int32_t *merged_host);
+/* The same for the lists of an all-hits result (every rank passes the same min_score and margin), merged as in
+ * swb_multi_align_all_hits: *offsets = [n_reads + 1], *list = [*n_hits * 4] (score, GLOBAL ref index, i, j), host
+ * arrays owned by the communicator, valid until its next call or swb_comm_destroy.  Both strands: oriented ids as for
+ * swb_comm_allgather_hits. */
+int  swb_comm_allgather_all_hits(swb_comm *c, const swb_result *res, const int64_t *global_ids, int64_t n_local_refs,
+                                 const int64_t **offsets, const int32_t **list, int64_t *n_hits);
 
 /* Integer / DPX issue-rate microbenchmark (roofline denominator, SURVEY.md 8d). */
 int swb_microbench_json(int device, int iters, char *buf, int buflen);

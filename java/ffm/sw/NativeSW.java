@@ -45,6 +45,12 @@ final class NativeSW
 	static final MethodHandle RESULT_HITS = h( "swb_result_hits" , FunctionDescriptor.of(ADDRESS, ADDRESS, ADDRESS) ) ;
 	static final MethodHandle MULTI_ALIGN_HITS = h( "swb_multi_align_hits" , FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS) ) ;
 	static final MethodHandle MULTI_RESULT_HITS = h( "swb_multi_result_hits" , FunctionDescriptor.of(ADDRESS, ADDRESS, ADDRESS) ) ;
+	static final MethodHandle ALIGN_ALL_HITS = h( "swb_align_all_hits" , FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS) ) ;
+	static final MethodHandle RESULT_HIT_OFFSETS = h( "swb_result_hit_offsets" , FunctionDescriptor.of(ADDRESS, ADDRESS, ADDRESS) ) ;
+	static final MethodHandle RESULT_HIT_LIST = h( "swb_result_hit_list" , FunctionDescriptor.of(ADDRESS, ADDRESS) ) ;
+	static final MethodHandle MULTI_ALIGN_ALL_HITS = h( "swb_multi_align_all_hits" , FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS) ) ;
+	static final MethodHandle MULTI_RESULT_HIT_OFFSETS = h( "swb_multi_result_hit_offsets" , FunctionDescriptor.of(ADDRESS, ADDRESS, ADDRESS) ) ;
+	static final MethodHandle MULTI_RESULT_HIT_LIST = h( "swb_multi_result_hit_list" , FunctionDescriptor.of(ADDRESS, ADDRESS) ) ;
 	static final MethodHandle SCORES      = h( "swb_result_scores" , FunctionDescriptor.of(ADDRESS, ADDRESS) ) ;
 	static final MethodHandle REF_TOTALS  = h( "swb_result_ref_totals" , FunctionDescriptor.of(ADDRESS, ADDRESS) ) ;
 	static final MethodHandle CELL_OFFS   = h( "swb_result_cell_offsets" , FunctionDescriptor.of(ADDRESS, ADDRESS) ) ;

@@ -45,6 +45,12 @@ final class NativeSW
 	static native int[] bestHits( long result ) ;
 	/** hits mode: {score, ref, i, j} x topK per read, padding (0, -1, 0, 0); empty for a plain result */
 	static native int[] resultHits( long result ) ;
+	/** all-hits mode (swb_align_all_hits): every pair with score >= minScore and >= the read's best score - margin traced */
+	static native long alignAllHits( long ctx , long refset , byte[] readBytes , long[] readOffsets , int match , int mismatch , int gap , int flags , int minScore , int margin ) ;
+	/** all-hits mode: nReads + 1 offsets into resultHitList; empty for any other result */
+	static native long[] resultHitOffsets( long result ) ;
+	/** all-hits mode: {score, ref, i, j} per listed pair, read by read, score descending then ref ascending */
+	static native int[] resultHitList( long result ) ;
 	static native long[] cellOffsets( long result ) ;
 	static native int[] cells( long result ) ;
 	static native int[] beginnings( long result ) ;

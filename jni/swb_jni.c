@@ -113,6 +113,41 @@ JNIEXPORT jintArray JNICALL Java_sw_NativeSW_resultHits(JNIEnv *e, jclass c, jlo
     const int32_t *h = swb_result_hits(r, &k);
     return ints(e, h, h ? swb_result_n_reads(r) * k * 4 : 0);
 }
+/* ---- all-hits mode: every pair within `margin` of the read's best score (and >= minScore) traced (swb_align_all_hits) ---- */
+JNIEXPORT jlong JNICALL Java_sw_NativeSW_alignAllHits(JNIEnv *e, jclass c, jlong ctx, jlong refset, jbyteArray readBytes,
+                                                      jlongArray readOffsets, jint match, jint mismatch, jint gap, jint flags,
+                                                      jint minScore, jint margin)
+{
+    (void)c;
+    const jsize n = (*e)->GetArrayLength(e, readOffsets) - 1;
+    jlong *o = (jlong *)(*e)->GetPrimitiveArrayCritical(e, readOffsets, 0);
+    jbyte *b = (jbyte *)(*e)->GetPrimitiveArrayCritical(e, readBytes, 0);
+    swb_result *res = 0;
+    const int rc = swb_align_all_hits(H(swb_ctx, ctx), H(swb_refset, refset), n, (const char *)b, (const int64_t *)o, match,
+                                      mismatch, gap, (uint32_t)flags, minScore, margin, &res);
+    (*e)->ReleasePrimitiveArrayCritical(e, readBytes, b, JNI_ABORT);
+    (*e)->ReleasePrimitiveArrayCritical(e, readOffsets, o, JNI_ABORT);
+    if (rc) { throw_last(e, "swb_align_all_hits"); return 0; }
+    return (jlong)(intptr_t)res;
+}
+/* n_reads + 1 offsets into resultHitList of an all-hits result; empty for any other */
+JNIEXPORT jlongArray JNICALL Java_sw_NativeSW_resultHitOffsets(JNIEnv *e, jclass c, jlong res)
+{
+    (void)c;
+    const swb_result *r = H(swb_result, res);
+    int64_t n = 0;
+    const int64_t *off = swb_result_hit_offsets(r, &n);
+    return longs(e, off, off ? swb_result_n_reads(r) + 1 : 0);
+}
+/* {score, ref, i, j} per listed pair of an all-hits result, read by read; empty for any other */
+JNIEXPORT jintArray JNICALL Java_sw_NativeSW_resultHitList(JNIEnv *e, jclass c, jlong res)
+{
+    (void)c;
+    const swb_result *r = H(swb_result, res);
+    int64_t n = 0;
+    const int64_t *off = swb_result_hit_offsets(r, &n);
+    return ints(e, swb_result_hit_list(r), off ? n * 4 : 0);
+}
 
 /* ---- one pair through the submission queue: the unchanged driver's per-pair OptAlignments.call (Distribution.java:419-426).
  * The call may wait for other threads' requests, so the bytes are copied out instead of held critical. */

@@ -43,6 +43,12 @@ SIGNATURES = {
     "swb_align_resident_hits": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_uint32, C.c_int32, C.c_int32,
                                           C.POINTER(_P)]),
     "swb_result_hits": (_I32P, [_P, _I32P]),
+    "swb_align_all_hits": (C.c_int, [_P, _P, C.c_int64, C.c_char_p, _I64P, C.c_int32, C.c_int32, C.c_int32,
+                                     C.c_uint32, C.c_int32, C.c_int32, C.POINTER(_P)]),
+    "swb_align_resident_all_hits": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_uint32, C.c_int32, C.c_int32,
+                                              C.POINTER(_P)]),
+    "swb_result_hit_offsets": (_I64P, [_P, _I64P]),
+    "swb_result_hit_list": (_I32P, [_P]),
     "swb_result_fetch": (C.c_int, [_P]),
     "swb_result_free": (None, [_P]),
     "swb_result_n_refs": (C.c_int64, [_P]),
@@ -81,6 +87,10 @@ SIGNATURES = {
     "swb_multi_align_hits": (C.c_int, [_P, C.c_int64, C.c_char_p, _I64P, C.c_int32, C.c_int32, C.c_int32, C.c_uint32,
                                        C.c_int32, C.c_int32, C.POINTER(_P)]),
     "swb_multi_result_hits": (_I32P, [_P, _I32P]),
+    "swb_multi_align_all_hits": (C.c_int, [_P, C.c_int64, C.c_char_p, _I64P, C.c_int32, C.c_int32, C.c_int32, C.c_uint32,
+                                           C.c_int32, C.c_int32, C.POINTER(_P)]),
+    "swb_multi_result_hit_offsets": (_I64P, [_P, _I64P]),
+    "swb_multi_result_hit_list": (_I32P, [_P]),
     "swb_multi_result_stats": (C.c_int, [_P, C.POINTER(C.c_double), C.c_int]),
     # multi-GPU (one process per device)
     "swb_comm_unique_id": (C.c_int, [C.c_char_p]),
@@ -89,6 +99,7 @@ SIGNATURES = {
     "swb_comm_allgather_best": (C.c_int, [_P, _P, _I64P, C.c_int64, _I32P]),
     "swb_comm_merged_device_ptr": (C.c_int, [_P, C.POINTER(_P), _I64P]),
     "swb_comm_allgather_hits": (C.c_int, [_P, _P, _I64P, C.c_int64, _I32P]),
+    "swb_comm_allgather_all_hits": (C.c_int, [_P, _P, _I64P, C.c_int64, C.POINTER(_I64P), C.POINTER(_I32P), _I64P]),
 }
 
 _lib = None

@@ -91,7 +91,7 @@ int AlignCall::run(int32_t *ext_scores, int32_t *ext_totals)
     if (ext_totals) res->d_totals.view(ext_totals, (size_t)o_refs); else CU(res->d_totals.alloc((size_t)o_refs, st));
     CU(res->d_best.alloc((size_t)o_reads * 4, st));
     CU(cudaMemsetAsync(res->d_scores.p, 0, std::max<size_t>(n_pairs, 1) * 4, st));
-    res->top_k = top_k; res->min_score = min_score;
+    res->top_k = top_k; res->min_score = min_score; res->margin = margin;
     if (top_k > 0) CU(res->d_hits.alloc((size_t)o_reads * top_k * 4, st));
 
     const auto t_wall0 = std::chrono::steady_clock::now();
@@ -108,6 +108,7 @@ int AlignCall::run(int32_t *ext_scores, int32_t *ext_totals)
     }
     DevBuf<uint32_t> keep;
     if (top_k > 0 && (rc = select_final_hits(keep))) return rc;
+    if (margin >= 0 && (rc = select_final_all_hits(keep))) return rc;
     if ((rc = assemble(keep))) return rc;
     return finish_stats(t_wall0);
 }
@@ -204,8 +205,8 @@ int AlignCall::fill_batch(int K, const std::vector<int32_t> &reads, int64_t rp0,
             }
         }
     ++n_batches;
-    // both strands in hits mode: the selection's slots, the forward read of each read pair, follow the read pairs
-    const bool fwd_slots = both && top_k > 0 && !(flags & SWB_F_SCORES_ONLY);
+    // both strands in hits / all-hits mode: the selection's slots, the forward read of each read pair, follow the read pairs
+    const bool fwd_slots = both && selecting() && !(flags & SWB_F_SCORES_ONLY);
     if (fwd_slots)
         for (int r = 0; r < n_rp; ++r) b.h_rp.push_back(b.h_rp[(size_t)r * 2]);
     CU(ctx->rp.reserve(b.h_rp.size(), st));
@@ -244,9 +245,9 @@ int AlignCall::fill_batch(int K, const std::vector<int32_t> &reads, int64_t rp0,
 int AlignCall::trace_batch(int K, Batch &b)
 {
     const bool scores_only = (flags & SWB_F_SCORES_ONLY) != 0;
-    // hits mode: the scan makes the batch's score rows exact, the selection marks the pairs the emit keeps
+    // hits / all-hits mode: the scan makes the batch's score rows exact, the selection marks the pairs the emit keeps
     size_t sel_words = 0;
-    if (top_k > 0 && !scores_only) {
+    if (selecting() && !scores_only) {
         sel_words = ((size_t)b.n_rp * 2 * (size_t)rs->n_refs + 31) / 32;
         CU(ctx->hit_sel.reserve(sel_words, st));
         b.P.sel = ctx->hit_sel.p;
@@ -314,7 +315,12 @@ int AlignCall::locate_cells(int K, const Batch &b, size_t sel_words, uint32_t &n
             CU(cudaMemsetAsync(ctx->hit_sel.p, 0, sel_words * 4, st));
             // both strands: one slot per read pair over the 2R oriented references; oriented o = 2r + s marks bit
             // (2 * rp + s) * R + r, the emit's bit of pair (r, strand s of read pair rp)
-            if (both)
+            // all-hits mode: a batch covers all references of its reads, so each read's best score is exact here
+            if (margin >= 0 && both)
+                CU(select_margin(P.rp_reads + (size_t)b.n_rp * 2, b.n_rp, 1, ctx->hit_sel.p, 2 * rs->n_refs, rs->n_refs, true));
+            else if (margin >= 0)
+                CU(select_margin(P.rp_reads, (int64_t)b.n_rp * 2, 1, ctx->hit_sel.p, rs->n_refs, 1));
+            else if (both)
                 CU(select_hits(P.rp_reads + (size_t)b.n_rp * 2, b.n_rp, 1, nullptr, ctx->hit_sel.p, 2 * rs->n_refs, rs->n_refs, true));
             else
                 CU(select_hits(P.rp_reads, (int64_t)b.n_rp * 2, 1, nullptr, ctx->hit_sel.p, rs->n_refs, 1));
@@ -350,12 +356,23 @@ cudaError_t AlignCall::select_hits(const int32_t *slots, int64_t n_slots, int wi
     return e;
 }
 
+// all-hits mode: the per-read maximum and the marking pass of swb_hits.cu over `slots` (score rows exact by now)
+cudaError_t AlignCall::select_margin(const int32_t *slots, int64_t n_slots, int with_best, uint32_t *bits, int64_t bit_slot,
+                                     int64_t bit_ref, bool oriented_bits)
+{
+    cudaError_t e = ctx->margin_best.reserve((size_t)std::max<int64_t>(n_slots, 1), st);
+    if (e == cudaSuccess) e = launch_select_margin(res->d_scores.p, o_refs, o_reads, slots, n_slots, min_score, margin, with_best, bits,
+                                                   bit_slot, bit_ref, oriented_bits, ctx->margin_best.p, st);
+    return e;
+}
+
 // the reads of the int32 wide path; hits mode: exact scores of every wide pair first, then the whole wide path over each
-// read's top k + best pair.  Both strands: `wide` holds (q, n + q) next to each other (classify_reads); the selection
-// runs once per read q over the oriented references, and each strand takes the references of its own orientation.
+// read's top k + best pair (all-hits mode: its listed pairs + best pair, a list of any length).  Both strands: `wide`
+// holds (q, n + q) next to each other (classify_reads); the selection runs once per read q over the oriented references,
+// and each strand takes the references of its own orientation.
 int AlignCall::run_wide_reads(const std::vector<int32_t> &wide)
 {
-    if (top_k <= 0 || (flags & SWB_F_SCORES_ONLY)) return run_wide_path(wide, (flags & SWB_F_SCORES_ONLY) != 0);
+    if (!selecting() || (flags & SWB_F_SCORES_ONLY)) return run_wide_path(wide, (flags & SWB_F_SCORES_ONLY) != 0);
     int rc = run_wide_path(wide, true);
     if (rc) return rc;
     std::vector<int32_t> slots;
@@ -364,6 +381,7 @@ int AlignCall::run_wide_reads(const std::vector<int32_t> &wide)
     DevBuf<int32_t> d_wr;
     CU(d_wr.alloc((size_t)nw, st));
     CU(cudaMemcpyAsync(d_wr.p, slots.data(), (size_t)nw * 4, cudaMemcpyHostToDevice, st));
+    if (margin >= 0) return run_wide_listed(wide, d_wr.p, nw);
     CU(timer.begin(STAT_SELECT_MS));
     int4 *d_sel = reinterpret_cast<int4 *>(res->d_hits.p);              // scratch here: the final selection rewrites it
     CU(select_hits(d_wr.p, nw, 1, d_sel, nullptr, 0, 0));
@@ -384,6 +402,76 @@ int AlignCall::run_wide_reads(const std::vector<int32_t> &wide)
         std::sort(refs_of[x].begin(), refs_of[x].end());
     }
     return run_wide_path(wide, false, &refs_of);
+}
+
+// all-hits mode, wide reads: slot x's pairs to trace are bits x * o_refs + o of a bit matrix (one row per slot), which
+// the host turns into each wide read's reference list
+int AlignCall::run_wide_listed(const std::vector<int32_t> &wide, const int32_t *d_slots, int64_t nw)
+{
+    const size_t words = ((size_t)nw * (size_t)o_refs + 31) / 32;
+    DevBuf<uint32_t> d_bits;
+    CU(d_bits.alloc(words, st));
+    CU(cudaMemsetAsync(d_bits.p, 0, words * 4, st));
+    CU(timer.begin(STAT_SELECT_MS));
+    CU(select_margin(d_slots, nw, 1, d_bits.p, o_refs, 1));
+    CU(timer.end());
+    launches += 2;
+    std::vector<uint32_t> h_bits(words);
+    CU(cudaMemcpyAsync(h_bits.data(), d_bits.p, words * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    std::vector<std::vector<int32_t>> refs_of(wide.size());
+    for (size_t x = 0; x < wide.size(); ++x) {
+        const int64_t sx = both ? (int64_t)(x / 2) : (int64_t)x;
+        for (int64_t o = 0; o < o_refs; ++o) {
+            const int64_t bit = sx * o_refs + o;
+            if (!((h_bits[(size_t)(bit >> 5)] >> (bit & 31)) & 1u)) continue;
+            if (!both) refs_of[x].push_back((int32_t)o);
+            else if ((o & 1) == (int64_t)(x & 1)) refs_of[x].push_back((int32_t)(o >> 1));
+        }
+    }
+    return run_wide_path(wide, false, &refs_of);
+}
+
+// all-hits mode: the final lists over all reads (every score is exact now) and, with cells, the listed pairs as the
+// pairs whose cells the assembly keeps.  One host sync for the list's length.
+int AlignCall::select_final_all_hits(DevBuf<uint32_t> &keep)
+{
+    const size_t n_pairs = (size_t)(rs->n_refs * rd->n_reads);
+    if (!(flags & SWB_F_SCORES_ONLY)) {
+        CU(keep.alloc((n_pairs + 31) / 32, st));
+        CU(cudaMemsetAsync(keep.p, 0, ((n_pairs + 31) / 32) * 4, st));
+    }
+    CU(timer.begin(STAT_SELECT_MS));
+    CU(select_margin(nullptr, o_reads, 0, keep.p, 1, o_reads));
+    const size_t n_count = margin_count_elems(o_refs, o_reads);
+    DevBuf<int64_t> count, off;
+    DevBuf<uint8_t> tmp;
+    CU(count.alloc(n_count, st));
+    CU(off.alloc(n_count, st));
+    size_t tmp_bytes = margin_list_tmp_bytes(o_refs, o_reads, 0);
+    CU(tmp.alloc(tmp_bytes, st));
+    CU(launch_margin_count(res->d_scores.p, o_refs, o_reads, min_score, margin, ctx->margin_best.p, count.p, off.p, tmp.p, tmp_bytes, st));
+    int64_t n_hits = 0;
+    CU(cudaMemcpyAsync(&n_hits, off.p + n_count - 1, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (n_hits >= ((int64_t)1 << 31)) return fail(SWB_E_UNSUPPORTED, "swb_align_all_hits: more than 2^31 listed pairs in one call");
+    res->n_hits = n_hits;
+    CU(res->d_hit_off.alloc((size_t)o_reads + 1, st));
+    CU(res->d_hit_list.alloc((size_t)n_hits * 4, st));
+    DevBuf<int4> list_tmp;
+    DevBuf<uint64_t> keys_tmp, keys_sorted;
+    DevBuf<uint32_t> idx_tmp, order;
+    CU(list_tmp.alloc((size_t)n_hits, st));
+    CU(keys_tmp.alloc((size_t)n_hits, st)); CU(keys_sorted.alloc((size_t)n_hits, st));
+    CU(idx_tmp.alloc((size_t)n_hits, st)); CU(order.alloc((size_t)n_hits, st));
+    tmp_bytes = margin_list_tmp_bytes(o_refs, o_reads, n_hits);
+    CU(tmp.alloc(tmp_bytes, st));
+    CU(launch_margin_write(res->d_scores.p, o_refs, o_reads, min_score, margin, ctx->margin_best.p, off.p, n_hits, list_tmp.p,
+                           keys_tmp.p, keys_sorted.p, idx_tmp.p, order.p, reinterpret_cast<int4 *>(res->d_hit_list.p),
+                           res->d_hit_off.p, tmp.p, tmp_bytes, st));
+    CU(timer.end());
+    launches += 8;
+    return SWB_OK;
 }
 
 // hits mode: the final lists (every score is exact now) and, with cells, the pairs whose cells the assembly keeps
@@ -472,6 +560,10 @@ int AlignCall::assemble(const DevBuf<uint32_t> &keep)
                               res->f_cells.p, res->d_best.p, res->d_hits.p, top_k, st));
         launches += 2;
     }
+    if (margin >= 0) {
+        CU(assemble_list_cells(res->d_hit_off.p, o_reads, res->d_hit_list.p, res->n_hits, res->f_cell_off.p, res->f_cells.p, st));
+        ++launches;
+    }
     CU(cudaStreamSynchronize(st));
     res->batches.clear();                     // per-batch buffers go back to the pool
     return SWB_OK;
@@ -504,8 +596,8 @@ static int check_call(const swb_ctx *ctx, const swb_refset *rs, const swb_reads 
 
 // One packed set (a whole small set, or one part of a large one): AlignCall::run, then the fetch unless SWB_F_NO_FETCH
 static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
-                      int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, int32_t *ext_scores, int32_t *ext_totals,
-                      swb_result **out)
+                      int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, int32_t margin, int32_t *ext_scores,
+                      int32_t *ext_totals, swb_result **out)
 {
     std::lock_guard<std::recursive_mutex> lk(ctx->mu);
     CU(cudaSetDevice(ctx->device));
@@ -513,6 +605,7 @@ static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, i
     AlignCall call{ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, res.get(), ctx->stream, {ctx, ctx->stream}};
     call.both = (flags & SWB_F_BOTH_STRANDS) != 0;
     call.o_refs = res->n_refs; call.o_reads = res->n_reads;
+    call.margin = margin;
     int rc = call.run(ext_scores, ext_totals);
     if (rc) return rc;
     swb_result *r = res.release();
@@ -654,8 +747,9 @@ static int check_hits_args(const char *who, int32_t top_k, int32_t min_score)
     return SWB_OK;
 }
 
+// top_k > 0: hits mode; margin >= 0: all-hits mode
 static int align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
-                          int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_result **out)
+                          int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, int32_t margin, swb_result **out)
 {
     if (!ctx || !rs || !rd || !out) return fail(SWB_E_INVALID, "swb_align: null argument");
     *out = nullptr;
@@ -666,14 +760,15 @@ static int align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *r
     if (flags & SWB_F_BOTH_STRANDS) {
         std::unique_ptr<swb_reads> rd2;
         if ((rc = both_strands_reads(ctx, rs, rd, rd2))) return rc;
-        return align_leaf(ctx, rs->parts.empty() ? rs : rs->whole, rd2.get(), match, mismatch, gap, flags, top_k, min_score, nullptr,
-                          nullptr, out);
+        return align_leaf(ctx, rs->parts.empty() ? rs : rs->whole, rd2.get(), match, mismatch, gap, flags, top_k, min_score, margin,
+                          nullptr, nullptr, out);
     }
-    if (rs->parts.empty()) return align_leaf(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, nullptr, nullptr, out);
+    if (rs->parts.empty()) return align_leaf(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, margin, nullptr, nullptr, out);
     // hits mode also runs on the set as one: its cell arrays are small (nothing to overlap), and the selection is then
-    // over all references at once, so no part keeps cells of a pair that a later part displaces from the top k
-    if (rs->whole && ((flags & (SWB_F_NO_FETCH | SWB_F_SCORES_ONLY)) || top_k > 0))
-        return align_leaf(ctx, rs->whole, rd, match, mismatch, gap, flags, top_k, min_score, nullptr, nullptr, out);
+    // over all references at once, so no part keeps cells of a pair that a later part displaces from the top k.  The
+    // same for all-hits mode: a read's best score, and with it the margin's bar, is only known over the whole set
+    if (rs->whole && ((flags & (SWB_F_NO_FETCH | SWB_F_SCORES_ONLY)) || top_k > 0 || margin >= 0))
+        return align_leaf(ctx, rs->whole, rd, match, mismatch, gap, flags, top_k, min_score, margin, nullptr, nullptr, out);
     // ---- a set of several parts: part by part; part k's results cross PCIe while part k + 1 computes -------------
     std::lock_guard<std::recursive_mutex> lk(ctx->mu);
     CU(cudaSetDevice(ctx->device));
@@ -692,7 +787,7 @@ static int align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *r
         const swb_refset *part = rs->parts[k];
         const int64_t first = rs->part_first[k];
         swb_result *sub = nullptr;
-        rc = align_leaf(ctx, part, rd, match, mismatch, gap, flags | SWB_F_NO_FETCH, 0, 1, res->d_scores.p + (size_t)first * (size_t)n_reads,
+        rc = align_leaf(ctx, part, rd, match, mismatch, gap, flags | SWB_F_NO_FETCH, 0, 1, -1, res->d_scores.p + (size_t)first * (size_t)n_reads,
                         res->d_totals.p + first, &sub);
         if (rc) return rc;
         res->subs.push_back(sub); res->sub_first.push_back(first); res->sub_copied.push_back(0);
@@ -716,7 +811,7 @@ static int align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *r
 int swb_align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
                        int32_t gap, uint32_t flags, swb_result **out)
 {
-    return align_resident(ctx, rs, rd, match, mismatch, gap, flags, 0, 1, out);
+    return align_resident(ctx, rs, rd, match, mismatch, gap, flags, 0, 1, -1, out);
 }
 
 int swb_align_resident_hits(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
@@ -725,11 +820,28 @@ int swb_align_resident_hits(swb_ctx *ctx, const swb_refset *rs, const swb_reads 
     if (out) *out = nullptr;
     const int rc = check_hits_args("swb_align_resident_hits", top_k, min_score);
     if (rc) return rc;
-    return align_resident(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, out);
+    return align_resident(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, -1, out);
+}
+
+static int check_all_hits_args(const char *who, int32_t min_score, int32_t margin)
+{
+    if (min_score < 1) return fail(SWB_E_INVALID, std::string(who) + ": min_score must be >= 1");
+    if (margin < 0) return fail(SWB_E_INVALID, std::string(who) + ": margin must be >= 0");
+    return SWB_OK;
+}
+
+int swb_align_resident_all_hits(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
+                                int32_t gap, uint32_t flags, int32_t min_score, int32_t margin, swb_result **out)
+{
+    if (out) *out = nullptr;
+    const int rc = check_all_hits_args("swb_align_resident_all_hits", min_score, margin);
+    if (rc) return rc;
+    return align_resident(ctx, rs, rd, match, mismatch, gap, flags, 0, min_score, margin, out);
 }
 
 static int align_host(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
-                      int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_result **out)
+                      int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, int32_t margin,
+                      swb_result **out)
 {
     if (!out) return fail(SWB_E_INVALID, "swb_align: out is null");
     *out = nullptr;
@@ -746,7 +858,7 @@ static int align_host(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const
     float h2d = 0;
     cudaEventElapsedTime(&h2d, e0, e1);
     cudaEventDestroy(e0); cudaEventDestroy(e1);
-    rc = align_resident(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, out);
+    rc = align_resident(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, margin, out);
     swb_reads_free(rd);
     if (rc == SWB_OK) (*out)->stats[STAT_H2D_MS] = h2d;
     return rc;
@@ -755,7 +867,7 @@ static int align_host(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const
 int swb_align(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
               int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, swb_result **out)
 {
-    return align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, 1, out);
+    return align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, 1, -1, out);
 }
 
 int swb_align_hits(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
@@ -764,7 +876,16 @@ int swb_align_hits(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const ch
     if (out) *out = nullptr;
     const int rc = check_hits_args("swb_align_hits", top_k, min_score);
     if (rc) return rc;
-    return align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, top_k, min_score, out);
+    return align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, top_k, min_score, -1, out);
+}
+
+int swb_align_all_hits(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
+                       int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t min_score, int32_t margin, swb_result **out)
+{
+    if (out) *out = nullptr;
+    const int rc = check_all_hits_args("swb_align_all_hits", min_score, margin);
+    if (rc) return rc;
+    return align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, min_score, margin, out);
 }
 
 int swb_result_fetch(swb_result *res)
@@ -794,6 +915,10 @@ int swb_result_fetch(swb_result *res)
     if ((rc = pull(res->d_totals.p, (size_t)res->n_refs * 4, (const void **)&res->totals))) return rc;
     if ((rc = pull(res->d_best.p, (size_t)res->n_reads * 16, (const void **)&res->best))) return rc;
     if (res->top_k > 0 && (rc = pull(res->d_hits.p, (size_t)res->n_reads * res->top_k * 16, (const void **)&res->hits))) return rc;
+    if (res->margin >= 0) {
+        if ((rc = pull(res->d_hit_off.p, ((size_t)res->n_reads + 1) * 8, (const void **)&res->hit_off))) return rc;
+        if ((rc = pull(res->d_hit_list.p, (size_t)res->n_hits * 16, (const void **)&res->hit_list))) return rc;
+    }
     if (full) {
         if ((rc = pull(res->f_cell_off.p, (n_pairs + 1) * 8, (const void **)&res->cell_off))) return rc;
         if ((rc = pull(res->f_cells.p, N * 8, (const void **)&res->cells))) return rc;

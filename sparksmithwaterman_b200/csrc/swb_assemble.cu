@@ -135,6 +135,19 @@ __global__ void hit_cells_kernel(const BatchDesc *batches, int nb, const uint64_
     best[4 * q + 3] = (int32_t)(B.wide ? wide::wide_key_j(key) : key_j(key));
 }
 
+// all-hits mode, thread per list entry: its read is found in hit_off, (i, j) = the pair's first kept cell
+__global__ void list_cells_kernel(const int64_t *hit_off, int64_t n_reads, int32_t *list, int64_t n_hits, const int64_t *cell_off,
+                                  const int32_t *cells)
+{
+    const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (k >= n_hits) return;
+    int64_t lo = 0, hi = n_reads;                                  // q = last read with hit_off[q] <= k
+    while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if (hit_off[mid] <= k) lo = mid; else hi = mid; }
+    int32_t *e = list + 4 * k;
+    const int64_t p = (int64_t)e[1] * n_reads + lo;
+    if (cell_off[p + 1] > cell_off[p]) { e[2] = cells[2 * cell_off[p]]; e[3] = cells[2 * cell_off[p] + 1]; }
+}
+
 size_t assemble_tmp_bytes(uint32_t n_cells)
 {
     size_t a = 0, b = 0;
@@ -210,6 +223,15 @@ cudaError_t assemble_hit_cells(const BatchDesc *batches, int nb, const uint64_t 
     const int threads = 256;
     hit_cells_kernel<<<(unsigned)((n_reads + threads - 1) / threads), threads, 0, st>>>(batches, nb, pair_sorted, order, n_all, n_pairs,
                                                                                       n_reads, cell_off, cells, best, hits, k);
+    return cudaGetLastError();
+}
+
+cudaError_t assemble_list_cells(const int64_t *hit_off, int64_t n_reads, int32_t *list, int64_t n_hits, const int64_t *cell_off,
+                                const int32_t *cells, cudaStream_t st)
+{
+    if (n_hits == 0) return cudaSuccess;
+    const int threads = 256;
+    list_cells_kernel<<<(unsigned)((n_hits + threads - 1) / threads), threads, 0, st>>>(hit_off, n_reads, list, n_hits, cell_off, cells);
     return cudaGetLastError();
 }
 

@@ -177,6 +177,7 @@ struct swb_ctx {
     // hits mode (swb_hits.cu): partial top-k lists, the selection bits of one batch
     DevBuf<uint64_t> hit_tmp;
     DevBuf<uint32_t> hit_sel;
+    DevBuf<uint64_t> margin_best;               // all-hits mode: best key per slot of one selection
     // pinned host buffers, recycled between results (cudaHostAlloc is slow; D2H into pageable memory too)
     struct PinBuf { void *p = nullptr; size_t bytes = 0; };
     std::vector<PinBuf> pin_free;
@@ -279,6 +280,12 @@ struct swb_result {
     int32_t top_k = 0, min_score = 1;            // hits mode (swb_align_hits): k > 0
     DevBuf<int32_t> d_hits;                      // [n_reads][k][4] (score, ref, i, j)
     const int32_t *hits = nullptr;               // host view after fetch
+    int32_t margin = -1;                         // all-hits mode (swb_align_all_hits): margin >= 0
+    int64_t n_hits = 0;
+    DevBuf<int64_t> d_hit_off;                   // [n_reads + 1] offsets into d_hit_list
+    DevBuf<int32_t> d_hit_list;                  // [n_hits][4] (score, ref, i, j)
+    const int64_t *hit_off = nullptr;            // host views after fetch
+    const int32_t *hit_list = nullptr;
     std::vector<BatchOut> batches;               // released once the result is assembled
     // assembled on the device (swb_assemble.cu), ABI order
     uint32_t total_cells = 0;
@@ -349,7 +356,7 @@ int strand_complement_codes(const swb_refset *rs, uint8_t comp_code[256]);
 int both_strands_reads(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, std::unique_ptr<swb_reads> &out);
 
 // One align call over one packed set (a whole set, or one part of a large one), step by step (swb_align.cu; the wide
-// path in swb_wide_host.cu).  top_k > 0: hits mode (swb_align_hits).
+// path in swb_wide_host.cu).  top_k > 0: hits mode (swb_align_hits); margin >= 0: all-hits mode (swb_align_all_hits).
 // Two views of the pairs: the fill, locate, traceback and assembly sort run over (rs->n_refs, rd->n_reads); the
 // totals, best hits and selections over the result's oriented (o_refs, o_reads).  They are the same unless `both`
 // (SWB_F_BOTH_STRANDS): rd then holds the 2n internal reads [reads; rc(reads)], and pair r * 2n + s * n + q of the
@@ -368,6 +375,10 @@ struct AlignCall {
     double ck_bytes = 0;
     bool both = false;
     int64_t o_refs = 0, o_reads = 0;
+    int32_t margin = -1;
+
+    // hits or all-hits mode: a selection between the tile scan and the emit decides which pairs are traced
+    bool selecting() const { return top_k > 0 || margin >= 0; }
 
     struct Batch;
     int run(int32_t *ext_scores, int32_t *ext_totals);
@@ -379,10 +390,14 @@ struct AlignCall {
     int locate_cells(int K, const Batch &b, size_t sel_words, uint32_t &n_cells);
     cudaError_t select_hits(const int32_t *slots, int64_t n_slots, int with_best, int4 *hits, uint32_t *bits, int64_t bit_slot,
                             int64_t bit_ref, bool oriented_bits = false);
+    cudaError_t select_margin(const int32_t *slots, int64_t n_slots, int with_best, uint32_t *bits, int64_t bit_slot, int64_t bit_ref,
+                              bool oriented_bits = false);
     int run_wide_reads(const std::vector<int32_t> &wide);
     // refs_of (nullable): refs_of[k] = the references (ascending) read reads[k] is aligned against; nullptr = all of them
     int run_wide_path(const std::vector<int32_t> &reads, bool scores_only, const std::vector<std::vector<int32_t>> *refs_of = nullptr);
+    int run_wide_listed(const std::vector<int32_t> &wide, const int32_t *d_slots, int64_t nw);
     int select_final_hits(DevBuf<uint32_t> &keep);
+    int select_final_all_hits(DevBuf<uint32_t> &keep);
     int assemble(const DevBuf<uint32_t> &keep);
     int finish_stats(std::chrono::steady_clock::time_point t_wall0);
 };

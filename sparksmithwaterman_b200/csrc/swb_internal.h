@@ -195,6 +195,9 @@ cudaError_t assemble_kept_count(const uint64_t *pair_sorted, uint32_t n_cells, i
 cudaError_t assemble_hit_cells(const BatchDesc *batches, int nb, const uint64_t *pair_sorted, const uint32_t *order, uint32_t n_all,
                                int64_t n_pairs, int64_t n_reads, const int64_t *cell_off, const int32_t *cells, int32_t *best,
                                int32_t *hits, int k, cudaStream_t st);
+// all-hits mode: (i, j) of every list entry = its pair's first kept cell
+cudaError_t assemble_list_cells(const int64_t *hit_off, int64_t n_reads, int32_t *list, int64_t n_hits, const int64_t *cell_off,
+                                const int32_t *cells, cudaStream_t st);
 
 // swb_hits.cu: per-read top k (score desc, ref asc) of scores[ref * n_reads + q] over q = slots[s] (slots null: q = s,
 // slot -1: skipped), written to hits[s * k ..] / bits as hits_merge_kernel describes.
@@ -202,6 +205,22 @@ size_t      select_hits_tmp_elems(int64_t n_refs, int64_t n_slots, int k);
 cudaError_t launch_select_hits(const int32_t *scores, int64_t n_refs, int64_t n_reads, const int32_t *slots, int64_t n_slots,
                                int k, int32_t min_score, int with_best, int4 *hits, uint32_t *bits, int64_t bit_slot,
                                int64_t bit_ref, bool oriented_bits, uint64_t *tmp, size_t tmp_elems, cudaStream_t st);
+// all-hits mode: best[s] = key of read slots[s]'s best pair ((score << 32) | ~ref, 0 = none); bits (nullable) as
+// hits_merge_kernel for every pair with score >= max(min_score, best - margin), plus the best pair if with_best
+cudaError_t launch_select_margin(const int32_t *scores, int64_t n_refs, int64_t n_reads, const int32_t *slots, int64_t n_slots,
+                                 int32_t min_score, int32_t margin, int with_best, uint32_t *bits, int64_t bit_slot, int64_t bit_ref,
+                                 bool oriented_bits, uint64_t *best, cudaStream_t st);
+// the final lists over all reads (best from launch_select_margin with slots null): count[n_reads * chunks + 1] -> off
+// (exclusive scan; off[last] = n_hits), then list[n_hits] (score, ref, 0, 0) by read, score descending, reference
+// ascending, and hit_off[n_reads + 1]
+size_t      margin_list_tmp_bytes(int64_t n_refs, int64_t n_reads, int64_t n_hits);
+size_t      margin_count_elems(int64_t n_refs, int64_t n_reads);
+cudaError_t launch_margin_count(const int32_t *scores, int64_t n_refs, int64_t n_reads, int32_t min_score, int32_t margin,
+                                const uint64_t *best, int64_t *count, int64_t *off, void *tmp, size_t tmp_bytes, cudaStream_t st);
+cudaError_t launch_margin_write(const int32_t *scores, int64_t n_refs, int64_t n_reads, int32_t min_score, int32_t margin,
+                                const uint64_t *best, const int64_t *off, int64_t n_hits, int4 *list_tmp, uint64_t *keys_tmp,
+                                uint64_t *keys_sorted, uint32_t *idx_tmp, uint32_t *order, int4 *list, int64_t *hit_off, void *tmp,
+                                size_t tmp_bytes, cudaStream_t st);
 
 cudaError_t launch_wide_pad_reads(const uint8_t *codes, const int64_t *read_off, const int32_t *reads, int n_reads,
                                   const int64_t *rpad_off, const int64_t *rpad_len, uint8_t *rpad, int64_t max_len,

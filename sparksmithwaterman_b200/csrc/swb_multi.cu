@@ -14,6 +14,8 @@
 #include <dlfcn.h>
 #include <nccl.h>          // types and prototypes only; the entry points are looked up with dlsym
 
+#include <cub/device/device_scan.cuh>
+
 #include <chrono>
 #include <thread>
 
@@ -135,6 +137,61 @@ __global__ void merge_hits_kernel(const int32_t *gathered, int world, int64_t n_
     }
 }
 
+// all-hits mode: the world's lists, read w's list at lists[w * T ..] with offsets offs[w * (n_reads + 1) ..] (relative
+// to the list's start), each in list order.  bar = max(min_score, global best - margin), the global best being the
+// largest head; count[q] = entries >= bar over all lists
+__device__ __forceinline__ int64_t all_hits_bar(const int4 *lists, const int64_t *offs, int world, int64_t n_reads, int64_t T,
+                                                int64_t q, int32_t min_score, int32_t margin)
+{
+    int64_t best = 0;
+    for (int w = 0; w < world; ++w) {
+        const int64_t *o = offs + (int64_t)w * (n_reads + 1);
+        if (o[q + 1] > o[q]) best = max(best, (int64_t)lists[(int64_t)w * T + o[q]].x);
+    }
+    return max((int64_t)min_score, best - (int64_t)margin);
+}
+
+__global__ void all_hits_count_kernel(const int32_t *lists, const int64_t *offs, int world, int64_t n_reads, int64_t T,
+                                      int32_t min_score, int32_t margin, int64_t *count)
+{
+    const int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (q >= n_reads) return;
+    const int4 *l = reinterpret_cast<const int4 *>(lists);
+    const int64_t bar = all_hits_bar(l, offs, world, n_reads, T, q, min_score, margin);
+    int64_t n = 0;
+    for (int w = 0; w < world; ++w) {
+        const int64_t *o = offs + (int64_t)w * (n_reads + 1);
+        for (int64_t k = o[q]; k < o[q + 1] && l[(int64_t)w * T + k].x >= bar; ++k) ++n;
+    }
+    count[q] = n;
+}
+
+// k-way merge of read q's filtered lists into merged[moff[q] ..]: score descending, then global reference ascending
+__global__ void all_hits_merge_kernel(const int32_t *lists, const int64_t *offs, int world, int64_t n_reads, int64_t T,
+                                      int32_t min_score, int32_t margin, const int64_t *moff, int32_t *merged)
+{
+    const int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (q >= n_reads) return;
+    const int4 *l = reinterpret_cast<const int4 *>(lists);
+    const int64_t bar = all_hits_bar(l, offs, world, n_reads, T, q, min_score, margin);
+    int64_t pos[kMaxHitsWorld];
+    for (int w = 0; w < world; ++w) pos[w] = offs[(int64_t)w * (n_reads + 1) + q];
+    int4 *out = reinterpret_cast<int4 *>(merged);
+    for (int64_t h = moff[q]; h < moff[q + 1]; ++h) {
+        int bw = -1;
+        int4 best = make_int4(0, -1, 0, 0);
+        for (int w = 0; w < world; ++w) {
+            if (pos[w] >= offs[(int64_t)w * (n_reads + 1) + q + 1]) continue;
+            const int4 e = l[(int64_t)w * T + pos[w]];
+            if (e.x < bar) continue;
+            if (bw < 0 || e.x > best.x || (e.x == best.x && e.y < best.y)) { best = e; bw = w; }
+        }
+        if (bw < 0) break;
+        ++pos[bw];
+        out[h] = best;
+    }
+}
+
 // send/gather/merge buffers of one device
 struct GatherBufs {
     DevBuf<int32_t> send, gathered, merged;
@@ -142,7 +199,17 @@ struct GatherBufs {
     DevBuf<int64_t> ids;
     int64_t n_ids = 0;
     DevBuf<int64_t> oids;                        // both strands: oriented local 2r + s -> oriented global 2 * ids[r] + s
-    void release() { send.release(); gathered.release(); merged.release(); hsend.release(); hgathered.release(); hmerged.release(); ids.release(); oids.release(); }
+    // all-hits mode: gathered offsets [world][n_reads + 1], lists padded to the largest total [world][T][4], the merge
+    DevBuf<int64_t> aoffs, acount, amoff;
+    DevBuf<int32_t> asend, alists, amerged;
+    DevBuf<uint8_t> atmp;
+    std::vector<int64_t> h_off;                  // merged lists on the host
+    std::vector<int32_t> h_list;
+    void release()
+    {
+        send.release(); gathered.release(); merged.release(); hsend.release(); hgathered.release(); hmerged.release(); ids.release(); oids.release();
+        aoffs.release(); acount.release(); amoff.release(); asend.release(); alists.release(); amerged.release(); atmp.release();
+    }
 };
 
 // localize -> allgather -> merge on `st` of the current device.  `grouped`: the caller brackets several devices'
@@ -186,6 +253,49 @@ cudaError_t enqueue_merge_hits(GatherBufs &g, int64_t n_reads, int k, int world,
     return cudaGetLastError();
 }
 
+// all-hits mode, step 1: the list of `res` -> global ids in g.asend (room for T entries)
+cudaError_t enqueue_localize_all_hits(GatherBufs &g, const int64_t *ids, int64_t n_ids, const swb_result *res, int64_t T, int world,
+                                      cudaStream_t st)
+{
+    cudaError_t e = g.asend.reserve((size_t)std::max<int64_t>(T, 1) * 4, st);
+    if (e == cudaSuccess) e = g.aoffs.reserve((size_t)(res->n_reads + 1) * world, st);
+    if (e == cudaSuccess) e = g.alists.reserve((size_t)std::max<int64_t>(T, 1) * 4 * world, st);
+    if (e != cudaSuccess || res->n_hits == 0) return e;
+    const int threads = 256;
+    hits_to_global_kernel<<<(unsigned)((res->n_hits + threads - 1) / threads), threads, 0, st>>>(res->d_hit_list.p, ids, n_ids, res->n_hits,
+                                                                                               g.asend.p);
+    return cudaGetLastError();
+}
+
+// all-hits mode, last step (after the gathers into g.aoffs / g.alists): count, scan, one sync for the merged length,
+// k-way merge, merged lists -> g.h_off / g.h_list
+int merge_all_hits(GatherBufs &g, int world, int64_t n_reads, int64_t T, int32_t min_score, int32_t margin, cudaStream_t st)
+{
+    const int threads = 128;
+    const unsigned blocks = (unsigned)((n_reads + threads - 1) / threads);
+    CU(g.acount.reserve((size_t)n_reads + 1, st));
+    CU(g.amoff.reserve((size_t)n_reads + 1, st));
+    CU(cudaMemsetAsync(g.acount.p + n_reads, 0, 8, st));
+    if (n_reads) all_hits_count_kernel<<<blocks, threads, 0, st>>>(g.alists.p, g.aoffs.p, world, n_reads, T, min_score, margin, g.acount.p);
+    CU(cudaGetLastError());
+    size_t tmp_bytes = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, (const int64_t *)nullptr, (int64_t *)nullptr, (int)n_reads + 1);
+    CU(g.atmp.reserve(std::max<size_t>(tmp_bytes, 1), st));
+    CU(cub::DeviceScan::ExclusiveSum(g.atmp.p, tmp_bytes, g.acount.p, g.amoff.p, (int)n_reads + 1, st));
+    g.h_off.assign((size_t)n_reads + 1, 0);
+    CU(cudaMemcpyAsync(g.h_off.data(), g.amoff.p, ((size_t)n_reads + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    const int64_t n = g.h_off[(size_t)n_reads];
+    g.h_list.assign((size_t)n * 4, 0);
+    if (n == 0) return SWB_OK;
+    CU(g.amerged.reserve((size_t)n * 4, st));
+    all_hits_merge_kernel<<<blocks, threads, 0, st>>>(g.alists.p, g.aoffs.p, world, n_reads, T, min_score, margin, g.amoff.p, g.amerged.p);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(g.h_list.data(), g.amerged.p, (size_t)n * 16, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return SWB_OK;
+}
+
 }  // namespace
 
 struct swb_comm {
@@ -215,6 +325,9 @@ struct swb_multi_result {
     std::vector<int32_t> merged;
     int32_t top_k = 0;                           // hits mode: merged_hits = [n_reads][k][4], global reference ids
     std::vector<int32_t> merged_hits;
+    bool all_hits = false;                       // all-hits mode: merged lists, global reference ids
+    std::vector<int64_t> merged_off;
+    std::vector<int32_t> merged_list;
     int64_t n_reads = 0;
     double stats[3] = {0, 0, 0};
 };
@@ -318,6 +431,49 @@ int swb_comm_allgather_hits(swb_comm *c, const swb_result *res, const int64_t *g
     CU(enqueue_merge_hits(c->g, n_reads, k, c->world, st));
     if (merged_host && n) CU(cudaMemcpyAsync(merged_host, c->g.hmerged.p, n * 16, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));        // global_ids / merged_host are the caller's
+    return SWB_OK;
+}
+
+int swb_comm_allgather_all_hits(swb_comm *c, const swb_result *res, const int64_t *global_ids, int64_t n_local_refs,
+                                const int64_t **offsets, const int32_t **list, int64_t *n_hits)
+{
+    if (!c || !res || !offsets || !list || !n_hits) return fail(SWB_E_INVALID, "swb_comm_allgather_all_hits: null argument");
+    *offsets = nullptr; *list = nullptr; *n_hits = 0;
+    if (res->ctx != c->ctx) return fail(SWB_E_INVALID, "swb_comm_allgather_all_hits: the result belongs to another context");
+    if (res->margin < 0) return fail(SWB_E_INVALID, "swb_comm_allgather_all_hits: not an all-hits result (swb_align_all_hits)");
+    if (c->world > kMaxHitsWorld) return fail(SWB_E_UNSUPPORTED, "swb_comm_allgather_all_hits: more than 64 ranks");
+    if (n_local_refs != res->n_refs) return fail(SWB_E_INVALID, "swb_comm_allgather_all_hits: global_ids must cover the shard's references");
+    if (n_local_refs > 0 && !global_ids) return fail(SWB_E_INVALID, "swb_comm_allgather_all_hits: global_ids is null");
+    swb_ctx *ctx = c->ctx;
+    std::lock_guard<std::recursive_mutex> lk(ctx->mu);
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const int64_t n_reads = res->n_reads, no = n_reads + 1;
+    const int world = c->world;
+    CU(c->g.ids.reserve((size_t)std::max<int64_t>(n_local_refs, 1), st));
+    c->g.n_ids = n_local_refs;
+    if (n_local_refs) CU(cudaMemcpyAsync(c->g.ids.p, global_ids, (size_t)n_local_refs * 8, cudaMemcpyHostToDevice, st));
+    CU(c->g.aoffs.reserve((size_t)no * world, st));
+    // the per-read offsets, then the largest total (one host sync), then the lists padded to it
+    int64_t T = res->n_hits;
+    if (world > 1) {
+        NC(nccl_api()->AllGather(res->d_hit_off.p, c->g.aoffs.p, (size_t)no, ncclInt64, c->comm, st));
+        std::vector<int64_t> h((size_t)no * world);
+        CU(cudaMemcpyAsync(h.data(), c->g.aoffs.p, h.size() * 8, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        for (int w = 0; w < world; ++w) T = std::max(T, h[(size_t)w * no + n_reads]);
+    } else {
+        CU(cudaMemcpyAsync(c->g.aoffs.p, res->d_hit_off.p, (size_t)no * 8, cudaMemcpyDeviceToDevice, st));
+    }
+    CU(enqueue_localize_all_hits(c->g, c->g.ids.p, c->g.n_ids, res, T, world, st));
+    if (world > 1) {
+        if (T) NC(nccl_api()->AllGather(c->g.asend.p, c->g.alists.p, (size_t)T * 4, ncclInt32, c->comm, st));
+    } else if (T) {
+        CU(cudaMemcpyAsync(c->g.alists.p, c->g.asend.p, (size_t)T * 16, cudaMemcpyDeviceToDevice, st));
+    }
+    const int rc = merge_all_hits(c->g, world, n_reads, T, res->min_score, res->margin, st);
+    if (rc) return rc;
+    *offsets = c->g.h_off.data(); *list = c->g.h_list.data(); *n_hits = c->g.h_off[(size_t)n_reads];
     return SWB_OK;
 }
 
@@ -461,20 +617,22 @@ const int64_t *swb_multi_shard_refs(const swb_multi *m, int32_t d, int64_t *n)
 
 }  // extern "C"
 
-// top_k > 0: hits mode (swb_multi_align_hits)
+// top_k > 0: hits mode (swb_multi_align_hits); margin >= 0: all-hits mode (swb_multi_align_all_hits)
 static int multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
-                       int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_multi_result **out)
+                       int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, int32_t margin,
+                       swb_multi_result **out)
 {
     if (!m || !out) return fail(SWB_E_INVALID, "swb_multi_align: null argument");
     *out = nullptr;
     const int n = (int)m->ctx.size();
     if (top_k > 0 && n > kMaxHitsWorld) return fail(SWB_E_UNSUPPORTED, "swb_multi_align_hits: more than 64 devices");
+    if (margin >= 0 && n > kMaxHitsWorld) return fail(SWB_E_UNSUPPORTED, "swb_multi_align_all_hits: more than 64 devices");
     for (int d = 0; d < n; ++d)
         if (!m->rs[(size_t)d]) return fail(SWB_E_INVALID, "swb_multi_align: no reference set loaded");
     std::lock_guard<std::mutex> lk(m->mu);
     const auto t0 = std::chrono::steady_clock::now();
     std::unique_ptr<swb_multi_result> res(new swb_multi_result());
-    res->m = m; res->n_reads = n_reads; res->top_k = top_k;
+    res->m = m; res->n_reads = n_reads; res->top_k = top_k; res->all_hits = margin >= 0;
     res->shard.assign((size_t)n, nullptr);
     auto drop = [&] { for (swb_result *r : res->shard) if (r) swb_result_free(r); res->shard.clear(); };
 
@@ -488,6 +646,9 @@ static int multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, co
                 rcs[(size_t)d] = top_k > 0
                     ? swb_align_hits(m->ctx[(size_t)d], m->rs[(size_t)d], n_reads, read_bytes, read_offsets, match, mismatch, gap,
                                      flags | SWB_F_NO_FETCH, top_k, min_score, &res->shard[(size_t)d])
+                    : margin >= 0
+                    ? swb_align_all_hits(m->ctx[(size_t)d], m->rs[(size_t)d], n_reads, read_bytes, read_offsets, match, mismatch, gap,
+                                         flags | SWB_F_NO_FETCH, min_score, margin, &res->shard[(size_t)d])
                     : swb_align(m->ctx[(size_t)d], m->rs[(size_t)d], n_reads, read_bytes, read_offsets, match, mismatch,
                                 gap, flags | SWB_F_NO_FETCH, &res->shard[(size_t)d]);
                 if (rcs[(size_t)d]) errs[(size_t)d] = swb_last_error();
@@ -502,6 +663,10 @@ static int multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, co
     // merge's order is the single-context order over the oriented references
     const auto t1 = std::chrono::steady_clock::now();
     const bool both = (flags & SWB_F_BOTH_STRANDS) != 0;
+    // all-hits mode: the shards' list lengths are known on the host after their calls; T = the largest
+    int64_t T = 0;
+    if (margin >= 0)
+        for (int d = 0; d < n; ++d) T = std::max(T, res->shard[(size_t)d]->n_hits);
     for (int d = 0; d < n; ++d) {
         swb_ctx *c = m->ctx[(size_t)d];
         GatherBufs &g = m->g[(size_t)d];
@@ -511,6 +676,7 @@ static int multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, co
         if (e == cudaSuccess) e = enqueue_localize(g, ids, n_ids, res->shard[(size_t)d]->d_best.p, n_reads, n, c->stream);
         if (e == cudaSuccess && top_k > 0)
             e = enqueue_localize_hits(g, ids, n_ids, res->shard[(size_t)d]->d_hits.p, n_reads, top_k, n, c->stream);
+        if (e == cudaSuccess && margin >= 0) e = enqueue_localize_all_hits(g, ids, n_ids, res->shard[(size_t)d], T, n, c->stream);
         if (e != cudaSuccess) { drop(); return cuda_fail(e, "swb_multi_align: best hits -> global ids"); }
     }
     if (n > 1 && n_reads > 0) {
@@ -522,6 +688,12 @@ static int multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, co
             if (r == ncclSuccess && top_k > 0)
                 r = a->AllGather(m->g[(size_t)d].hsend.p, m->g[(size_t)d].hgathered.p, (size_t)n_reads * top_k * 4, ncclInt32,
                                  m->comms[(size_t)d], m->ctx[(size_t)d]->stream);
+            if (r == ncclSuccess && margin >= 0)
+                r = a->AllGather(res->shard[(size_t)d]->d_hit_off.p, m->g[(size_t)d].aoffs.p, (size_t)n_reads + 1, ncclInt64,
+                                 m->comms[(size_t)d], m->ctx[(size_t)d]->stream);
+            if (r == ncclSuccess && margin >= 0 && T > 0)
+                r = a->AllGather(m->g[(size_t)d].asend.p, m->g[(size_t)d].alists.p, (size_t)T * 4, ncclInt32, m->comms[(size_t)d],
+                                 m->ctx[(size_t)d]->stream);
         }
         const ncclResult_t r2 = a->GroupEnd();
         if (r == ncclSuccess) r = r2;
@@ -546,6 +718,20 @@ static int multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, co
                 e = cudaMemcpyAsync(res->merged_hits.data(), g.hmerged.p, (size_t)n_reads * top_k * 16, cudaMemcpyDeviceToHost, c->stream);
         }
         if (e != cudaSuccess) { drop(); return cuda_fail(e, "swb_multi_align: merge"); }
+    }
+    // all-hits mode: the lists are merged on device 0 (one more host sync there for the merged length)
+    if (margin >= 0) {
+        swb_ctx *c = m->ctx[0];
+        GatherBufs &g = m->g[0];
+        cudaError_t e = cudaSetDevice(c->device);
+        if (e == cudaSuccess && n == 1)
+            e = cudaMemcpyAsync(g.aoffs.p, res->shard[0]->d_hit_off.p, ((size_t)n_reads + 1) * 8, cudaMemcpyDeviceToDevice, c->stream);
+        if (e == cudaSuccess && n == 1 && T > 0)
+            e = cudaMemcpyAsync(g.alists.p, g.asend.p, (size_t)T * 16, cudaMemcpyDeviceToDevice, c->stream);
+        if (e != cudaSuccess) { drop(); return cuda_fail(e, "swb_multi_align_all_hits: merge"); }
+        const int rc = merge_all_hits(g, n, n_reads, T, min_score, margin, c->stream);
+        if (rc) { const std::string err = swb_last_error(); drop(); return fail(rc, err); }
+        res->merged_off = g.h_off; res->merged_list = g.h_list;
     }
     for (int d = 0; d < n; ++d) {
         cudaSetDevice(m->ctx[(size_t)d]->device);
@@ -578,7 +764,7 @@ extern "C" {
 int swb_multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
                     int32_t mismatch, int32_t gap, uint32_t flags, swb_multi_result **out)
 {
-    return multi_align(m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, 1, out);
+    return multi_align(m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, 1, -1, out);
 }
 
 int swb_multi_align_hits(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
@@ -587,7 +773,16 @@ int swb_multi_align_hits(swb_multi *m, int64_t n_reads, const char *read_bytes, 
     if (out) *out = nullptr;
     if (top_k < 1 || top_k > 32) return fail(SWB_E_INVALID, "swb_multi_align_hits: top_k must be 1 .. 32");
     if (min_score < 1) return fail(SWB_E_INVALID, "swb_multi_align_hits: min_score must be >= 1");
-    return multi_align(m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, top_k, min_score, out);
+    return multi_align(m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, top_k, min_score, -1, out);
+}
+
+int swb_multi_align_all_hits(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
+                             int32_t mismatch, int32_t gap, uint32_t flags, int32_t min_score, int32_t margin, swb_multi_result **out)
+{
+    if (out) *out = nullptr;
+    if (min_score < 1) return fail(SWB_E_INVALID, "swb_multi_align_all_hits: min_score must be >= 1");
+    if (margin < 0) return fail(SWB_E_INVALID, "swb_multi_align_all_hits: margin must be >= 0");
+    return multi_align(m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, min_score, margin, out);
 }
 
 void swb_multi_result_free(swb_multi_result *res)
@@ -608,6 +803,13 @@ const int32_t *swb_multi_result_hits(const swb_multi_result *res, int32_t *top_k
     if (top_k) *top_k = ok ? res->top_k : 0;
     return ok ? res->merged_hits.data() : nullptr;
 }
+const int64_t *swb_multi_result_hit_offsets(const swb_multi_result *res, int64_t *n_hits)
+{
+    const bool ok = res && res->all_hits;
+    if (n_hits) *n_hits = ok ? res->merged_off[(size_t)res->n_reads] : 0;
+    return ok ? res->merged_off.data() : nullptr;
+}
+const int32_t *swb_multi_result_hit_list(const swb_multi_result *res) { return (res && res->all_hits) ? res->merged_list.data() : nullptr; }
 int swb_multi_result_stats(const swb_multi_result *res, double *out, int n)
 {
     if (!res || !out) return fail(SWB_E_INVALID, "swb_multi_result_stats: null");

@@ -40,6 +40,13 @@ def reverse_complement(seq) -> bytes:
     return _b(seq).translate(COMPLEMENT)[::-1]
 
 
+def _mode(top_k, margin) -> str:
+    """Which entry a call takes: "plain", "hits" (top_k) or "all_hits" (margin); both at once is a ValueError."""
+    if top_k is not None and margin is not None:
+        raise ValueError("top_k (hits mode) and margin (all-hits mode) select different modes: pass one of them")
+    return "plain" if top_k is None and margin is None else ("hits" if margin is None else "all_hits")
+
+
 def _flags(scores_only: bool, fetch: bool, tie_gt: bool, both_strands: bool) -> int:
     return ((SWB_F_SCORES_ONLY if scores_only else 0) | (0 if fetch else SWB_F_NO_FETCH) | (SWB_F_TIE_GT if tie_gt else 0)
             | (SWB_F_BOTH_STRANDS if both_strands else 0))
@@ -131,21 +138,29 @@ class RefSet:
 
     def align(self, reads, scores=DEFAULT_SCORES, scores_only: bool = False, fetch: bool = True,
               tie_gt: bool = False, *, top_k: int | None = None, min_score: int = 1,
-              both_strands: bool = False) -> "AlignResult":
+              both_strands: bool = False, margin: int | None = None) -> "AlignResult":
         """Host-buffer path (swb_align): H2D of the reads, compute, D2H of the results.
         tie_gt: DistributedSW's strict-'>' tie rule in the traceback (SWB_F_TIE_GT).
         top_k: hits mode (swb_align_hits) -- every pair is scored, but only each read's top_k best pairs with
         score >= min_score are traced (AlignResult.hits / read_hits).
+        margin: all-hits mode (swb_align_all_hits) -- every pair with score >= min_score and score >= the read's best
+        score - margin is listed and traced, with no cap on the count (AlignResult.hit_offsets / hit_list / read_hits).
+        margin=0 gives each read's co-optimal references.  Passing both top_k and margin is a ValueError.
         both_strands: every read and its reverse complement (SWB_F_BOTH_STRANDS); the result has 2 * n_refs oriented
         references, o = 2r (read as given) and o = 2r + 1 (reverse complement) -- AlignResult.oriented."""
         if isinstance(reads, Reads):
-            return reads.align(scores, scores_only, fetch, tie_gt, top_k=top_k, min_score=min_score, both_strands=both_strands)
+            return reads.align(scores, scores_only, fetch, tie_gt, top_k=top_k, min_score=min_score, both_strands=both_strands,
+                               margin=margin)
+        mode = _mode(top_k, margin)
         data, off, bs = concat(reads)
         flags = _flags(scores_only, fetch, tie_gt, both_strands)
         h = C.c_void_p()
-        if top_k is None:
+        if mode == "plain":
             check(self.eng.lib.swb_align(self.eng.h, self.h, len(bs), data, _i64p(off),
                                          scores[0], scores[1], scores[2], flags, C.byref(h)))
+        elif mode == "all_hits":
+            check(self.eng.lib.swb_align_all_hits(self.eng.h, self.h, len(bs), data, _i64p(off),
+                                                  scores[0], scores[1], scores[2], flags, min_score, margin, C.byref(h)))
         else:
             check(self.eng.lib.swb_align_hits(self.eng.h, self.h, len(bs), data, _i64p(off),
                                               scores[0], scores[1], scores[2], flags, top_k, min_score, C.byref(h)))
@@ -177,12 +192,16 @@ class Reads:
 
     def align(self, scores=DEFAULT_SCORES, scores_only: bool = False, fetch: bool = True,
               tie_gt: bool = False, *, top_k: int | None = None, min_score: int = 1,
-              both_strands: bool = False) -> "AlignResult":
+              both_strands: bool = False, margin: int | None = None) -> "AlignResult":
+        mode = _mode(top_k, margin)
         flags = _flags(scores_only, fetch, tie_gt, both_strands)
         h = C.c_void_p()
         lib = self.rs.eng.lib
-        if top_k is None:
+        if mode == "plain":
             check(lib.swb_align_resident(self.rs.eng.h, self.rs.h, self.h, scores[0], scores[1], scores[2], flags, C.byref(h)))
+        elif mode == "all_hits":
+            check(lib.swb_align_resident_all_hits(self.rs.eng.h, self.rs.h, self.h, scores[0], scores[1], scores[2], flags,
+                                                  min_score, margin, C.byref(h)))
         else:
             check(lib.swb_align_resident_hits(self.rs.eng.h, self.rs.h, self.h, scores[0], scores[1], scores[2], flags,
                                               top_k, min_score, C.byref(h)))
@@ -253,11 +272,32 @@ class AlignResult:
             return np.zeros((self.n_reads, 0, 4), np.int32)
         return self._arr(p, self.n_reads * k.value * 4, np.int32).reshape(self.n_reads, k.value, 4)
 
+    @property
+    def hit_offsets(self) -> np.ndarray:
+        """All-hits mode: [n_reads + 1] int64, read q's entries are hit_list[hit_offsets[q]:hit_offsets[q + 1]].
+        Empty for any other result (or before the fetch)."""
+        n = C.c_int64()
+        p = self.lib.swb_result_hit_offsets(self.h, C.byref(n))
+        return self._arr(p, self.n_reads + 1, np.int64) if p else np.zeros(0, np.int64)
+
+    @property
+    def hit_list(self) -> np.ndarray:
+        """All-hits mode: [n_hits, 4] int32 (score, ref, i, j), per read score descending then ref ascending."""
+        n = C.c_int64()
+        self.lib.swb_result_hit_offsets(self.h, C.byref(n))
+        return self._arr(self.lib.swb_result_hit_list(self.h), n.value * 4, np.int32).reshape(-1, 4)
+
+    def _read_entries(self, read: int) -> np.ndarray:
+        off = self.hit_offsets
+        if len(off):
+            return self.hit_list[off[read]:off[read + 1]]
+        return self.hits[read]
+
     def read_hits(self, read: int):
-        """Hits mode: [(ref, score, cells, sites)] of read `read`'s hits in hit order; cells / sites as pair().
-        A both-strands result gives [(ref, strand, score, cells, sites)], ref the reference's own index."""
+        """Hits or all-hits mode: [(ref, score, cells, sites)] of read `read`'s hits in hit order; cells / sites as
+        pair().  A both-strands result gives [(ref, strand, score, cells, sites)], ref the reference's own index."""
         out = []
-        for score, ref, _, _ in self.hits[read]:
+        for score, ref, _, _ in self._read_entries(read):
             if ref < 0:
                 break
             _, cells, sites = self.pair(int(ref), read)

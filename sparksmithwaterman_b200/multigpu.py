@@ -55,6 +55,29 @@ def merge_top_hits(records: np.ndarray) -> np.ndarray:
     return out.astype(np.int32)
 
 
+def merge_all_hits(offsets: Sequence[np.ndarray], lists: Sequence[np.ndarray], min_score: int, margin: int):
+    """All-hits merge over ranks.  Rank w's lists: offsets[w] [n_reads + 1] and lists[w] [n_w, 4] (score, global ref
+    id, i, j), each read's entries in list order (score descending, then ref ascending), selected against the rank's
+    LOCAL best.  The global best of read q is the largest head; its entries with score >= max(min_score, best - margin)
+    over all ranks, in list order, are read q's merged list.  Returns (offsets [n_reads + 1] int64, list [n, 4] int32)."""
+    n_reads = len(offsets[0]) - 1
+    out_off, out = [0], []
+    for q in range(n_reads):
+        parts = [np.asarray(l, dtype=np.int64).reshape(-1, 4)[o[q]:o[q + 1]] for o, l in zip(offsets, lists)]
+        parts = [p for p in parts if len(p)]
+        if parts:
+            e = np.concatenate(parts)
+            bar = max(int(min_score), int(e[:, 0].max()) - int(margin))
+            e = e[e[:, 0] >= bar]
+            e = e[np.lexsort((e[:, 1], -e[:, 0]))]
+            out.append(e)
+            out_off.append(out_off[-1] + len(e))
+        else:
+            out_off.append(out_off[-1])
+    lst = np.concatenate(out).astype(np.int32) if out else np.zeros((0, 4), np.int32)
+    return np.asarray(out_off, dtype=np.int64), lst.reshape(-1, 4)
+
+
 def oriented_ids(global_ids: Sequence[int]) -> np.ndarray:
     """A shard's global reference ids -> the oriented ids a both-strands result needs (Comm.allgather_best / _hits):
     entry 2r + s is 2 * global_ids[r] + s."""
@@ -90,7 +113,7 @@ def allgather_best_hits(best_global, group=None):
 import ctypes as _C
 
 from . import _ffi
-from .engine import AlignResult, DEFAULT_SCORES, concat, _flags, _i64p
+from .engine import AlignResult, DEFAULT_SCORES, concat, _flags, _i64p, _mode
 from ._ffi import SWB_F_NO_FETCH, SWB_F_SCORES_ONLY, SWB_F_TIE_GT, check  # noqa: F401
 
 
@@ -148,14 +171,19 @@ class MultiEngine:
         return sh.value, loc.value
 
     def align(self, reads, scores=DEFAULT_SCORES, scores_only: bool = False, fetch: bool = True, tie_gt: bool = False,
-              *, top_k: int | None = None, min_score: int = 1, both_strands: bool = False):
+              *, top_k: int | None = None, min_score: int = 1, both_strands: bool = False, margin: int | None = None):
         """top_k: hits mode (swb_multi_align_hits), every shard in hits mode and the hit lists merged (MultiResult.hits).
+        margin: all-hits mode (swb_multi_align_all_hits), the lists merged (MultiResult.hit_offsets / hit_list).
         both_strands: SWB_F_BOTH_STRANDS; merged records and MultiResult.pair use oriented global ids 2 * ref + strand."""
+        mode = _mode(top_k, margin)
         data, off, bs = concat(reads)
         flags = _flags(scores_only, fetch, tie_gt, both_strands)
         h = _C.c_void_p()
-        if top_k is None:
+        if mode == "plain":
             check(self.lib.swb_multi_align(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags, _C.byref(h)))
+        elif mode == "all_hits":
+            check(self.lib.swb_multi_align_all_hits(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags,
+                                                    min_score, margin, _C.byref(h)))
         else:
             check(self.lib.swb_multi_align_hits(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags,
                                                 top_k, min_score, _C.byref(h)))
@@ -197,6 +225,23 @@ class MultiResult:
         if not p or n == 0:
             return np.zeros((n, k.value, 4), np.int32)
         return np.ctypeslib.as_array(p, shape=(n * k.value * 4,)).copy().reshape(n, k.value, 4)
+
+    @property
+    def hit_offsets(self) -> np.ndarray:
+        """All-hits mode: merged [n_reads + 1] offsets into hit_list; empty for any other result."""
+        n = _C.c_int64()
+        p = self.lib.swb_multi_result_hit_offsets(self.h, _C.byref(n))
+        return np.ctypeslib.as_array(p, shape=(len(self.reads) + 1,)).copy() if p else np.zeros(0, np.int64)
+
+    @property
+    def hit_list(self) -> np.ndarray:
+        """All-hits mode: merged [n_hits, 4] (score, GLOBAL ref id, i, j)."""
+        n = _C.c_int64()
+        self.lib.swb_multi_result_hit_offsets(self.h, _C.byref(n))
+        p = self.lib.swb_multi_result_hit_list(self.h)
+        if not p or n.value == 0:
+            return np.zeros((0, 4), np.int32)
+        return np.ctypeslib.as_array(p, shape=(n.value * 4,)).copy().reshape(-1, 4)
 
     @property
     def stats(self) -> dict:
@@ -265,3 +310,13 @@ class Comm:
         check(self.lib.swb_comm_allgather_hits(self.h, res.h, _i64p(ids), len(ids),
                                                out.ctypes.data_as(_C.POINTER(_C.c_int32)) if out.size else None))
         return out
+
+    def allgather_all_hits(self, res: AlignResult, global_ids):
+        """Lists of an all-hits result of this rank's shard -> merged (offsets [n_reads + 1], list [n, 4]) with global
+        ref ids."""
+        ids = np.ascontiguousarray(global_ids, dtype=np.int64)
+        po, pl, n = _C.POINTER(_C.c_int64)(), _C.POINTER(_C.c_int32)(), _C.c_int64()
+        check(self.lib.swb_comm_allgather_all_hits(self.h, res.h, _i64p(ids), len(ids), _C.byref(po), _C.byref(pl), _C.byref(n)))
+        off = np.ctypeslib.as_array(po, shape=(res.n_reads + 1,)).copy()
+        lst = np.ctypeslib.as_array(pl, shape=(n.value * 4,)).copy().reshape(-1, 4) if n.value else np.zeros((0, 4), np.int32)
+        return off, lst
