@@ -110,6 +110,34 @@ def align(ref, read, match: int = 5, mismatch: int = -3, gap: int = -4,
         L.sw_oracle_free(C.byref(r))
 
 
+def align_raw(ref, read, match: int = 5, mismatch: int = -3, gap: int = -4, lowmem: bool = False,
+              tie_gt: bool = False) -> dict:
+    """One pair through the C oracle as numpy arrays, copied in bulk: score, cells [n, 2] int32, beginnings [n] int32,
+    aln_off [n + 1] int64, and the concatenated aligned strings ref_aln / read_aln as uint8.  Same order as align()."""
+    import numpy as np
+    L = lib()
+    ref_b, read_b = _b(ref), _b(read)
+    r = _Result()
+    fn = L.sw_oracle_align_gt if tie_gt else (L.sw_oracle_align_lowmem if lowmem else L.sw_oracle_align)
+    if fn(ref_b, len(ref_b), read_b, len(read_b), match, mismatch, gap, C.byref(r)) != 0:
+        raise MemoryError("oracle allocation failed")
+    try:
+        n = int(r.n_cells)
+
+        def arr(ptr, k, dtype):
+            return np.ctypeslib.as_array(ptr, shape=(k,)).copy() if k else np.zeros(0, dtype)
+        aln_off = arr(r.aln_off, n + 1, np.int64) if n else np.zeros(1, np.int64)
+        total = int(aln_off[-1])
+        return {"score": int(r.score),
+                "cells": arr(r.cells, 2 * n, np.int32).reshape(n, 2),
+                "beginnings": arr(r.beginning, n, np.int32),
+                "aln_off": aln_off,
+                "ref_aln": np.frombuffer(C.string_at(C.addressof(r.ref_aln.contents), total), np.uint8) if total else np.zeros(0, np.uint8),
+                "read_aln": np.frombuffer(C.string_at(C.addressof(r.read_aln.contents), total), np.uint8) if total else np.zeros(0, np.uint8)}
+    finally:
+        L.sw_oracle_free(C.byref(r))
+
+
 def score(ref, read, match: int = 5, mismatch: int = -3, gap: int = -4) -> Tuple[int, int]:
     """(max score, number of max cells), two-row memory."""
     L = lib()

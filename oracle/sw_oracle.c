@@ -321,11 +321,24 @@ int sw_oracle_align_gt(const char *ref, int64_t n, const char *read, int64_t m,
             for (int64_t p = 0; p < depth; ++p) { ra[k][p] = stack[2 * (depth - 1 - p)]; qa[k][p] = stack[2 * (depth - 1 - p) + 1]; }
             order[k] = k;
         }
-        /* stable insertion sort by beginning (lists are short in tests) */
-        for (int64_t a = 1; a < nc; ++a) {
-            const int64_t x = order[a]; int64_t b = a;
-            while (b > 0 && beg[order[b - 1]] > beg[x]) { order[b] = order[b - 1]; --b; }
-            order[b] = x;
+        /* stable sort by beginning: a bottom-up merge sort, O(n log n) also when a list of ~10^5 cells arrives with
+           its beginnings far from sorted (a tandem repeat lists its max cells diagonal by diagonal) */
+        {
+            int64_t *tmp = (int64_t *)malloc(((size_t)nc + 1) * sizeof(int64_t));
+            if (!tmp) goto oom;
+            int64_t *src = order, *dst = tmp;
+            for (int64_t w = 1; w < nc; w *= 2) {
+                for (int64_t lo = 0; lo < nc; lo += 2 * w) {
+                    const int64_t mid = lo + w < nc ? lo + w : nc, hi = lo + 2 * w < nc ? lo + 2 * w : nc;
+                    int64_t a = lo, b = mid, k = lo;
+                    while (a < mid && b < hi) dst[k++] = beg[src[b]] < beg[src[a]] ? src[b++] : src[a++];
+                    while (a < mid) dst[k++] = src[a++];
+                    while (b < hi) dst[k++] = src[b++];
+                }
+                int64_t *t = src; src = dst; dst = t;
+            }
+            if (src != order) memcpy(order, src, (size_t)nc * sizeof(int64_t));
+            free(tmp);
         }
         int64_t total = 0;
         for (int64_t k = 0; k < nc; ++k) total += len[k];

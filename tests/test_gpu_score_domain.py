@@ -196,9 +196,9 @@ def test_largest_scores_inside_the_call_domain(engine, scores):
     assert int(res.scores.max()) == max(scores[0], scores[1], 0) * EDGE_M
     _check(res, refs, reads, scores, max_cells=100)
     res.free(); rs.free()
-    check_hits(engine, refs, reads, scores, k=2, max_cells=50)
+    check_hits(engine, refs, reads, scores, k=2)
     for margin in (0, 2**31 - 1):
-        check_all_hits(engine, refs, reads, scores, margin=margin, max_cells=50)
+        check_all_hits(engine, refs, reads, scores, margin=margin)
 
 
 @pytest.mark.parametrize("scores", edge_score_sets(BIG_OUT), ids=["match", "gap", "mismatch"])

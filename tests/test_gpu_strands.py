@@ -12,7 +12,7 @@ import oracle
 import sparksmithwaterman_b200 as swb
 from sparksmithwaterman_b200 import synth
 from sparksmithwaterman_b200.engine import reverse_complement
-from tests.helpers import launched_kernels, launches, parts_workspace
+from tests.helpers import launched_kernels, launches, parts_workspace, result_ops
 from tests.test_hits_host import top_hits_ref
 
 pytestmark = pytest.mark.gpu
@@ -26,10 +26,6 @@ def _wrap_sum(a):
     return (a.astype(np.int64).sum(axis=1) & 0xFFFFFFFF).astype(np.uint32).view(np.int32)
 
 
-def _ops(res, cells):
-    return [res.ops(int(c)).tolist() for c in cells]
-
-
 def check_strands(eng, refs, reads, scores=(5, -3, -4), k=None, min_score=1, **kw):
     """The both-strands call against the plain call over reads + rc(reads)."""
     rs = eng.load_refset(refs)
@@ -40,7 +36,7 @@ def check_strands(eng, refs, reads, scores=(5, -3, -4), k=None, min_score=1, **k
 
 
 def _check(rs, refs, reads, scores, k, min_score, scores_only=False, tie_gt=False, fetch=True, resident=False,
-           rc=reverse_complement, max_ops=400):
+           rc=reverse_complement):
     n, R = len(reads), len(refs)
     plain = rs.align(list(reads) + [rc(q) for q in reads], scores, scores_only=scores_only, tie_gt=tie_gt).cache()
     if resident:
@@ -77,8 +73,7 @@ def _check(rs, refs, reads, scores, k, min_score, scores_only=False, tie_gt=Fals
         assert (res.cell_offsets == off_p).all()
         assert (res.cells == cells_p).all()
         assert (res.beginnings == plain.beginnings).all() and (res.op_lens == plain.op_lens).all()
-        sample = range(min(res.total_cells, max_ops))
-        assert _ops(res, sample) == _ops(plain, sample)
+        assert np.array_equal(result_ops(res, 0, res.total_cells), result_ops(plain, 0, plain.total_cells))
         return res
     hits = res.hits
     assert (hits[:, :, :2] == top_hits_ref(exp, k, min_score)[:, :, :2]).all()
@@ -98,7 +93,7 @@ def _check(rs, refs, reads, scores, k, min_score, scores_only=False, tie_gt=Fals
             assert (res.cells[b0:b0 + c] == cells_p[p0:p0 + c]).all()
             assert (res.beginnings[b0:b0 + c] == plain.beginnings[p0:p0 + c]).all()
             assert (res.op_lens[b0:b0 + c] == plain.op_lens[p0:p0 + c]).all()
-            assert _ops(res, range(b0, b0 + min(c, 20))) == _ops(plain, range(p0, p0 + min(c, 20)))
+            assert np.array_equal(result_ops(res, b0, b0 + c), result_ops(plain, p0, p0 + c))
     assert (cnt_b[~mask] == 0).all()
     return res
 
