@@ -1,6 +1,7 @@
 // swb_align.cu -- the align driver: the steps of one call over a packed set (K classes of short reads in batches of
-// read pairs, the wide reads, hits mode's selections, the device-side assembly), a set cut into parts aligned part by
-// part with each part's results crossing PCIe while the next one computes, and the fetch of a result to the host.
+// read pairs, the wide reads, the selections of hits and all-hits mode, the device-side assembly), a set cut into parts
+// aligned part by part with each part's results crossing PCIe while the next one computes, and the fetch of a result to
+// the host.
 #include "swb_host.h"
 
 using namespace swbh;
@@ -55,11 +56,11 @@ int record_words(int K) { return ((K + 1 + 7) / 8 + CB / 8) * 8; }         // pe
 // error paths).  SWB_F_BOTH_STRANDS: rd holds the 2n internal reads and the result is oriented, 2R references x n reads;
 // its cells and pairs count both strands.
 using ResultPtr = std::unique_ptr<swb_result, void (*)(swb_result *)>;
-ResultPtr new_result(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, uint32_t flags)
+ResultPtr new_result(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, uint32_t flags, const Selection &sel)
 {
     ResultPtr res(new swb_result(), swb_result_free);
     ctx->live.fetch_add(1);
-    res->ctx = ctx; res->n_refs = rs->n_refs; res->n_reads = rd->n_reads; res->flags = flags;
+    res->ctx = ctx; res->n_refs = rs->n_refs; res->n_reads = rd->n_reads; res->flags = flags; res->sel = sel;
     res->ref_len = rs->len_orig; res->read_len = rd->len;
     if (flags & SWB_F_BOTH_STRANDS) {
         res->n_refs = 2 * rs->n_refs; res->n_reads = rd->n_reads / 2;
@@ -91,8 +92,7 @@ int AlignCall::run(int32_t *ext_scores, int32_t *ext_totals)
     if (ext_totals) res->d_totals.view(ext_totals, (size_t)o_refs); else CU(res->d_totals.alloc((size_t)o_refs, st));
     CU(res->d_best.alloc((size_t)o_reads * 4, st));
     CU(cudaMemsetAsync(res->d_scores.p, 0, std::max<size_t>(n_pairs, 1) * 4, st));
-    res->top_k = top_k; res->min_score = min_score; res->margin = margin;
-    if (top_k > 0) CU(res->d_hits.alloc((size_t)o_reads * top_k * 4, st));
+    if (sel.mode == Selection::TOP_K) CU(res->d_hits.alloc((size_t)o_reads * sel.top_k * 4, st));
 
     const auto t_wall0 = std::chrono::steady_clock::now();
     ctx->ev_used = 0;                                    // the timer's spans reuse the context's events
@@ -107,8 +107,7 @@ int AlignCall::run(int32_t *ext_scores, int32_t *ext_totals)
         if (!wide.empty() && (rc = run_wide_reads(wide))) return rc;
     }
     DevBuf<uint32_t> keep;
-    if (top_k > 0 && (rc = select_final_hits(keep))) return rc;
-    if (margin >= 0 && (rc = select_final_all_hits(keep))) return rc;
+    if (sel.mode != Selection::NONE && (rc = select_final(keep))) return rc;
     if ((rc = assemble(keep))) return rc;
     return finish_stats(t_wall0);
 }
@@ -206,7 +205,7 @@ int AlignCall::fill_batch(int K, const std::vector<int32_t> &reads, int64_t rp0,
         }
     ++n_batches;
     // both strands in hits / all-hits mode: the selection's slots, the forward read of each read pair, follow the read pairs
-    const bool fwd_slots = both && selecting() && !(flags & SWB_F_SCORES_ONLY);
+    const bool fwd_slots = both && sel.mode != Selection::NONE && !(flags & SWB_F_SCORES_ONLY);
     if (fwd_slots)
         for (int r = 0; r < n_rp; ++r) b.h_rp.push_back(b.h_rp[(size_t)r * 2]);
     CU(ctx->rp.reserve(b.h_rp.size(), st));
@@ -247,7 +246,7 @@ int AlignCall::trace_batch(int K, Batch &b)
     const bool scores_only = (flags & SWB_F_SCORES_ONLY) != 0;
     // hits / all-hits mode: the scan makes the batch's score rows exact, the selection marks the pairs the emit keeps
     size_t sel_words = 0;
-    if (selecting() && !scores_only) {
+    if (sel.mode != Selection::NONE && !scores_only) {
         sel_words = ((size_t)b.n_rp * 2 * (size_t)rs->n_refs + 31) / 32;
         CU(ctx->hit_sel.reserve(sel_words, st));
         b.P.sel = ctx->hit_sel.p;
@@ -290,7 +289,7 @@ int AlignCall::trace_batch(int K, Batch &b)
 }
 
 // candidate tiles -> exact pair scores and, unless scores only, the batch's max-cell keys (unsorted, ctx->keys_tmp).
-// sel_words > 0 (hits mode): the selection between the scan and the emit marks the pairs whose cells the emit keeps.
+// sel_words > 0 (a selection): marked between the scan and the emit, the pairs whose cells the emit keeps.
 // One host sync for the two counts; lists that did not fit are made again with the counted sizes.
 int AlignCall::locate_cells(int K, const Batch &b, size_t sel_words, uint32_t &n_cells)
 {
@@ -311,21 +310,13 @@ int AlignCall::locate_cells(int K, const Batch &b, size_t sel_words, uint32_t &n
                          ctx->sm_count, 0, st));
         launches += 2;
         if (sel_words) {
-            CU(timer.begin(STAT_SELECT_MS));
             CU(cudaMemsetAsync(ctx->hit_sel.p, 0, sel_words * 4, st));
             // both strands: one slot per read pair over the 2R oriented references; oriented o = 2r + s marks bit
-            // (2 * rp + s) * R + r, the emit's bit of pair (r, strand s of read pair rp)
-            // all-hits mode: a batch covers all references of its reads, so each read's best score is exact here
-            if (margin >= 0 && both)
-                CU(select_margin(P.rp_reads + (size_t)b.n_rp * 2, b.n_rp, 1, ctx->hit_sel.p, 2 * rs->n_refs, rs->n_refs, true));
-            else if (margin >= 0)
-                CU(select_margin(P.rp_reads, (int64_t)b.n_rp * 2, 1, ctx->hit_sel.p, rs->n_refs, 1));
-            else if (both)
-                CU(select_hits(P.rp_reads + (size_t)b.n_rp * 2, b.n_rp, 1, nullptr, ctx->hit_sel.p, 2 * rs->n_refs, rs->n_refs, true));
-            else
-                CU(select_hits(P.rp_reads, (int64_t)b.n_rp * 2, 1, nullptr, ctx->hit_sel.p, rs->n_refs, 1));
-            CU(timer.end());
-            launches += 2;
+            // (2 * rp + s) * R + r, the emit's bit of pair (r, strand s of read pair rp).  A batch covers all references
+            // of its reads, so each read's best score (the margin's bar) is exact here
+            const int rc = both ? mark_selection(P.rp_reads + (size_t)b.n_rp * 2, b.n_rp, 1, ctx->hit_sel.p, 2 * rs->n_refs, rs->n_refs, true)
+                                : mark_selection(P.rp_reads, (int64_t)b.n_rp * 2, 1, ctx->hit_sel.p, rs->n_refs, 1);
+            if (rc) return rc;
         }
         if (!scores_only) {
             CU(launch_locate(K, P, ctx->tasks.p, d_ntasks, cap_tasks, ctx->task_hits.p, ctx->keys_tmp.p, cap_cells, d_ncells,
@@ -344,105 +335,77 @@ int AlignCall::locate_cells(int K, const Batch &b, size_t sel_words, uint32_t &n
     return SWB_OK;
 }
 
-// hits mode: top k + best pair of the reads `slots` (score rows exact by now) -> `bits` / `hits` (swb_hits.cu)
-// over the oriented view: slots are oriented reads, the references oriented references
-cudaError_t AlignCall::select_hits(const int32_t *slots, int64_t n_slots, int with_best, int4 *hits, uint32_t *bits, int64_t bit_slot,
-                                   int64_t bit_ref, bool oriented_bits)
+// marks the pairs the selection keeps among the reads `slots` (nullptr: every read; their score rows are exact by now)
+// in `bits`, and each read's best pair with `with_best`; hits mode also writes the reads' top k lists to `hits` when
+// it is not null (swb_hits.cu).  Over the oriented view: slots are oriented reads, the references oriented references;
+// pair (slot, o) is bit slot * bit_slot + o * bit_ref, or with `oriented_bits` slot * bit_slot + (o & 1) * bit_ref + (o >> 1)
+int AlignCall::mark_selection(const int32_t *slots, int64_t n_slots, int with_best, uint32_t *bits, int64_t bit_slot,
+                              int64_t bit_ref, bool oriented_bits, int4 *hits)
 {
-    const size_t te = select_hits_tmp_elems(o_refs, n_slots, top_k);
-    cudaError_t e = ctx->hit_tmp.reserve(te, st);
-    if (e == cudaSuccess) e = launch_select_hits(res->d_scores.p, o_refs, o_reads, slots, n_slots, top_k, min_score, with_best,
-                                                 hits, bits, bit_slot, bit_ref, oriented_bits, ctx->hit_tmp.p, te, st);
-    return e;
+    CU(timer.begin(STAT_SELECT_MS));
+    if (sel.mode == Selection::TOP_K) {
+        const size_t te = select_hits_tmp_elems(o_refs, n_slots, sel.top_k);
+        CU(ctx->hit_tmp.reserve(te, st));
+        CU(launch_select_hits(res->d_scores.p, o_refs, o_reads, slots, n_slots, sel.top_k, sel.min_score, with_best, hits, bits,
+                              bit_slot, bit_ref, oriented_bits, ctx->hit_tmp.p, te, st));
+    } else {
+        CU(ctx->margin_best.reserve((size_t)std::max<int64_t>(n_slots, 1), st));
+        CU(launch_select_margin(res->d_scores.p, o_refs, o_reads, slots, n_slots, sel.min_score, sel.margin, with_best, bits, bit_slot,
+                                bit_ref, oriented_bits, ctx->margin_best.p, st));
+    }
+    CU(timer.end());
+    launches += 2;
+    return SWB_OK;
 }
 
-// all-hits mode: the per-read maximum and the marking pass of swb_hits.cu over `slots` (score rows exact by now)
-cudaError_t AlignCall::select_margin(const int32_t *slots, int64_t n_slots, int with_best, uint32_t *bits, int64_t bit_slot,
-                                     int64_t bit_ref, bool oriented_bits)
-{
-    cudaError_t e = ctx->margin_best.reserve((size_t)std::max<int64_t>(n_slots, 1), st);
-    if (e == cudaSuccess) e = launch_select_margin(res->d_scores.p, o_refs, o_reads, slots, n_slots, min_score, margin, with_best, bits,
-                                                   bit_slot, bit_ref, oriented_bits, ctx->margin_best.p, st);
-    return e;
-}
-
-// the reads of the int32 wide path; hits mode: exact scores of every wide pair first, then the whole wide path over each
-// read's top k + best pair (all-hits mode: its listed pairs + best pair, a list of any length).  Both strands: `wide`
-// holds (q, n + q) next to each other (classify_reads); the selection runs once per read q over the oriented references,
-// and each strand takes the references of its own orientation.
+// the reads of the int32 wide path.  With a selection: exact scores of every wide pair first, then the whole wide path
+// over each read's selected pairs and its best pair.  Slot x's selected references are row x of a bit matrix
+// [slots x o_refs], which the host reads once.  Both strands: `wide` holds (q, n + q) next to each other
+// (classify_reads); the selection runs once per read q over the oriented references, and each strand takes the
+// references of its own orientation.
 int AlignCall::run_wide_reads(const std::vector<int32_t> &wide)
 {
-    if (!selecting() || (flags & SWB_F_SCORES_ONLY)) return run_wide_path(wide, (flags & SWB_F_SCORES_ONLY) != 0);
+    const bool scores_only = (flags & SWB_F_SCORES_ONLY) != 0;
+    if (sel.mode == Selection::NONE || scores_only) return run_wide_path(wide, scores_only);
     int rc = run_wide_path(wide, true);
     if (rc) return rc;
     std::vector<int32_t> slots;
     for (size_t x = 0; x < wide.size(); x += both ? 2 : 1) slots.push_back(wide[x]);
     const int64_t nw = (int64_t)slots.size();
-    DevBuf<int32_t> d_wr;
-    CU(d_wr.alloc((size_t)nw, st));
-    CU(cudaMemcpyAsync(d_wr.p, slots.data(), (size_t)nw * 4, cudaMemcpyHostToDevice, st));
-    if (margin >= 0) return run_wide_listed(wide, d_wr.p, nw);
-    CU(timer.begin(STAT_SELECT_MS));
-    int4 *d_sel = reinterpret_cast<int4 *>(res->d_hits.p);              // scratch here: the final selection rewrites it
-    CU(select_hits(d_wr.p, nw, 1, d_sel, nullptr, 0, 0));
-    CU(timer.end());
-    launches += 2;
-    std::vector<int4> h_sel((size_t)nw * top_k);
-    CU(cudaMemcpyAsync(h_sel.data(), d_sel, h_sel.size() * sizeof(int4), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    std::vector<std::vector<int32_t>> refs_of(wide.size());
-    for (size_t x = 0; x < wide.size(); ++x) {
-        const size_t sx = both ? x / 2 : x;
-        for (int h = 0; h < top_k; ++h) {
-            const int32_t o = h_sel[sx * top_k + h].y;
-            if (o < 0) continue;
-            if (!both) refs_of[x].push_back(o);
-            else if ((o & 1) == (int32_t)(x & 1)) refs_of[x].push_back(o >> 1);
-        }
-        std::sort(refs_of[x].begin(), refs_of[x].end());
-    }
-    return run_wide_path(wide, false, &refs_of);
-}
-
-// all-hits mode, wide reads: slot x's pairs to trace are bits x * o_refs + o of a bit matrix (one row per slot), which
-// the host turns into each wide read's reference list
-int AlignCall::run_wide_listed(const std::vector<int32_t> &wide, const int32_t *d_slots, int64_t nw)
-{
     const size_t words = ((size_t)nw * (size_t)o_refs + 31) / 32;
+    DevBuf<int32_t> d_wr;
     DevBuf<uint32_t> d_bits;
+    CU(d_wr.alloc((size_t)nw, st));
     CU(d_bits.alloc(words, st));
+    CU(cudaMemcpyAsync(d_wr.p, slots.data(), (size_t)nw * 4, cudaMemcpyHostToDevice, st));
     CU(cudaMemsetAsync(d_bits.p, 0, words * 4, st));
-    CU(timer.begin(STAT_SELECT_MS));
-    CU(select_margin(d_slots, nw, 1, d_bits.p, o_refs, 1));
-    CU(timer.end());
-    launches += 2;
+    if ((rc = mark_selection(d_wr.p, nw, 1, d_bits.p, o_refs, 1))) return rc;
     std::vector<uint32_t> h_bits(words);
     CU(cudaMemcpyAsync(h_bits.data(), d_bits.p, words * 4, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     std::vector<std::vector<int32_t>> refs_of(wide.size());
-    for (size_t x = 0; x < wide.size(); ++x) {
-        const int64_t sx = both ? (int64_t)(x / 2) : (int64_t)x;
-        for (int64_t o = 0; o < o_refs; ++o) {
-            const int64_t bit = sx * o_refs + o;
-            if (!((h_bits[(size_t)(bit >> 5)] >> (bit & 31)) & 1u)) continue;
-            if (!both) refs_of[x].push_back((int32_t)o);
-            else if ((o & 1) == (int64_t)(x & 1)) refs_of[x].push_back((int32_t)(o >> 1));
+    for (size_t w = 0; w < words; ++w)
+        for (uint32_t m = h_bits[w]; m; m &= m - 1) {                   // ascending bits: each row's references ascending
+            const int64_t bit = (int64_t)w * 32 + __builtin_ctz(m), x = bit / o_refs, o = bit % o_refs;
+            if (both) refs_of[(size_t)(2 * x + (o & 1))].push_back((int32_t)(o >> 1));
+            else refs_of[(size_t)x].push_back((int32_t)o);
         }
-    }
     return run_wide_path(wide, false, &refs_of);
 }
 
-// all-hits mode: the final lists over all reads (every score is exact now) and, with cells, the listed pairs as the
-// pairs whose cells the assembly keeps.  One host sync for the list's length.
-int AlignCall::select_final_all_hits(DevBuf<uint32_t> &keep)
+// the final selection over all reads (every score is exact now): the result's lists and, with cells, the selected
+// pairs as the pairs whose cells the assembly keeps.  Hits mode: the top k lists.  All-hits mode: the lists built from
+// the marking pass's per-read best, with one host sync for their length.
+int AlignCall::select_final(DevBuf<uint32_t> &keep)
 {
     const size_t n_pairs = (size_t)(rs->n_refs * rd->n_reads);
     if (!(flags & SWB_F_SCORES_ONLY)) {
         CU(keep.alloc((n_pairs + 31) / 32, st));
         CU(cudaMemsetAsync(keep.p, 0, ((n_pairs + 31) / 32) * 4, st));
     }
+    int rc = mark_selection(nullptr, o_reads, 0, keep.p, 1, o_reads, false, reinterpret_cast<int4 *>(res->d_hits.p));
+    if (rc || sel.mode == Selection::TOP_K) return rc;
     CU(timer.begin(STAT_SELECT_MS));
-    CU(select_margin(nullptr, o_reads, 0, keep.p, 1, o_reads));
     const size_t n_count = margin_count_elems(o_refs, o_reads);
     DevBuf<int64_t> count, off;
     DevBuf<uint8_t> tmp;
@@ -450,7 +413,8 @@ int AlignCall::select_final_all_hits(DevBuf<uint32_t> &keep)
     CU(off.alloc(n_count, st));
     size_t tmp_bytes = margin_list_tmp_bytes(o_refs, o_reads, 0);
     CU(tmp.alloc(tmp_bytes, st));
-    CU(launch_margin_count(res->d_scores.p, o_refs, o_reads, min_score, margin, ctx->margin_best.p, count.p, off.p, tmp.p, tmp_bytes, st));
+    CU(launch_margin_count(res->d_scores.p, o_refs, o_reads, sel.min_score, sel.margin, ctx->margin_best.p, count.p, off.p, tmp.p,
+                           tmp_bytes, st));
     int64_t n_hits = 0;
     CU(cudaMemcpyAsync(&n_hits, off.p + n_count - 1, 8, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
@@ -466,26 +430,11 @@ int AlignCall::select_final_all_hits(DevBuf<uint32_t> &keep)
     CU(idx_tmp.alloc((size_t)n_hits, st)); CU(order.alloc((size_t)n_hits, st));
     tmp_bytes = margin_list_tmp_bytes(o_refs, o_reads, n_hits);
     CU(tmp.alloc(tmp_bytes, st));
-    CU(launch_margin_write(res->d_scores.p, o_refs, o_reads, min_score, margin, ctx->margin_best.p, off.p, n_hits, list_tmp.p,
+    CU(launch_margin_write(res->d_scores.p, o_refs, o_reads, sel.min_score, sel.margin, ctx->margin_best.p, off.p, n_hits, list_tmp.p,
                            keys_tmp.p, keys_sorted.p, idx_tmp.p, order.p, reinterpret_cast<int4 *>(res->d_hit_list.p),
                            res->d_hit_off.p, tmp.p, tmp_bytes, st));
     CU(timer.end());
-    launches += 8;
-    return SWB_OK;
-}
-
-// hits mode: the final lists (every score is exact now) and, with cells, the pairs whose cells the assembly keeps
-int AlignCall::select_final_hits(DevBuf<uint32_t> &keep)
-{
-    const size_t n_pairs = (size_t)(rs->n_refs * rd->n_reads);
-    if (!(flags & SWB_F_SCORES_ONLY)) {
-        CU(keep.alloc((n_pairs + 31) / 32, st));
-        CU(cudaMemsetAsync(keep.p, 0, ((n_pairs + 31) / 32) * 4, st));
-    }
-    CU(timer.begin(STAT_SELECT_MS));
-    CU(select_hits(nullptr, o_reads, 0, reinterpret_cast<int4 *>(res->d_hits.p), keep.p, 1, o_reads));
-    CU(timer.end());
-    launches += 2;
+    launches += 6;
     return SWB_OK;
 }
 
@@ -557,10 +506,10 @@ int AlignCall::assemble(const DevBuf<uint32_t> &keep)
     launches += 8;
     if (keep.p) {
         CU(assemble_hit_cells(d_desc.p, (int)descs.size(), d_pair_sorted.p, d_order.p, N, (int64_t)n_pairs, o_reads, res->f_cell_off.p,
-                              res->f_cells.p, res->d_best.p, res->d_hits.p, top_k, st));
+                              res->f_cells.p, res->d_best.p, res->d_hits.p, sel.top_k, st));
         launches += 2;
     }
-    if (margin >= 0) {
+    if (sel.mode == Selection::MARGIN) {
         CU(assemble_list_cells(res->d_hit_off.p, o_reads, res->d_hit_list.p, res->n_hits, res->f_cell_off.p, res->f_cells.p, st));
         ++launches;
     }
@@ -596,16 +545,14 @@ static int check_call(const swb_ctx *ctx, const swb_refset *rs, const swb_reads 
 
 // One packed set (a whole small set, or one part of a large one): AlignCall::run, then the fetch unless SWB_F_NO_FETCH
 static int align_leaf(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
-                      int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, int32_t margin, int32_t *ext_scores,
-                      int32_t *ext_totals, swb_result **out)
+                      int32_t gap, uint32_t flags, const Selection &sel, int32_t *ext_scores, int32_t *ext_totals, swb_result **out)
 {
     std::lock_guard<std::recursive_mutex> lk(ctx->mu);
     CU(cudaSetDevice(ctx->device));
-    ResultPtr res = new_result(ctx, rs, rd, flags);
-    AlignCall call{ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, res.get(), ctx->stream, {ctx, ctx->stream}};
+    ResultPtr res = new_result(ctx, rs, rd, flags, sel);
+    AlignCall call{ctx, rs, rd, match, mismatch, gap, flags, sel, res.get(), ctx->stream, {ctx, ctx->stream}};
     call.both = (flags & SWB_F_BOTH_STRANDS) != 0;
     call.o_refs = res->n_refs; call.o_reads = res->n_reads;
-    call.margin = margin;
     int rc = call.run(ext_scores, ext_totals);
     if (rc) return rc;
     swb_result *r = res.release();
@@ -740,16 +687,10 @@ int finish_parts_fetch(swb_result *res)
 
 }  // namespace
 
-static int check_hits_args(const char *who, int32_t top_k, int32_t min_score)
-{
-    if (top_k < 1 || top_k > 32) return fail(SWB_E_INVALID, std::string(who) + ": top_k must be 1 .. 32");
-    if (min_score < 1) return fail(SWB_E_INVALID, std::string(who) + ": min_score must be >= 1");
-    return SWB_OK;
-}
+}  // extern "C"
 
-// top_k > 0: hits mode; margin >= 0: all-hits mode
 static int align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
-                          int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, int32_t margin, swb_result **out)
+                          int32_t gap, uint32_t flags, const Selection &sel, swb_result **out)
 {
     if (!ctx || !rs || !rd || !out) return fail(SWB_E_INVALID, "swb_align: null argument");
     *out = nullptr;
@@ -760,21 +701,20 @@ static int align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *r
     if (flags & SWB_F_BOTH_STRANDS) {
         std::unique_ptr<swb_reads> rd2;
         if ((rc = both_strands_reads(ctx, rs, rd, rd2))) return rc;
-        return align_leaf(ctx, rs->parts.empty() ? rs : rs->whole, rd2.get(), match, mismatch, gap, flags, top_k, min_score, margin,
-                          nullptr, nullptr, out);
+        return align_leaf(ctx, rs->parts.empty() ? rs : rs->whole, rd2.get(), match, mismatch, gap, flags, sel, nullptr, nullptr, out);
     }
-    if (rs->parts.empty()) return align_leaf(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, margin, nullptr, nullptr, out);
-    // hits mode also runs on the set as one: its cell arrays are small (nothing to overlap), and the selection is then
-    // over all references at once, so no part keeps cells of a pair that a later part displaces from the top k.  The
-    // same for all-hits mode: a read's best score, and with it the margin's bar, is only known over the whole set
-    if (rs->whole && ((flags & (SWB_F_NO_FETCH | SWB_F_SCORES_ONLY)) || top_k > 0 || margin >= 0))
-        return align_leaf(ctx, rs->whole, rd, match, mismatch, gap, flags, top_k, min_score, margin, nullptr, nullptr, out);
+    if (rs->parts.empty()) return align_leaf(ctx, rs, rd, match, mismatch, gap, flags, sel, nullptr, nullptr, out);
+    // a selection also runs on the set as one: its cell arrays are small (nothing to overlap), and the selection is then
+    // over all references at once, so no part keeps cells of a pair that a later part displaces from the top k, and a
+    // read's best score, and with it the margin's bar, is known over the whole set
+    if (rs->whole && ((flags & (SWB_F_NO_FETCH | SWB_F_SCORES_ONLY)) || sel.mode != Selection::NONE))
+        return align_leaf(ctx, rs->whole, rd, match, mismatch, gap, flags, sel, nullptr, nullptr, out);
     // ---- a set of several parts: part by part; part k's results cross PCIe while part k + 1 computes -------------
     std::lock_guard<std::recursive_mutex> lk(ctx->mu);
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const auto t_wall0 = std::chrono::steady_clock::now();
-    ResultPtr res = new_result(ctx, rs, rd, flags);
+    ResultPtr res = new_result(ctx, rs, rd, flags, sel);
     const int64_t n_refs = rs->n_refs, n_reads = rd->n_reads;
     const size_t n_pairs = (size_t)(n_refs * n_reads);
     CU(res->d_scores.alloc(n_pairs, st));
@@ -787,7 +727,7 @@ static int align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *r
         const swb_refset *part = rs->parts[k];
         const int64_t first = rs->part_first[k];
         swb_result *sub = nullptr;
-        rc = align_leaf(ctx, part, rd, match, mismatch, gap, flags | SWB_F_NO_FETCH, 0, 1, -1, res->d_scores.p + (size_t)first * (size_t)n_reads,
+        rc = align_leaf(ctx, part, rd, match, mismatch, gap, flags | SWB_F_NO_FETCH, sel, res->d_scores.p + (size_t)first * (size_t)n_reads,
                         res->d_totals.p + first, &sub);
         if (rc) return rc;
         res->subs.push_back(sub); res->sub_first.push_back(first); res->sub_copied.push_back(0);
@@ -808,40 +748,8 @@ static int align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *r
     return SWB_OK;
 }
 
-int swb_align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
-                       int32_t gap, uint32_t flags, swb_result **out)
-{
-    return align_resident(ctx, rs, rd, match, mismatch, gap, flags, 0, 1, -1, out);
-}
-
-int swb_align_resident_hits(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
-                            int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_result **out)
-{
-    if (out) *out = nullptr;
-    const int rc = check_hits_args("swb_align_resident_hits", top_k, min_score);
-    if (rc) return rc;
-    return align_resident(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, -1, out);
-}
-
-static int check_all_hits_args(const char *who, int32_t min_score, int32_t margin)
-{
-    if (min_score < 1) return fail(SWB_E_INVALID, std::string(who) + ": min_score must be >= 1");
-    if (margin < 0) return fail(SWB_E_INVALID, std::string(who) + ": margin must be >= 0");
-    return SWB_OK;
-}
-
-int swb_align_resident_all_hits(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
-                                int32_t gap, uint32_t flags, int32_t min_score, int32_t margin, swb_result **out)
-{
-    if (out) *out = nullptr;
-    const int rc = check_all_hits_args("swb_align_resident_all_hits", min_score, margin);
-    if (rc) return rc;
-    return align_resident(ctx, rs, rd, match, mismatch, gap, flags, 0, min_score, margin, out);
-}
-
-static int align_host(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
-                      int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, int32_t margin,
-                      swb_result **out)
+int swbh::align_host(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
+                     int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, const Selection &sel, swb_result **out)
 {
     if (!out) return fail(SWB_E_INVALID, "swb_align: out is null");
     *out = nullptr;
@@ -858,34 +766,60 @@ static int align_host(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const
     float h2d = 0;
     cudaEventElapsedTime(&h2d, e0, e1);
     cudaEventDestroy(e0); cudaEventDestroy(e1);
-    rc = align_resident(ctx, rs, rd, match, mismatch, gap, flags, top_k, min_score, margin, out);
+    rc = align_resident(ctx, rs, rd, match, mismatch, gap, flags, sel, out);
     swb_reads_free(rd);
     if (rc == SWB_OK) (*out)->stats[STAT_H2D_MS] = h2d;
     return rc;
 }
 
+extern "C" {
+
+int swb_align_resident(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
+                       int32_t gap, uint32_t flags, swb_result **out)
+{
+    return align_resident(ctx, rs, rd, match, mismatch, gap, flags, Selection{}, out);
+}
+
+int swb_align_resident_hits(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
+                            int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_result **out)
+{
+    const Selection sel{Selection::TOP_K, top_k, min_score};
+    if (out) *out = nullptr;
+    const int rc = check_selection("swb_align_resident_hits", sel);
+    return rc ? rc : align_resident(ctx, rs, rd, match, mismatch, gap, flags, sel, out);
+}
+
+int swb_align_resident_all_hits(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, int32_t match, int32_t mismatch,
+                                int32_t gap, uint32_t flags, int32_t min_score, int32_t margin, swb_result **out)
+{
+    const Selection sel{Selection::MARGIN, 0, min_score, margin};
+    if (out) *out = nullptr;
+    const int rc = check_selection("swb_align_resident_all_hits", sel);
+    return rc ? rc : align_resident(ctx, rs, rd, match, mismatch, gap, flags, sel, out);
+}
+
 int swb_align(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
               int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, swb_result **out)
 {
-    return align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, 1, -1, out);
+    return align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, Selection{}, out);
 }
 
 int swb_align_hits(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
                    int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_result **out)
 {
+    const Selection sel{Selection::TOP_K, top_k, min_score};
     if (out) *out = nullptr;
-    const int rc = check_hits_args("swb_align_hits", top_k, min_score);
-    if (rc) return rc;
-    return align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, top_k, min_score, -1, out);
+    const int rc = check_selection("swb_align_hits", sel);
+    return rc ? rc : align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, sel, out);
 }
 
 int swb_align_all_hits(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
                        int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, int32_t min_score, int32_t margin, swb_result **out)
 {
+    const Selection sel{Selection::MARGIN, 0, min_score, margin};
     if (out) *out = nullptr;
-    const int rc = check_all_hits_args("swb_align_all_hits", min_score, margin);
-    if (rc) return rc;
-    return align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, min_score, margin, out);
+    const int rc = check_selection("swb_align_all_hits", sel);
+    return rc ? rc : align_host(ctx, rs, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, sel, out);
 }
 
 int swb_result_fetch(swb_result *res)
@@ -914,8 +848,9 @@ int swb_result_fetch(swb_result *res)
     if ((rc = pull(res->d_scores.p, n_pairs * 4, (const void **)&res->scores))) return rc;
     if ((rc = pull(res->d_totals.p, (size_t)res->n_refs * 4, (const void **)&res->totals))) return rc;
     if ((rc = pull(res->d_best.p, (size_t)res->n_reads * 16, (const void **)&res->best))) return rc;
-    if (res->top_k > 0 && (rc = pull(res->d_hits.p, (size_t)res->n_reads * res->top_k * 16, (const void **)&res->hits))) return rc;
-    if (res->margin >= 0) {
+    if (res->sel.mode == Selection::TOP_K && (rc = pull(res->d_hits.p, (size_t)res->n_reads * res->sel.top_k * 16, (const void **)&res->hits)))
+        return rc;
+    if (res->sel.mode == Selection::MARGIN) {
         if ((rc = pull(res->d_hit_off.p, ((size_t)res->n_reads + 1) * 8, (const void **)&res->hit_off))) return rc;
         if ((rc = pull(res->d_hit_list.p, (size_t)res->n_hits * 16, (const void **)&res->hit_list))) return rc;
     }

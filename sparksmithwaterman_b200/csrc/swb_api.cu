@@ -437,16 +437,16 @@ const int32_t *swb_result_ref_totals(const swb_result *r) { return (r && r->fetc
 const int32_t *swb_result_best_hits(const swb_result *r) { return (r && r->fetched) ? r->best : nullptr; }
 const int32_t *swb_result_hits(const swb_result *r, int32_t *top_k)
 {
-    if (top_k) *top_k = r ? r->top_k : 0;
-    return (r && r->fetched && r->top_k > 0) ? r->hits : nullptr;
+    if (top_k) *top_k = r ? r->sel.top_k : 0;                    // 0 outside hits mode
+    return (r && r->fetched && r->sel.mode == Selection::TOP_K) ? r->hits : nullptr;
 }
 const int64_t *swb_result_hit_offsets(const swb_result *r, int64_t *n_hits)
 {
-    const bool ok = r && r->fetched && r->margin >= 0;
+    const bool ok = r && r->fetched && r->sel.mode == Selection::MARGIN;
     if (n_hits) *n_hits = ok ? r->n_hits : 0;
     return ok ? r->hit_off : nullptr;
 }
-const int32_t *swb_result_hit_list(const swb_result *r) { return (r && r->fetched && r->margin >= 0) ? r->hit_list : nullptr; }
+const int32_t *swb_result_hit_list(const swb_result *r) { return (r && r->fetched && r->sel.mode == Selection::MARGIN) ? r->hit_list : nullptr; }
 const int64_t *swb_result_cell_offsets(const swb_result *r) { return (r && r->fetched) ? r->cell_off : nullptr; }
 int64_t swb_result_total_cells(const swb_result *r) { return r ? (int64_t)r->total_cells : 0; }
 const int32_t *swb_result_cells(const swb_result *r) { return (r && r->fetched) ? r->cells : nullptr; }
@@ -457,7 +457,7 @@ int64_t swb_result_pair_cell_count(const swb_result *r, int64_t pair)
 {
     if (!r || !r->fetched || pair < 0 || pair >= r->n_refs * r->n_reads) return -1;
     if (r->flags & SWB_F_SCORES_ONLY) return -1;
-    if (r->scores[(size_t)pair] == 0 && r->top_k == 0 && r->margin < 0) {   // hits / all-hits mode: a score-0 pair is never listed, its range is empty
+    if (r->scores[(size_t)pair] == 0 && r->sel.mode == Selection::NONE) {   // hits / all-hits mode: a score-0 pair is never listed, its range is empty
         const int64_t ref = pair / r->n_reads, rd = pair % r->n_reads;
         return (int64_t)r->ref_len[(size_t)ref] * r->read_len[(size_t)rd];     // every cell ties at 0
     }
@@ -470,7 +470,7 @@ int swb_result_pair_cell(const swb_result *r, int64_t pair, int64_t k, int32_t *
     const int64_t cnt = swb_result_pair_cell_count(r, pair);
     if (cnt < 0) return fail(SWB_E_RANGE, "swb_result_pair_cell: bad pair");
     if (k < 0 || k >= cnt) return fail(SWB_E_RANGE, "swb_result_pair_cell: bad cell index");
-    if (r->scores[(size_t)pair] == 0 && r->top_k == 0 && r->margin < 0) {
+    if (r->scores[(size_t)pair] == 0 && r->sel.mode == Selection::NONE) {
         const int64_t n = r->ref_len[(size_t)(pair / r->n_reads)];
         if (i) *i = (int32_t)(k / n + 1);
         if (j) *j = (int32_t)(k % n + 1);

@@ -131,6 +131,23 @@ template <class T> struct DevBuf {
 
 inline int upper(int c) { return (c >= 'a' && c <= 'z') ? c - 32 : c; }
 
+// Which pairs of a call are traced (include/swb200.h): all of them (swb_align), each read's top_k best pairs with score
+// >= min_score (hits mode, swb_align_hits), or each read's pairs with score >= max(min_score, read's best - margin)
+// (all-hits mode, swb_align_all_hits).  The entry points build it and check it once (check_selection).
+struct Selection {
+    enum Mode { NONE, TOP_K, MARGIN } mode = NONE;
+    int32_t top_k = 0, min_score = 1, margin = 0;
+};
+
+// the argument rules of the selecting entry points; `who` names the entry in the message
+inline int check_selection(const char *who, const Selection &sel)
+{
+    if (sel.mode == Selection::TOP_K && (sel.top_k < 1 || sel.top_k > 32)) return fail(SWB_E_INVALID, std::string(who) + ": top_k must be 1 .. 32");
+    if (sel.mode != Selection::NONE && sel.min_score < 1) return fail(SWB_E_INVALID, std::string(who) + ": min_score must be >= 1");
+    if (sel.mode == Selection::MARGIN && sel.margin < 0) return fail(SWB_E_INVALID, std::string(who) + ": margin must be >= 0");
+    return SWB_OK;
+}
+
 // grid of a grid-stride loop over n elements
 inline int grid_for(int64_t n, int threads, int sm_count)
 {
@@ -277,11 +294,10 @@ struct swb_result {
     bool fetched = false;
     std::vector<int32_t> ref_len, read_len;
     DevBuf<int32_t> d_scores, d_totals, d_best;
-    int32_t top_k = 0, min_score = 1;            // hits mode (swb_align_hits): k > 0
-    DevBuf<int32_t> d_hits;                      // [n_reads][k][4] (score, ref, i, j)
+    swbh::Selection sel;
+    DevBuf<int32_t> d_hits;                      // hits mode: [n_reads][k][4] (score, ref, i, j)
     const int32_t *hits = nullptr;               // host view after fetch
-    int32_t margin = -1;                         // all-hits mode (swb_align_all_hits): margin >= 0
-    int64_t n_hits = 0;
+    int64_t n_hits = 0;                          // all-hits mode: entries of d_hit_list
     DevBuf<int64_t> d_hit_off;                   // [n_reads + 1] offsets into d_hit_list
     DevBuf<int32_t> d_hit_list;                  // [n_hits][4] (score, ref, i, j)
     const int64_t *hit_off = nullptr;            // host views after fetch
@@ -356,7 +372,10 @@ int strand_complement_codes(const swb_refset *rs, uint8_t comp_code[256]);
 int both_strands_reads(swb_ctx *ctx, const swb_refset *rs, const swb_reads *rd, std::unique_ptr<swb_reads> &out);
 
 // One align call over one packed set (a whole set, or one part of a large one), step by step (swb_align.cu; the wide
-// path in swb_wide_host.cu).  top_k > 0: hits mode (swb_align_hits); margin >= 0: all-hits mode (swb_align_all_hits).
+// path in swb_wide_host.cu).  With a selection (hits or all-hits mode) every pair is scored and only the selected ones
+// are traced: a short-read batch marks its selection between the tile scan and the emit, the wide reads are scored
+// first and then traced over their selected references, and a final selection over all reads makes the result's lists
+// and the pairs whose cells the assembly keeps.
 // Two views of the pairs: the fill, locate, traceback and assembly sort run over (rs->n_refs, rd->n_reads); the
 // totals, best hits and selections over the result's oriented (o_refs, o_reads).  They are the same unless `both`
 // (SWB_F_BOTH_STRANDS): rd then holds the 2n internal reads [reads; rc(reads)], and pair r * 2n + s * n + q of the
@@ -367,7 +386,7 @@ struct AlignCall {
     const swb_reads *rd;
     int32_t match, mismatch, gap;
     uint32_t flags;
-    int32_t top_k, min_score;
+    Selection sel;
     swb_result *res;
     cudaStream_t st;
     PhaseTimer timer;
@@ -375,10 +394,6 @@ struct AlignCall {
     double ck_bytes = 0;
     bool both = false;
     int64_t o_refs = 0, o_reads = 0;
-    int32_t margin = -1;
-
-    // hits or all-hits mode: a selection between the tile scan and the emit decides which pairs are traced
-    bool selecting() const { return top_k > 0 || margin >= 0; }
 
     struct Batch;
     int run(int32_t *ext_scores, int32_t *ext_totals);
@@ -388,18 +403,18 @@ struct AlignCall {
     int fill_batch(int K, const std::vector<int32_t> &reads, int64_t rp0, int n_rp, const swb_refset::SegTables &segt, Batch &b);
     int trace_batch(int K, Batch &b);
     int locate_cells(int K, const Batch &b, size_t sel_words, uint32_t &n_cells);
-    cudaError_t select_hits(const int32_t *slots, int64_t n_slots, int with_best, int4 *hits, uint32_t *bits, int64_t bit_slot,
-                            int64_t bit_ref, bool oriented_bits = false);
-    cudaError_t select_margin(const int32_t *slots, int64_t n_slots, int with_best, uint32_t *bits, int64_t bit_slot, int64_t bit_ref,
-                              bool oriented_bits = false);
+    int mark_selection(const int32_t *slots, int64_t n_slots, int with_best, uint32_t *bits, int64_t bit_slot, int64_t bit_ref,
+                       bool oriented_bits = false, int4 *hits = nullptr);
     int run_wide_reads(const std::vector<int32_t> &wide);
     // refs_of (nullable): refs_of[k] = the references (ascending) read reads[k] is aligned against; nullptr = all of them
     int run_wide_path(const std::vector<int32_t> &reads, bool scores_only, const std::vector<std::vector<int32_t>> *refs_of = nullptr);
-    int run_wide_listed(const std::vector<int32_t> &wide, const int32_t *d_slots, int64_t nw);
-    int select_final_hits(DevBuf<uint32_t> &keep);
-    int select_final_all_hits(DevBuf<uint32_t> &keep);
+    int select_final(DevBuf<uint32_t> &keep);
     int assemble(const DevBuf<uint32_t> &keep);
     int finish_stats(std::chrono::steady_clock::time_point t_wall0);
 };
+
+// an align call on host reads (swb_align*): upload, align, the H2D time in the result's stats
+int align_host(swb_ctx *ctx, const swb_refset *rs, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
+               int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, const Selection &sel, swb_result **out);
 
 }  // namespace swbh

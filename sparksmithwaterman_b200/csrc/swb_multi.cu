@@ -75,6 +75,19 @@ int nccl_fail(ncclResult_t r, const char *what)
         if (r_ != ncclSuccess) return nccl_fail(r_, #x);                       \
     } while (0)
 
+// all-gather of `count` elements per rank into recv [world][count] on `st`; a world of one copies on the device (and
+// never loads NCCL)
+int gather(const void *send, void *recv, size_t count, ncclDataType_t type, ncclComm_t comm, int world, cudaStream_t st)
+{
+    if (count == 0) return SWB_OK;
+    if (world > 1) {
+        const ncclResult_t r = nccl_api()->AllGather(send, recv, count, type, comm, st);
+        return r == ncclSuccess ? SWB_OK : nccl_fail(r, "ncclAllGather");
+    }
+    CU(cudaMemcpyAsync(recv, send, count * (type == ncclInt64 ? 8 : 4), cudaMemcpyDeviceToDevice, st));
+    return SWB_OK;
+}
+
 // shard-local reference index -> global index (ids), -1 stays -1 (a shard without references)
 __global__ void best_to_global_kernel(const int32_t *best, const int64_t *ids, int64_t n_ids, int64_t n_reads, int32_t *out)
 {
@@ -212,8 +225,8 @@ struct GatherBufs {
     }
 };
 
-// localize -> allgather -> merge on `st` of the current device.  `grouped`: the caller brackets several devices'
-// collectives with ncclGroupStart / ncclGroupEnd (single-process form) and launches the merge afterwards.
+// The three steps of an exchange, on `st` of the current device: localize (shard-local reference ids -> global ids, into
+// the send buffer), gather (into the gathered buffer), merge.
 cudaError_t enqueue_localize(GatherBufs &g, const int64_t *ids, int64_t n_ids, const int32_t *d_best, int64_t n_reads, int world, cudaStream_t st)
 {
     cudaError_t e = g.send.reserve((size_t)n_reads * 4, st);
@@ -323,14 +336,33 @@ struct swb_multi_result {
     swb_multi *m = nullptr;
     std::vector<swb_result *> shard;
     std::vector<int32_t> merged;
-    int32_t top_k = 0;                           // hits mode: merged_hits = [n_reads][k][4], global reference ids
-    std::vector<int32_t> merged_hits;
-    bool all_hits = false;                       // all-hits mode: merged lists, global reference ids
-    std::vector<int64_t> merged_off;
+    Selection sel;
+    std::vector<int32_t> merged_hits;            // hits mode: [n_reads][k][4], global reference ids
+    std::vector<int64_t> merged_off;             // all-hits mode: merged lists, global reference ids
     std::vector<int32_t> merged_list;
     int64_t n_reads = 0;
     double stats[3] = {0, 0, 0};
 };
+
+// the checks of a swb_comm_allgather_* call on a result that must be of selection `mode` (NONE: any), then the shard's
+// global ids on the device (c->g.ids).  The caller holds the context's lock.
+static int comm_prepare(const char *who, swb_comm *c, const swb_result *res, Selection::Mode mode, const int64_t *global_ids,
+                        int64_t n_local_refs)
+{
+    const std::string w(who);
+    if (res->ctx != c->ctx) return fail(SWB_E_INVALID, w + ": the result belongs to another context");
+    if (mode == Selection::TOP_K && res->sel.mode != mode) return fail(SWB_E_INVALID, w + ": not a hits-mode result (swb_align_hits)");
+    if (mode == Selection::MARGIN && res->sel.mode != mode) return fail(SWB_E_INVALID, w + ": not an all-hits result (swb_align_all_hits)");
+    if (mode != Selection::NONE && c->world > kMaxHitsWorld) return fail(SWB_E_UNSUPPORTED, w + ": more than 64 ranks");
+    if (n_local_refs != res->n_refs) return fail(SWB_E_INVALID, w + ": global_ids must cover the shard's references");
+    if (n_local_refs > 0 && !global_ids) return fail(SWB_E_INVALID, w + ": global_ids is null");
+    cudaStream_t st = c->ctx->stream;
+    CU(cudaSetDevice(c->ctx->device));
+    CU(c->g.ids.reserve((size_t)std::max<int64_t>(n_local_refs, 1), st));
+    c->g.n_ids = n_local_refs;
+    if (n_local_refs) CU(cudaMemcpyAsync(c->g.ids.p, global_ids, (size_t)n_local_refs * 8, cudaMemcpyHostToDevice, st));
+    return SWB_OK;
+}
 
 extern "C" {
 
@@ -379,24 +411,14 @@ int swb_comm_allgather_best(swb_comm *c, const swb_result *res, const int64_t *g
                             int32_t *merged_host)
 {
     if (!c || !res) return fail(SWB_E_INVALID, "swb_comm_allgather_best: null argument");
-    if (res->ctx != c->ctx) return fail(SWB_E_INVALID, "swb_comm_allgather_best: the result belongs to another context");
-    if (n_local_refs != res->n_refs) return fail(SWB_E_INVALID, "swb_comm_allgather_best: global_ids must cover the shard's references");
-    if (n_local_refs > 0 && !global_ids) return fail(SWB_E_INVALID, "swb_comm_allgather_best: global_ids is null");
-    swb_ctx *ctx = c->ctx;
-    std::lock_guard<std::recursive_mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
+    std::lock_guard<std::recursive_mutex> lk(c->ctx->mu);
+    int rc = comm_prepare("swb_comm_allgather_best", c, res, Selection::NONE, global_ids, n_local_refs);
+    if (rc) return rc;
+    cudaStream_t st = c->ctx->stream;
     const int64_t n_reads = res->n_reads;
     c->n_reads = n_reads;
-    CU(c->g.ids.reserve((size_t)std::max<int64_t>(n_local_refs, 1), st));
-    c->g.n_ids = n_local_refs;
-    if (n_local_refs) CU(cudaMemcpyAsync(c->g.ids.p, global_ids, (size_t)n_local_refs * 8, cudaMemcpyHostToDevice, st));
     CU(enqueue_localize(c->g, c->g.ids.p, c->g.n_ids, res->d_best.p, n_reads, c->world, st));
-    if (c->world > 1) {
-        if (n_reads) NC(nccl_api()->AllGather(c->g.send.p, c->g.gathered.p, (size_t)n_reads * 4, ncclInt32, c->comm, st));
-    } else if (n_reads) {
-        CU(cudaMemcpyAsync(c->g.gathered.p, c->g.send.p, (size_t)n_reads * 16, cudaMemcpyDeviceToDevice, st));
-    }
+    if ((rc = gather(c->g.send.p, c->g.gathered.p, (size_t)n_reads * 4, ncclInt32, c->comm, c->world, st))) return rc;
     CU(enqueue_merge(c->g, n_reads, c->world, st));
     if (merged_host && n_reads) CU(cudaMemcpyAsync(merged_host, c->g.merged.p, (size_t)n_reads * 16, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));        // global_ids / merged_host are the caller's
@@ -407,27 +429,15 @@ int swb_comm_allgather_hits(swb_comm *c, const swb_result *res, const int64_t *g
                             int32_t *merged_host)
 {
     if (!c || !res) return fail(SWB_E_INVALID, "swb_comm_allgather_hits: null argument");
-    if (res->ctx != c->ctx) return fail(SWB_E_INVALID, "swb_comm_allgather_hits: the result belongs to another context");
-    if (res->top_k <= 0) return fail(SWB_E_INVALID, "swb_comm_allgather_hits: not a hits-mode result (swb_align_hits)");
-    if (c->world > kMaxHitsWorld) return fail(SWB_E_UNSUPPORTED, "swb_comm_allgather_hits: more than 64 ranks");
-    if (n_local_refs != res->n_refs) return fail(SWB_E_INVALID, "swb_comm_allgather_hits: global_ids must cover the shard's references");
-    if (n_local_refs > 0 && !global_ids) return fail(SWB_E_INVALID, "swb_comm_allgather_hits: global_ids is null");
-    swb_ctx *ctx = c->ctx;
-    std::lock_guard<std::recursive_mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
+    std::lock_guard<std::recursive_mutex> lk(c->ctx->mu);
+    int rc = comm_prepare("swb_comm_allgather_hits", c, res, Selection::TOP_K, global_ids, n_local_refs);
+    if (rc) return rc;
+    cudaStream_t st = c->ctx->stream;
     const int64_t n_reads = res->n_reads;
-    const int k = res->top_k;
+    const int k = res->sel.top_k;
     const size_t n = (size_t)n_reads * k;
-    CU(c->g.ids.reserve((size_t)std::max<int64_t>(n_local_refs, 1), st));
-    c->g.n_ids = n_local_refs;
-    if (n_local_refs) CU(cudaMemcpyAsync(c->g.ids.p, global_ids, (size_t)n_local_refs * 8, cudaMemcpyHostToDevice, st));
     CU(enqueue_localize_hits(c->g, c->g.ids.p, c->g.n_ids, res->d_hits.p, n_reads, k, c->world, st));
-    if (c->world > 1) {
-        if (n) NC(nccl_api()->AllGather(c->g.hsend.p, c->g.hgathered.p, n * 4, ncclInt32, c->comm, st));
-    } else if (n) {
-        CU(cudaMemcpyAsync(c->g.hgathered.p, c->g.hsend.p, n * 16, cudaMemcpyDeviceToDevice, st));
-    }
+    if ((rc = gather(c->g.hsend.p, c->g.hgathered.p, n * 4, ncclInt32, c->comm, c->world, st))) return rc;
     CU(enqueue_merge_hits(c->g, n_reads, k, c->world, st));
     if (merged_host && n) CU(cudaMemcpyAsync(merged_host, c->g.hmerged.p, n * 16, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));        // global_ids / merged_host are the caller's
@@ -439,40 +449,25 @@ int swb_comm_allgather_all_hits(swb_comm *c, const swb_result *res, const int64_
 {
     if (!c || !res || !offsets || !list || !n_hits) return fail(SWB_E_INVALID, "swb_comm_allgather_all_hits: null argument");
     *offsets = nullptr; *list = nullptr; *n_hits = 0;
-    if (res->ctx != c->ctx) return fail(SWB_E_INVALID, "swb_comm_allgather_all_hits: the result belongs to another context");
-    if (res->margin < 0) return fail(SWB_E_INVALID, "swb_comm_allgather_all_hits: not an all-hits result (swb_align_all_hits)");
-    if (c->world > kMaxHitsWorld) return fail(SWB_E_UNSUPPORTED, "swb_comm_allgather_all_hits: more than 64 ranks");
-    if (n_local_refs != res->n_refs) return fail(SWB_E_INVALID, "swb_comm_allgather_all_hits: global_ids must cover the shard's references");
-    if (n_local_refs > 0 && !global_ids) return fail(SWB_E_INVALID, "swb_comm_allgather_all_hits: global_ids is null");
-    swb_ctx *ctx = c->ctx;
-    std::lock_guard<std::recursive_mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
+    std::lock_guard<std::recursive_mutex> lk(c->ctx->mu);
+    int rc = comm_prepare("swb_comm_allgather_all_hits", c, res, Selection::MARGIN, global_ids, n_local_refs);
+    if (rc) return rc;
+    cudaStream_t st = c->ctx->stream;
     const int64_t n_reads = res->n_reads, no = n_reads + 1;
     const int world = c->world;
-    CU(c->g.ids.reserve((size_t)std::max<int64_t>(n_local_refs, 1), st));
-    c->g.n_ids = n_local_refs;
-    if (n_local_refs) CU(cudaMemcpyAsync(c->g.ids.p, global_ids, (size_t)n_local_refs * 8, cudaMemcpyHostToDevice, st));
     CU(c->g.aoffs.reserve((size_t)no * world, st));
     // the per-read offsets, then the largest total (one host sync), then the lists padded to it
+    if ((rc = gather(res->d_hit_off.p, c->g.aoffs.p, (size_t)no, ncclInt64, c->comm, world, st))) return rc;
     int64_t T = res->n_hits;
     if (world > 1) {
-        NC(nccl_api()->AllGather(res->d_hit_off.p, c->g.aoffs.p, (size_t)no, ncclInt64, c->comm, st));
         std::vector<int64_t> h((size_t)no * world);
         CU(cudaMemcpyAsync(h.data(), c->g.aoffs.p, h.size() * 8, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         for (int w = 0; w < world; ++w) T = std::max(T, h[(size_t)w * no + n_reads]);
-    } else {
-        CU(cudaMemcpyAsync(c->g.aoffs.p, res->d_hit_off.p, (size_t)no * 8, cudaMemcpyDeviceToDevice, st));
     }
     CU(enqueue_localize_all_hits(c->g, c->g.ids.p, c->g.n_ids, res, T, world, st));
-    if (world > 1) {
-        if (T) NC(nccl_api()->AllGather(c->g.asend.p, c->g.alists.p, (size_t)T * 4, ncclInt32, c->comm, st));
-    } else if (T) {
-        CU(cudaMemcpyAsync(c->g.alists.p, c->g.asend.p, (size_t)T * 16, cudaMemcpyDeviceToDevice, st));
-    }
-    const int rc = merge_all_hits(c->g, world, n_reads, T, res->min_score, res->margin, st);
-    if (rc) return rc;
+    if ((rc = gather(c->g.asend.p, c->g.alists.p, (size_t)T * 4, ncclInt32, c->comm, world, st))) return rc;
+    if ((rc = merge_all_hits(c->g, world, n_reads, T, res->sel.min_score, res->sel.margin, st))) return rc;
     *offsets = c->g.h_off.data(); *list = c->g.h_list.data(); *n_hits = c->g.h_off[(size_t)n_reads];
     return SWB_OK;
 }
@@ -617,22 +612,21 @@ const int64_t *swb_multi_shard_refs(const swb_multi *m, int32_t d, int64_t *n)
 
 }  // extern "C"
 
-// top_k > 0: hits mode (swb_multi_align_hits); margin >= 0: all-hits mode (swb_multi_align_all_hits)
-static int multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
-                       int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, int32_t margin,
-                       swb_multi_result **out)
+// one align call per shard (phase 1), then each mode's per-read records exchanged between the devices (phase 2) and the
+// shards' results fetched (phase 3).  `who` names the entry point in the messages.
+static int multi_align(const char *who, swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets,
+                       int32_t match, int32_t mismatch, int32_t gap, uint32_t flags, const Selection &sel, swb_multi_result **out)
 {
     if (!m || !out) return fail(SWB_E_INVALID, "swb_multi_align: null argument");
     *out = nullptr;
     const int n = (int)m->ctx.size();
-    if (top_k > 0 && n > kMaxHitsWorld) return fail(SWB_E_UNSUPPORTED, "swb_multi_align_hits: more than 64 devices");
-    if (margin >= 0 && n > kMaxHitsWorld) return fail(SWB_E_UNSUPPORTED, "swb_multi_align_all_hits: more than 64 devices");
+    if (sel.mode != Selection::NONE && n > kMaxHitsWorld) return fail(SWB_E_UNSUPPORTED, std::string(who) + ": more than 64 devices");
     for (int d = 0; d < n; ++d)
         if (!m->rs[(size_t)d]) return fail(SWB_E_INVALID, "swb_multi_align: no reference set loaded");
     std::lock_guard<std::mutex> lk(m->mu);
     const auto t0 = std::chrono::steady_clock::now();
     std::unique_ptr<swb_multi_result> res(new swb_multi_result());
-    res->m = m; res->n_reads = n_reads; res->top_k = top_k; res->all_hits = margin >= 0;
+    res->m = m; res->n_reads = n_reads; res->sel = sel;
     res->shard.assign((size_t)n, nullptr);
     auto drop = [&] { for (swb_result *r : res->shard) if (r) swb_result_free(r); res->shard.clear(); };
 
@@ -643,14 +637,8 @@ static int multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, co
         std::vector<std::thread> th;
         for (int d = 0; d < n; ++d)
             th.emplace_back([&, d] {
-                rcs[(size_t)d] = top_k > 0
-                    ? swb_align_hits(m->ctx[(size_t)d], m->rs[(size_t)d], n_reads, read_bytes, read_offsets, match, mismatch, gap,
-                                     flags | SWB_F_NO_FETCH, top_k, min_score, &res->shard[(size_t)d])
-                    : margin >= 0
-                    ? swb_align_all_hits(m->ctx[(size_t)d], m->rs[(size_t)d], n_reads, read_bytes, read_offsets, match, mismatch, gap,
-                                         flags | SWB_F_NO_FETCH, min_score, margin, &res->shard[(size_t)d])
-                    : swb_align(m->ctx[(size_t)d], m->rs[(size_t)d], n_reads, read_bytes, read_offsets, match, mismatch,
-                                gap, flags | SWB_F_NO_FETCH, &res->shard[(size_t)d]);
+                rcs[(size_t)d] = align_host(m->ctx[(size_t)d], m->rs[(size_t)d], n_reads, read_bytes, read_offsets, match, mismatch, gap,
+                                            flags | SWB_F_NO_FETCH, sel, &res->shard[(size_t)d]);
                 if (rcs[(size_t)d]) errs[(size_t)d] = swb_last_error();
             });
         for (auto &t : th) t.join();
@@ -658,80 +646,68 @@ static int multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, co
     for (int d = 0; d < n; ++d)
         if (rcs[(size_t)d]) { const int rc = rcs[(size_t)d]; const std::string e = errs[(size_t)d]; drop(); return fail(rc, "shard " + std::to_string(d) + ": " + e); }
 
-    // phase 2: best hits -> global ids -> one all-gather over NVLink -> merge, on every device's engine stream.  Both
-    // strands: the shards' records hold oriented local ids 2r + s, localized to oriented global ids 2 * gid + s, so the
-    // merge's order is the single-context order over the oriented references
+    // phase 2: the best hits (and the mode's lists) -> global ids -> all-gathered over NVLink -> merged, on every device's
+    // engine stream.  Both strands: the shards' records hold oriented local ids 2r + s, localized to oriented global ids
+    // 2 * gid + s, so the merge's order is the single-context order over the oriented references
     const auto t1 = std::chrono::steady_clock::now();
     const bool both = (flags & SWB_F_BOTH_STRANDS) != 0;
     // all-hits mode: the shards' list lengths are known on the host after their calls; T = the largest
     int64_t T = 0;
-    if (margin >= 0)
+    if (sel.mode == Selection::MARGIN)
         for (int d = 0; d < n; ++d) T = std::max(T, res->shard[(size_t)d]->n_hits);
     for (int d = 0; d < n; ++d) {
         swb_ctx *c = m->ctx[(size_t)d];
         GatherBufs &g = m->g[(size_t)d];
+        const swb_result *sh = res->shard[(size_t)d];
         const int64_t *ids = both ? g.oids.p : g.ids.p;
         const int64_t n_ids = both ? 2 * g.n_ids : g.n_ids;
         cudaError_t e = cudaSetDevice(c->device);
-        if (e == cudaSuccess) e = enqueue_localize(g, ids, n_ids, res->shard[(size_t)d]->d_best.p, n_reads, n, c->stream);
-        if (e == cudaSuccess && top_k > 0)
-            e = enqueue_localize_hits(g, ids, n_ids, res->shard[(size_t)d]->d_hits.p, n_reads, top_k, n, c->stream);
-        if (e == cudaSuccess && margin >= 0) e = enqueue_localize_all_hits(g, ids, n_ids, res->shard[(size_t)d], T, n, c->stream);
+        if (e == cudaSuccess) e = enqueue_localize(g, ids, n_ids, sh->d_best.p, n_reads, n, c->stream);
+        if (e == cudaSuccess && sel.mode == Selection::TOP_K)
+            e = enqueue_localize_hits(g, ids, n_ids, sh->d_hits.p, n_reads, sel.top_k, n, c->stream);
+        if (e == cudaSuccess && sel.mode == Selection::MARGIN) e = enqueue_localize_all_hits(g, ids, n_ids, sh, T, n, c->stream);
         if (e != cudaSuccess) { drop(); return cuda_fail(e, "swb_multi_align: best hits -> global ids"); }
     }
-    if (n > 1 && n_reads > 0) {
-        NcclApi *a = nccl_api();
-        ncclResult_t r = a->GroupStart();
-        for (int d = 0; d < n && r == ncclSuccess; ++d) {
-            r = a->AllGather(m->g[(size_t)d].send.p, m->g[(size_t)d].gathered.p, (size_t)n_reads * 4, ncclInt32, m->comms[(size_t)d],
-                             m->ctx[(size_t)d]->stream);
-            if (r == ncclSuccess && top_k > 0)
-                r = a->AllGather(m->g[(size_t)d].hsend.p, m->g[(size_t)d].hgathered.p, (size_t)n_reads * top_k * 4, ncclInt32,
-                                 m->comms[(size_t)d], m->ctx[(size_t)d]->stream);
-            if (r == ncclSuccess && margin >= 0)
-                r = a->AllGather(res->shard[(size_t)d]->d_hit_off.p, m->g[(size_t)d].aoffs.p, (size_t)n_reads + 1, ncclInt64,
-                                 m->comms[(size_t)d], m->ctx[(size_t)d]->stream);
-            if (r == ncclSuccess && margin >= 0 && T > 0)
-                r = a->AllGather(m->g[(size_t)d].asend.p, m->g[(size_t)d].alists.p, (size_t)T * 4, ncclInt32, m->comms[(size_t)d],
-                                 m->ctx[(size_t)d]->stream);
-        }
-        const ncclResult_t r2 = a->GroupEnd();
-        if (r == ncclSuccess) r = r2;
-        if (r != ncclSuccess) { drop(); return nccl_fail(r, "swb_multi_align: ncclAllGather"); }
+    // the gathers of all devices, as one NCCL group
+    NcclApi *a = n > 1 ? nccl_api() : nullptr;
+    ncclResult_t r = a ? a->GroupStart() : ncclSuccess;
+    int rc = r == ncclSuccess ? SWB_OK : nccl_fail(r, "ncclGroupStart");
+    for (int d = 0; d < n && !rc; ++d) {
+        GatherBufs &g = m->g[(size_t)d];
+        const ncclComm_t comm = a ? m->comms[(size_t)d] : nullptr;
+        cudaStream_t st = m->ctx[(size_t)d]->stream;
+        rc = gather(g.send.p, g.gathered.p, (size_t)n_reads * 4, ncclInt32, comm, n, st);
+        if (!rc && sel.mode == Selection::TOP_K) rc = gather(g.hsend.p, g.hgathered.p, (size_t)n_reads * sel.top_k * 4, ncclInt32, comm, n, st);
+        if (!rc && sel.mode == Selection::MARGIN)
+            rc = gather(res->shard[(size_t)d]->d_hit_off.p, g.aoffs.p, (size_t)n_reads + 1, ncclInt64, comm, n, st);
+        if (!rc && sel.mode == Selection::MARGIN) rc = gather(g.asend.p, g.alists.p, (size_t)T * 4, ncclInt32, comm, n, st);
     }
+    if (a && (r = a->GroupEnd()) != ncclSuccess && !rc) rc = nccl_fail(r, "ncclGroupEnd");
+    if (rc) { const std::string err = swb_last_error(); drop(); return fail(rc, "swb_multi_align: " + err); }
+    // the merges of every device; the host copies come from device 0
     res->merged.assign((size_t)n_reads * 4, 0);
-    if (top_k > 0) res->merged_hits.assign((size_t)n_reads * top_k * 4, 0);
+    if (sel.mode == Selection::TOP_K) res->merged_hits.assign((size_t)n_reads * sel.top_k * 4, 0);
     for (int d = 0; d < n; ++d) {
         swb_ctx *c = m->ctx[(size_t)d];
         GatherBufs &g = m->g[(size_t)d];
         cudaError_t e = cudaSetDevice(c->device);
-        if (e == cudaSuccess && n == 1 && n_reads)
-            e = cudaMemcpyAsync(g.gathered.p, g.send.p, (size_t)n_reads * 16, cudaMemcpyDeviceToDevice, c->stream);
         if (e == cudaSuccess) e = enqueue_merge(g, n_reads, n, c->stream);
         if (e == cudaSuccess && d == 0 && n_reads)
             e = cudaMemcpyAsync(res->merged.data(), g.merged.p, (size_t)n_reads * 16, cudaMemcpyDeviceToHost, c->stream);
-        if (top_k > 0 && n_reads) {
-            if (e == cudaSuccess && n == 1)
-                e = cudaMemcpyAsync(g.hgathered.p, g.hsend.p, (size_t)n_reads * top_k * 16, cudaMemcpyDeviceToDevice, c->stream);
-            if (e == cudaSuccess) e = enqueue_merge_hits(g, n_reads, top_k, n, c->stream);
+        if (sel.mode == Selection::TOP_K && n_reads) {
+            if (e == cudaSuccess) e = enqueue_merge_hits(g, n_reads, sel.top_k, n, c->stream);
             if (e == cudaSuccess && d == 0)
-                e = cudaMemcpyAsync(res->merged_hits.data(), g.hmerged.p, (size_t)n_reads * top_k * 16, cudaMemcpyDeviceToHost, c->stream);
+                e = cudaMemcpyAsync(res->merged_hits.data(), g.hmerged.p, (size_t)n_reads * sel.top_k * 16, cudaMemcpyDeviceToHost, c->stream);
         }
         if (e != cudaSuccess) { drop(); return cuda_fail(e, "swb_multi_align: merge"); }
     }
     // all-hits mode: the lists are merged on device 0 (one more host sync there for the merged length)
-    if (margin >= 0) {
-        swb_ctx *c = m->ctx[0];
-        GatherBufs &g = m->g[0];
-        cudaError_t e = cudaSetDevice(c->device);
-        if (e == cudaSuccess && n == 1)
-            e = cudaMemcpyAsync(g.aoffs.p, res->shard[0]->d_hit_off.p, ((size_t)n_reads + 1) * 8, cudaMemcpyDeviceToDevice, c->stream);
-        if (e == cudaSuccess && n == 1 && T > 0)
-            e = cudaMemcpyAsync(g.alists.p, g.asend.p, (size_t)T * 16, cudaMemcpyDeviceToDevice, c->stream);
-        if (e != cudaSuccess) { drop(); return cuda_fail(e, "swb_multi_align_all_hits: merge"); }
-        const int rc = merge_all_hits(g, n, n_reads, T, min_score, margin, c->stream);
+    if (sel.mode == Selection::MARGIN) {
+        const cudaError_t e = cudaSetDevice(m->ctx[0]->device);
+        rc = e == cudaSuccess ? merge_all_hits(m->g[0], n, n_reads, T, sel.min_score, sel.margin, m->ctx[0]->stream)
+                              : cuda_fail(e, "swb_multi_align_all_hits: merge");
         if (rc) { const std::string err = swb_last_error(); drop(); return fail(rc, err); }
-        res->merged_off = g.h_off; res->merged_list = g.h_list;
+        res->merged_off = m->g[0].h_off; res->merged_list = m->g[0].h_list;
     }
     for (int d = 0; d < n; ++d) {
         cudaSetDevice(m->ctx[(size_t)d]->device);
@@ -764,25 +740,25 @@ extern "C" {
 int swb_multi_align(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
                     int32_t mismatch, int32_t gap, uint32_t flags, swb_multi_result **out)
 {
-    return multi_align(m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, 1, -1, out);
+    return multi_align("swb_multi_align", m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, Selection{}, out);
 }
 
 int swb_multi_align_hits(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
                          int32_t mismatch, int32_t gap, uint32_t flags, int32_t top_k, int32_t min_score, swb_multi_result **out)
 {
+    const Selection sel{Selection::TOP_K, top_k, min_score};
     if (out) *out = nullptr;
-    if (top_k < 1 || top_k > 32) return fail(SWB_E_INVALID, "swb_multi_align_hits: top_k must be 1 .. 32");
-    if (min_score < 1) return fail(SWB_E_INVALID, "swb_multi_align_hits: min_score must be >= 1");
-    return multi_align(m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, top_k, min_score, -1, out);
+    const int rc = check_selection("swb_multi_align_hits", sel);
+    return rc ? rc : multi_align("swb_multi_align_hits", m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, sel, out);
 }
 
 int swb_multi_align_all_hits(swb_multi *m, int64_t n_reads, const char *read_bytes, const int64_t *read_offsets, int32_t match,
                              int32_t mismatch, int32_t gap, uint32_t flags, int32_t min_score, int32_t margin, swb_multi_result **out)
 {
+    const Selection sel{Selection::MARGIN, 0, min_score, margin};
     if (out) *out = nullptr;
-    if (min_score < 1) return fail(SWB_E_INVALID, "swb_multi_align_all_hits: min_score must be >= 1");
-    if (margin < 0) return fail(SWB_E_INVALID, "swb_multi_align_all_hits: margin must be >= 0");
-    return multi_align(m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, 0, min_score, margin, out);
+    const int rc = check_selection("swb_multi_align_all_hits", sel);
+    return rc ? rc : multi_align("swb_multi_align_all_hits", m, n_reads, read_bytes, read_offsets, match, mismatch, gap, flags, sel, out);
 }
 
 void swb_multi_result_free(swb_multi_result *res)
@@ -799,17 +775,17 @@ swb_result *swb_multi_result_shard(swb_multi_result *res, int32_t d)
 const int32_t *swb_multi_result_best_hits(const swb_multi_result *res) { return res ? res->merged.data() : nullptr; }
 const int32_t *swb_multi_result_hits(const swb_multi_result *res, int32_t *top_k)
 {
-    const bool ok = res && res->top_k > 0;
-    if (top_k) *top_k = ok ? res->top_k : 0;
+    const bool ok = res && res->sel.mode == Selection::TOP_K;
+    if (top_k) *top_k = ok ? res->sel.top_k : 0;
     return ok ? res->merged_hits.data() : nullptr;
 }
 const int64_t *swb_multi_result_hit_offsets(const swb_multi_result *res, int64_t *n_hits)
 {
-    const bool ok = res && res->all_hits;
+    const bool ok = res && res->sel.mode == Selection::MARGIN;
     if (n_hits) *n_hits = ok ? res->merged_off[(size_t)res->n_reads] : 0;
     return ok ? res->merged_off.data() : nullptr;
 }
-const int32_t *swb_multi_result_hit_list(const swb_multi_result *res) { return (res && res->all_hits) ? res->merged_list.data() : nullptr; }
+const int32_t *swb_multi_result_hit_list(const swb_multi_result *res) { return (res && res->sel.mode == Selection::MARGIN) ? res->merged_list.data() : nullptr; }
 int swb_multi_result_stats(const swb_multi_result *res, double *out, int n)
 {
     if (!res || !out) return fail(SWB_E_INVALID, "swb_multi_result_stats: null");

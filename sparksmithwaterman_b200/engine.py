@@ -47,6 +47,17 @@ def _mode(top_k, margin) -> str:
     return "plain" if top_k is None and margin is None else ("hits" if margin is None else "all_hits")
 
 
+def _entry(lib, name: str, top_k, min_score, margin):
+    """The C entry point of a call's mode (_mode): `name`, name + "_hits" or name + "_all_hits", and the selection
+    arguments it takes after the flags."""
+    mode = _mode(top_k, margin)
+    if mode == "plain":
+        return getattr(lib, name), ()
+    if mode == "hits":
+        return getattr(lib, name + "_hits"), (top_k, min_score)
+    return getattr(lib, name + "_all_hits"), (min_score, margin)
+
+
 def _flags(scores_only: bool, fetch: bool, tie_gt: bool, both_strands: bool) -> int:
     return ((SWB_F_SCORES_ONLY if scores_only else 0) | (0 if fetch else SWB_F_NO_FETCH) | (SWB_F_TIE_GT if tie_gt else 0)
             | (SWB_F_BOTH_STRANDS if both_strands else 0))
@@ -151,19 +162,11 @@ class RefSet:
         if isinstance(reads, Reads):
             return reads.align(scores, scores_only, fetch, tie_gt, top_k=top_k, min_score=min_score, both_strands=both_strands,
                                margin=margin)
-        mode = _mode(top_k, margin)
+        fn, sel = _entry(self.eng.lib, "swb_align", top_k, min_score, margin)
         data, off, bs = concat(reads)
         flags = _flags(scores_only, fetch, tie_gt, both_strands)
         h = C.c_void_p()
-        if mode == "plain":
-            check(self.eng.lib.swb_align(self.eng.h, self.h, len(bs), data, _i64p(off),
-                                         scores[0], scores[1], scores[2], flags, C.byref(h)))
-        elif mode == "all_hits":
-            check(self.eng.lib.swb_align_all_hits(self.eng.h, self.h, len(bs), data, _i64p(off),
-                                                  scores[0], scores[1], scores[2], flags, min_score, margin, C.byref(h)))
-        else:
-            check(self.eng.lib.swb_align_hits(self.eng.h, self.h, len(bs), data, _i64p(off),
-                                              scores[0], scores[1], scores[2], flags, top_k, min_score, C.byref(h)))
+        check(fn(self.eng.h, self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags, *sel, C.byref(h)))
         return AlignResult(self, bs, h, scores_only, both_strands=both_strands)
 
 
@@ -193,18 +196,10 @@ class Reads:
     def align(self, scores=DEFAULT_SCORES, scores_only: bool = False, fetch: bool = True,
               tie_gt: bool = False, *, top_k: int | None = None, min_score: int = 1,
               both_strands: bool = False, margin: int | None = None) -> "AlignResult":
-        mode = _mode(top_k, margin)
+        fn, sel = _entry(self.rs.eng.lib, "swb_align_resident", top_k, min_score, margin)
         flags = _flags(scores_only, fetch, tie_gt, both_strands)
         h = C.c_void_p()
-        lib = self.rs.eng.lib
-        if mode == "plain":
-            check(lib.swb_align_resident(self.rs.eng.h, self.rs.h, self.h, scores[0], scores[1], scores[2], flags, C.byref(h)))
-        elif mode == "all_hits":
-            check(lib.swb_align_resident_all_hits(self.rs.eng.h, self.rs.h, self.h, scores[0], scores[1], scores[2], flags,
-                                                  min_score, margin, C.byref(h)))
-        else:
-            check(lib.swb_align_resident_hits(self.rs.eng.h, self.rs.h, self.h, scores[0], scores[1], scores[2], flags,
-                                              top_k, min_score, C.byref(h)))
+        check(fn(self.rs.eng.h, self.rs.h, self.h, scores[0], scores[1], scores[2], flags, *sel, C.byref(h)))
         return AlignResult(self.rs, self.seqs, h, scores_only, both_strands=both_strands)
 
 

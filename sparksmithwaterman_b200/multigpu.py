@@ -113,7 +113,7 @@ def allgather_best_hits(best_global, group=None):
 import ctypes as _C
 
 from . import _ffi
-from .engine import AlignResult, DEFAULT_SCORES, concat, _flags, _i64p, _mode
+from .engine import AlignResult, DEFAULT_SCORES, concat, _entry, _flags, _i64p
 from ._ffi import SWB_F_NO_FETCH, SWB_F_SCORES_ONLY, SWB_F_TIE_GT, check  # noqa: F401
 
 
@@ -175,18 +175,11 @@ class MultiEngine:
         """top_k: hits mode (swb_multi_align_hits), every shard in hits mode and the hit lists merged (MultiResult.hits).
         margin: all-hits mode (swb_multi_align_all_hits), the lists merged (MultiResult.hit_offsets / hit_list).
         both_strands: SWB_F_BOTH_STRANDS; merged records and MultiResult.pair use oriented global ids 2 * ref + strand."""
-        mode = _mode(top_k, margin)
+        fn, sel = _entry(self.lib, "swb_multi_align", top_k, min_score, margin)
         data, off, bs = concat(reads)
         flags = _flags(scores_only, fetch, tie_gt, both_strands)
         h = _C.c_void_p()
-        if mode == "plain":
-            check(self.lib.swb_multi_align(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags, _C.byref(h)))
-        elif mode == "all_hits":
-            check(self.lib.swb_multi_align_all_hits(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags,
-                                                    min_score, margin, _C.byref(h)))
-        else:
-            check(self.lib.swb_multi_align_hits(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags,
-                                                top_k, min_score, _C.byref(h)))
+        check(fn(self.h, len(bs), data, _i64p(off), scores[0], scores[1], scores[2], flags, *sel, _C.byref(h)))
         return MultiResult(self, bs, h, scores_only, both_strands)
 
 
