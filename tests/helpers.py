@@ -142,10 +142,11 @@ def assert_pair_equal(got, exp, tie_gt=False, where=""):
         raise AssertionError(f"op {at} (cell {cell}) {where}: {ops[at]} != {exp['ops'][at]}")
 
 
-def check_pairs(eng, refs, reads, scores=(5, -3, -4), pairs=None, max_cells=None, tie_gt=False):
+def check_pairs(eng, refs, reads, scores=(5, -3, -4), pairs=None, max_cells=None, tie_gt=False, lowmem=False):
     """Every pair (or `pairs`) of one plain call against the oracle, every max cell: assert_pair_equal.  max_cells
     limits only the check of the host string builder (swb_result_materialize) to each pair's first max_cells cells.
-    Identical (reference, read) pairs share one oracle run."""
+    Identical (reference, read) pairs share one oracle run.  lowmem: the oracle's low-memory form (a 4 Mbp x 150
+    pair needs about 3 GB with full matrices); the tie_gt oracle has no such form."""
     rs = eng.load_refset(refs)
     res = rs.align(reads, scores, tie_gt=tie_gt).cache()
     n_checked = 0
@@ -154,7 +155,7 @@ def check_pairs(eng, refs, reads, scores=(5, -3, -4), pairs=None, max_cells=None
     for (r, q) in it:
         k = (refs[r], reads[q])
         if k not in memo:
-            memo[k] = oracle_arrays(refs[r], reads[q], scores, tie_gt=tie_gt)
+            memo[k] = oracle_arrays(refs[r], reads[q], scores, tie_gt=tie_gt, lowmem=lowmem)
         exp = memo[k]
         got = result_arrays(res, r, q)
         assert_pair_equal(got, exp, tie_gt, where=f"ref={r} read={q}")

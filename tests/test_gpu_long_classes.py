@@ -90,8 +90,10 @@ def test_other_score_sets(engine, scores):
 
 
 def test_long_reference_in_segments(engine):
-    """A reference longer than two fill segments (8,192 columns each, warm-up window m + match * m / |gap| + 1):
-    planted copies of the reads at segment seams."""
+    """References of 40 and 20 kbp, both longer than two fill segments.  The call has few items, so the warm-up window
+    (W_al, from m + match * m / |gap| + 1) sets the segment length: 2 * W_al = 1,472 columns for the K = 40 read and
+    2,336 for the K = 64 reads.  Copies of the reads are planted at multiples of 8,192 columns; the cuts of the other
+    regimes are covered in test_gpu_long_refs.py."""
     rnd = random.Random(3)
     ref = list(_rand(rnd, 40000))
     r1, r2 = _rand(rnd, 480), _rand(rnd, 300)
