@@ -142,18 +142,29 @@ def assert_pair_equal(got, exp, tie_gt=False, where=""):
         raise AssertionError(f"op {at} (cell {cell}) {where}: {ops[at]} != {exp['ops'][at]}")
 
 
-def check_pairs(eng, refs, reads, scores=(5, -3, -4), pairs=None, max_cells=None, tie_gt=False, lowmem=False):
+def oracle_key(ref, read, scores, tie_gt):
+    return ref, read, tuple(scores), bool(tie_gt)
+
+
+def check_pairs(eng, refs, reads, scores=(5, -3, -4), pairs=None, max_cells=None, tie_gt=False, lowmem=False,
+                memo=None, kernels=None):
     """Every pair (or `pairs`) of one plain call against the oracle, every max cell: assert_pair_equal.  max_cells
     limits only the check of the host string builder (swb_result_materialize) to each pair's first max_cells cells.
     Identical (reference, read) pairs share one oracle run.  lowmem: the oracle's low-memory form (a 4 Mbp x 150
-    pair needs about 3 GB with full matrices); the tie_gt oracle has no such form."""
+    pair needs about 3 GB with full matrices); the tie_gt oracle has no such form.  memo: a dict of oracle results
+    (keyed by oracle_key) shared between calls.  kernels: a list that receives the call's launches
+    (launched_kernels)."""
     rs = eng.load_refset(refs)
-    res = rs.align(reads, scores, tie_gt=tie_gt).cache()
+    if kernels is None:
+        res = rs.align(reads, scores, tie_gt=tie_gt).cache()
+    else:
+        res, launched = launched_kernels(lambda: rs.align(reads, scores, tie_gt=tie_gt).cache())
+        kernels.extend(launched)
     n_checked = 0
-    memo = {}
+    memo = {} if memo is None else memo
     it = pairs if pairs is not None else [(r, q) for r in range(len(refs)) for q in range(len(reads))]
     for (r, q) in it:
-        k = (refs[r], reads[q])
+        k = oracle_key(refs[r], reads[q], scores, tie_gt)
         if k not in memo:
             memo[k] = oracle_arrays(refs[r], reads[q], scores, tie_gt=tie_gt, lowmem=lowmem)
         exp = memo[k]

@@ -7,6 +7,7 @@ import pytest
 
 import oracle
 from tests.helpers import check_pairs
+from tests.wide_trace_cases import wide_shape
 
 pytestmark = pytest.mark.gpu
 
@@ -78,8 +79,9 @@ def test_long_pair_homologous(engine):
 @pytest.mark.parametrize("scores", [(5, -3, -4), (2, -1, -2)])
 def test_few_long_walks_cluster_traceback(engine, tie_gt, scores):
     """Few max cells with long paths take the pipelined CTA-wide traceback (cluster of CTAs per cell, per-tile exit
-    tables, table chain + parallel re-walk): a homologous pair, a gappy one (low score density: the 16 x 8 corridor),
-    a low-complexity one where directions tie all along the path, under both tie rules (SmithWaterman.java:227-249
+    tables, table chain + parallel re-walk): a homologous pair, a gappy one (low score density: the 16 x 8 corridor,
+    except for the pair of the '>' rule's seed with (5, -3, -4), which scores just enough for 32 x 4), a low-complexity
+    one where directions tie all along the path, under both tie rules (SmithWaterman.java:227-249
     '>=' cascade, DistributedSW.java:310-326 strict '>': there the host layer re-orders the cells diagonal-major and
     stably by beginning, sw.distributed_order)."""
     from sparksmithwaterman_b200 import sw
@@ -102,6 +104,9 @@ def test_few_long_walks_cluster_traceback(engine, tie_gt, scores):
             assert score == exp.score, (r, q)
             assert cells == exp.cells, (r, q)
             assert sites == exp.sites, (r, q)
+            if (r, q) == (0, 1):                                        # the gappy pair's corridor shape
+                wide = not (tie_gt and scores == (5, -3, -4))
+                assert all(wide_shape(exp.score, scores[0], i, j) == wide for i, j in exp.cells), exp.cells
     res.free(); rs.free()
 
 
